@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the hot path (BVH traversal + ray/triangle intersection).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2]/[4]): synthetic displaced geodesic icosphere, 1 003 520 OBJ faces ->
@@ -14,6 +14,11 @@ One JSON line on stdout (rank 0): value = whole-job Mrays/s with rays resident i
 metric through b2rt_trace_closest with pinned HOST buffers (H2D + D2H inside the timed region);
 roofline = algorithmic bytes (48 B/ray stream + counted node/leaf bytes) / kernel time vs the measured
 HBM peak; cpu_baseline = the reference's own Intersect() (oracle/_ref) on the host cores, bounded sample.
+
+--dump-outputs DIR (rank 0) writes what the timed closest-hit and any-hit steps returned for a fixed, seeded sample of
+the stream's rays as DIR/<name>.npy, so that two builds can be compared output for output: the inputs depend only on
+the arguments. The bench writes nothing into the tree (it may be read-only); generated scenes, their binary caches and
+a rebuilt scene generator go to B2RT_SCENE_DIR, by default a per-user directory under the system's temp directory.
 """
 import argparse
 import importlib.util
@@ -22,15 +27,19 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True            # no __pycache__ in the tree for the modules imported from it
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "mini-opencl-raytracer_b200")
-SCENE_DIR = os.environ.get("B2RT_SCENE_DIR", "/tmp/b2rt_scenes")
+SCENE_DIR = os.environ.get("B2RT_SCENE_DIR") or os.path.join(tempfile.gettempdir(), "b2rt_scenes-%d" % os.getuid())
 RADIUS = 10.0
+DUMP_RAYS = 1 << 20                       # --dump-outputs: rays drawn for the sample (about 40 MB of .npy files)
 
 
 def product():
@@ -86,10 +95,16 @@ def measured_traffic(frequency, rays):
 def scenegen(*argv):
     """Synthetic scenes are written by a stand-alone executable (host/scene_gen.cpp with its own main, built by
     build.py), so that the reference arm can synthesise the identical workload without loading a product library."""
-    exe = os.path.join(PKG, "scenegen")
     src = os.path.join(PKG, "host", "scene_gen.cpp")
-    if not os.path.exists(exe) or os.path.getmtime(exe) < os.path.getmtime(src):
-        subprocess.check_call(["g++", "-std=c++17", "-O2", "-DB2RT_SCENEGEN_MAIN", src, "-o", exe])
+
+    def fresh(exe):
+        return os.path.exists(exe) and os.path.getmtime(exe) >= os.path.getmtime(src)
+    exe = os.path.join(PKG, "scenegen")
+    if not fresh(exe):
+        exe = os.path.join(SCENE_DIR, "scenegen")
+        if not fresh(exe):
+            os.makedirs(SCENE_DIR, exist_ok=True)
+            subprocess.check_call(["g++", "-std=c++17", "-O2", "-DB2RT_SCENEGEN_MAIN", src, "-o", exe])
     return int(subprocess.check_output([exe] + [str(a) for a in argv]).split()[-1])
 
 
@@ -299,10 +314,23 @@ def run_b200(args, rank, world, local_rank):
     value = world * n * args.steps / (total_ms * 1e-3) / 1e6
     kernel_ms = statistics.mean(per)
     log("[bench r%d] closest-hit per-step ms: %s" % (rank, " ".join("%.3f" % x for x in per)))
+    dump = {}
+    if rank == 0 and args.dump_outputs:
+        sel = np.arange(n) if n <= DUMP_RAYS else np.unique(np.random.default_rng(0).integers(0, n, DUMP_RAYS))
+        d_sel = torch.from_numpy(sel).cuda()
+        h = d_hits[d_sel].cpu().numpy().view(prod.HIT_DTYPE).reshape(-1)
+        dump.update(ray_index=sel.astype(np.float64), closest_t=h["t"].copy(), closest_u=h["u"].copy(), closest_v=h["v"].copy(),
+                    closest_tri=h["tri"].astype(np.float64))                    # 4294967295 = miss
 
     # ---- any-hit on the same stream ---------------------------------------------------------------------------
     any_ms, _, _ = timed(lambda: ctx.trace_any_device(d_rays.data_ptr(), n, d_occ.data_ptr(), stream.cuda_stream), args.steps, args.warmup)
     any_value = world * n * args.steps / (any_ms * 1e-3) / 1e6
+    if dump:
+        dump["any_occluded"] = d_occ[d_sel].cpu().numpy().view(np.uint32).astype(np.float64)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+        log("[bench] outputs of the last timed steps (%d sampled rays) written to %s" % (sel.size, args.dump_outputs))
 
     # ---- configs[2]: 1 M-face displaced-icosphere geometry, 4K camera rays from outside -> primary hits -> one cosine-weighted
     # bounce ray per hit, closest-hit on that incoherent batch. Bounces off ONE convex sphere all escape (r1: hit fraction
@@ -743,7 +771,10 @@ def main():
     ap.add_argument("--tiled-faces", type=int, default=10_000_000, help="tiled 4K frame (BASELINE.json configs[3]): OBJ faces of the scattered scene; 0 = cornell.obj only")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-frames", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's hits (and any-hit flags) for a seeded sample of the rays as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     if args.warmup < 3 and args.impl == "b200":
         log("[bench] note: --warmup %d < 3; the timing rules ask for >= 3" % args.warmup)
     rank = int(os.environ.get("RANK", "0"))

@@ -205,11 +205,12 @@ namespace
     }
 }
 
-// Returns the number of OBJ faces written, or -1 on I/O error / bad arguments.
+// Returns the number of OBJ faces written, or -1 on I/O error / bad arguments. Paths of any length are accepted, like
+// CLOBJloader::LoadInto does (the reference's loader overflows an 80-byte buffer beyond ~75 characters).
 extern "C" long long g3d_write_icosphere_obj(const char* path, int frequency, double radius, double amplitude, unsigned long long seed)
 {
     std::string objPath(path ? path : "");
-    if (objPath.size() < 5 || objPath.size() > 75 || frequency < 1 || frequency > 2048) return -1;
+    if (objPath.size() < 5 || frequency < 1 || frequency > 2048) return -1;
     Rng rng(seed);
     return writeSpheres(objPath, frequency, { D3{ 0, 0, 0 } }, radius, amplitude, rng);
 }
@@ -219,7 +220,7 @@ extern "C" long long g3d_write_icosphere_obj(const char* path, int frequency, do
 extern "C" long long g3d_write_spheres_obj(const char* path, int count, int frequency, double extent, double radius, double amplitude, unsigned long long seed)
 {
     std::string objPath(path ? path : "");
-    if (objPath.size() < 5 || objPath.size() > 75 || frequency < 1 || frequency > 2048 || count < 1 || count > 100000) return -1;
+    if (objPath.size() < 5 || frequency < 1 || frequency > 2048 || count < 1 || count > 100000) return -1;
     Rng rng(seed);
     std::vector<D3> centres;
     for (int i = 0; i < count; ++i) centres.push_back(D3{ (rng.uniform() * 2 - 1) * extent, (rng.uniform() * 2 - 1) * extent, (rng.uniform() * 2 - 1) * extent });
@@ -229,7 +230,7 @@ extern "C" long long g3d_write_spheres_obj(const char* path, int count, int freq
 extern "C" long long g3d_write_scattered_obj(const char* path, long long count, double extent, double edgeMin, double edgeMax, unsigned long long seed)
 {
     std::string objPath(path ? path : "");
-    if (objPath.size() < 5 || objPath.size() > 75 || count < 1) return -1;
+    if (objPath.size() < 5 || count < 1) return -1;
     if (!writeMtl(objPath)) return -1;
     FILE* file = std::fopen(objPath.c_str(), "w");
     if (!file) return -1;
