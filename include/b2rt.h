@@ -207,6 +207,21 @@ int b2rt_read_pixels_rgba8(b2rt_context* ctx, void* dst, size_t bytes);
 int b2rt_build_bvh(b2rt_context* ctx, const void* triangles, uint64_t n_triangles, void* nodes_out, uint64_t nodes_capacity,
                    uint64_t* n_nodes_out, uint32_t* order_out);
 
+/* Scene build on the device (new). d_triangles = CLTriangle[n_triangles] in LOADER order in device memory of this
+ * handle's device (the root device of a group; device or managed memory, else B2RT_INVALID_VALUE). Builds the binary BVH
+ * exactly like b2rt_build_bvh does from the same triangles (same groups, byte-identical nodes and order), re-orders the
+ * triangles on the device, creates two new buffers -- the re-ordered CLTriangle[] and the CLLinearBVHNode[] -- binds them
+ * to slots 1 and 2 (previously bound buffers are unbound, not released) and derives the compressed wide BVH on the device,
+ * byte-identical to what b2rt_upload_scene derives on the host from the same arrays: no host copy of the scene is made.
+ * On a b2rt_create_multi handle the root builds and every device gets copies. Bind the material buffer (slot 3) first.
+ * d_order_out (may be NULL): device uint32[n_triangles], order[k] = input index of triangle k. Rejects a NULL or empty
+ * array, n_triangles >= 2^31 - 1 (B2RT_INVALID_VALUE) and non-finite vertex positions or unquantisable bounds
+ * (B2RT_INVALID_ARG_VALUE); after a failure the previously bound scene is still usable. Rebinding slot 1, 2 or 3 later
+ * falls back to the host derivation; b2rt_refit_scene works on the device-built scene. The build is ordered behind the
+ * work already enqueued on cuda_stream (NULL = the context's stream) and is synchronous on return. */
+int b2rt_build_scene_device(b2rt_context* ctx, const void* d_triangles, uint64_t n_triangles, uint32_t* d_order_out,
+                            b2rt_buffer* triangles_out, b2rt_buffer* nodes_out, uint64_t* n_nodes_out, void* cuda_stream);
+
 /* Refit (new): `triangles` = CLTriangle[n_triangles] with NEW vertex data for the bound scene, same count and order
  * (animated / deformed geometry). The bound triangle buffer is replaced, the bound CLLinearBVHNode buffer gets the boxes
  * refitted bottom-up (read it back with b2rt_read_buffer to see the tree in the reference's format), and the compressed
@@ -244,7 +259,8 @@ int b2rt_camera_rays_device(b2rt_context* ctx, size_t gid_begin, size_t gid_end,
  *    image over a peer mapping, so b2rt_read_buffer / b2rt_read_pixels after it return the complete frame (the root's
  *    stream waits for all devices);
  *  - b2rt_trace_closest / b2rt_trace_any cut the host ray stream into contiguous ranges, one per device;
- *  - the *_device entry points, b2rt_build_bvh and b2rt_execute_bands address one device: the root.
+ *  - the *_device entry points, b2rt_build_bvh and b2rt_execute_bands address one device: the root
+ *    (b2rt_build_scene_device builds there and copies the scene to every device).
  * n_devices == 1 gives an ordinary handle. CLRaytracer code written against the single-device calls runs unchanged. */
 int b2rt_create_multi(const int* device_ids, int n_devices, b2rt_context** out);
 /* Devices behind a handle (b2rt_create_multi), or ranks of its job (b2rt_comm_init); 1 otherwise. */

@@ -44,7 +44,7 @@ def _run(cmd, verbose):
 
 
 def build_b2rt(force=False, verbose=True):
-    srcs = [os.path.join(CSRC, f) for f in ("kernels.cu", "lbvh.cu", "api.cu", "multi.cu", "refit.cu", "wide_bvh.cpp")]
+    srcs = [os.path.join(CSRC, f) for f in ("kernels.cu", "lbvh.cu", "api.cu", "multi.cu", "refit.cu", "scene_build.cu", "wide_bvh.cpp")]
     deps = srcs + [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(INCLUDE, "b2rt.h"), __file__]
     if not force and not _stale(LIB_B2RT, deps):
         return LIB_B2RT

@@ -29,6 +29,7 @@ SYMBOLS = [
     "b2rt_get_counters", "b2rt_reset_counters", "b2rt_launch_count", "b2rt_device_count",
     "b2rt_create_multi", "b2rt_group_size", "b2rt_group_info", "b2rt_comm_unique_id", "b2rt_comm_init", "b2rt_comm_share_output",
     "b2rt_execute_shard", "b2rt_shard_bands", "b2rt_refit_scene", "b2rt_stage_times",
+    "b2rt_build_scene_device",
 ]
 
 
@@ -104,6 +105,7 @@ def lib():
         "b2rt_launch_count": (u64, [vp]),
         "b2rt_device_count": (C.c_int, []),
         "b2rt_refit_scene": (C.c_int, [vp, vp, u64]),
+        "b2rt_build_scene_device": (C.c_int, [vp, vp, u64, vp, C.POINTER(u64), C.POINTER(u64), C.POINTER(u64), vp]),
         "b2rt_stage_times": (C.c_int, [vp, C.POINTER(u32), C.POINTER(C.c_float), u32, C.POINTER(u32)]),
         "b2rt_create_multi": (C.c_int, [C.POINTER(C.c_int), C.c_int, C.POINTER(vp)]),
         "b2rt_group_size": (C.c_int, [vp]),
@@ -265,6 +267,42 @@ class Context:
         self._ck(self._L.b2rt_build_bvh(self._h, _ptr(t), nt, _ptr(nodes), nodes.shape[0], C.byref(n_nodes), _ptr(order)))
         self.last_build_seconds = time.perf_counter() - t0          # the C call alone (grouping, device build, flattening)
         return np.ascontiguousarray(t.reshape(nt, TRI_BYTES)[order]), nodes[: n_nodes.value].copy(), order
+
+    def build_scene_device(self, d_triangles, n, d_order=0, stream=0):
+        """b2rt_build_scene_device: the whole scene built on the device from n loader-order CLTriangles at device address
+        d_triangles (e.g. a torch CUDA tensor's data_ptr()). Binds the two new buffers to slots 1 and 2; bind the
+        materials first. d_order: optional device uint32[n] receiving order[k] = input index of triangle k.
+        Returns (triangle buffer id, node buffer id, node count)."""
+        bt, bn, nn = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)
+        t0 = time.perf_counter()
+        self._ck(self._L.b2rt_build_scene_device(self._h, C.c_void_p(int(d_triangles)), int(n), C.c_void_p(int(d_order)), C.byref(bt), C.byref(bn),
+                                                 C.byref(nn), C.c_void_p(int(stream))))
+        self.last_build_seconds = time.perf_counter() - t0
+        return bt.value, bn.value, nn.value
+
+    def read_scene(self):
+        """The bound triangle (slot 1) and node (slot 2) buffers read back: ((n, 256) uint8, (m, 48) uint8)."""
+        out = []
+        for slot, rec in ((1, TRI_BYTES), (2, NODE_BYTES)):
+            buf, size, ptr = C.c_uint64(0), C.c_size_t(0), C.c_void_p()
+            self._ck(self._L.b2rt_bound_buffer(self._h, slot, C.byref(buf)))
+            self._ck(self._L.b2rt_device_pointer(self._h, buf, C.byref(ptr), C.byref(size)))
+            a = np.empty((size.value // rec, rec), dtype=np.uint8)
+            self._ck(self._L.b2rt_read_buffer(self._h, buf, _ptr(a), a.nbytes))
+            out.append(a)
+        self.finish()
+        return out[0], out[1]
+
+    def set_materials(self, mats):
+        """A new material buffer (CLMaterial[]) bound to slot 3; the previous one is released. Returns its id."""
+        m, nm = _raw(mats, MAT_BYTES, "materials")
+        old, buf = C.c_uint64(0), C.c_uint64(0)
+        self._ck(self._L.b2rt_bound_buffer(self._h, 3, C.byref(old)))
+        self._ck(self._L.b2rt_buffer_create(self._h, MEM_READ_ONLY | MEM_COPY_HOST_PTR, m.nbytes, _ptr(m), C.byref(buf)))
+        self.set_arg(3, buf.value)
+        if old.value and old.value != buf.value:
+            self._ck(self._L.b2rt_buffer_release(self._h, old.value))
+        return buf.value
 
     def resize(self, width, height):
         self._ck(self._L.b2rt_resize(self._h, int(width), int(height)))

@@ -138,18 +138,33 @@ int ensure_scene(b2rt_context* ctx) {
     CK(cudaMemcpyAsync(ctx->d_child_bin, w.child_bin.data(), w.child_bin.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaMemcpyAsync(ctx->d_leaf_dir, w.leaf_dir.data(), w.leaf_dir.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
+    // the 256 B/triangle host shadow is only needed for this build
+    bt->shadow.clear(); bt->shadow.shrink_to_fit();
+    bn->shadow.clear(); bn->shadow.shrink_to_fit();
+    DerivedScene d;
+    d.n_tris = n_tris; d.n_nodes = n_nodes; d.n_wide_nodes = w.nodes.size(); d.n_leaf_blocks = w.n_leaf_blocks;
+    d.wide_bytes = wb; d.leaf_bytes = lb; d.shade_bytes = sb;
+    d.max_depth_binary = w.max_depth_binary; d.max_depth_wide = w.max_depth_wide; d.stack_bound = bound;
+    return install_scene(ctx, d);
+}
+
+int install_scene(b2rt_context* ctx, const DerivedScene& d) {
+    Buffer* bt = find(ctx, ctx->bound[B2RT_ARG_BUFFER_SCENE]);
+    Buffer* bn = find(ctx, ctx->bound[B2RT_ARG_BUFFER_NODE]);
+    Buffer* bm = find(ctx, ctx->bound[B2RT_ARG_BUFFER_MATERIAL]);
     memset(&ctx->info, 0, sizeof(ctx->info));
-    ctx->info.n_triangles = n_tris;
-    ctx->info.n_nodes = n_nodes;
+    ctx->info.n_triangles = d.n_tris;
+    ctx->info.n_nodes = d.n_nodes;
     ctx->info.n_materials = bm ? bm->bytes / sizeof(RefMaterial) : 0;
-    ctx->info.n_wide_nodes = w.nodes.size();
-    ctx->info.n_leaf_blocks = w.n_leaf_blocks;
-    ctx->info.wide_node_bytes = wb;
-    ctx->info.leaf_bytes = lb;
-    ctx->info.shading_bytes = sb;
-    ctx->info.max_depth_binary = w.max_depth_binary;
-    ctx->info.max_depth_wide = w.max_depth_wide;
+    ctx->info.n_wide_nodes = d.n_wide_nodes;
+    ctx->info.n_leaf_blocks = d.n_leaf_blocks;
+    ctx->info.wide_node_bytes = d.wide_bytes;
+    ctx->info.leaf_bytes = d.leaf_bytes;
+    ctx->info.shading_bytes = d.shade_bytes;
+    ctx->info.max_depth_binary = d.max_depth_binary;
+    ctx->info.max_depth_wide = d.max_depth_wide;
     ctx->info.sm_count = (uint32_t)ctx->sm_count;
+    const uint32_t bound = d.stack_bound;
     ctx->stack_bound = bound;
     ctx->view.wide = static_cast<const U4*>(ctx->d_wide);
     ctx->view.leaf = static_cast<const U4*>(ctx->d_leaf);
@@ -157,14 +172,11 @@ int ensure_scene(b2rt_context* ctx) {
     ctx->view.mats = bm ? static_cast<const RefMaterial*>(bm->d_ptr) : nullptr;
     ctx->view.tris = static_cast<const RefTriangle*>(bt->d_ptr);
     ctx->view.nodes = static_cast<const RefNode*>(bn->d_ptr);
-    ctx->view.n_tris = (uint32_t)n_tris;
-    ctx->view.n_nodes = (uint32_t)n_nodes;
+    ctx->view.n_tris = (uint32_t)d.n_tris;
+    ctx->view.n_nodes = (uint32_t)d.n_nodes;
     ctx->view.n_mats = (uint32_t)ctx->info.n_materials;
-    ctx->view.n_wide = (uint32_t)w.nodes.size();
+    ctx->view.n_wide = (uint32_t)d.n_wide_nodes;
     ctx->view.one_bits = 0x3F800000u;
-    // the 256 B/triangle host shadow is only needed for this build
-    bt->shadow.clear(); bt->shadow.shrink_to_fit();
-    bn->shadow.clear(); bn->shadow.shrink_to_fit();
     int occ = 0;
     CK(trace_occupancy(false, bound, &occ));
     ctx->grid_closest = ctx->sm_count * std::max(occ, 1);

@@ -116,6 +116,18 @@ void free_tail(b2rt_context* ctx);
 void scene_l2_setup(b2rt_context* ctx);
 int buffer_create_single(b2rt_context* ctx, uint32_t flags, size_t bytes, const void* host_ptr, b2rt_buffer* out, bool zero_fill);
 bool context_alive(const b2rt_context* ctx);
+
+// What install_scene needs to know about a freshly derived compressed wide BVH (host: wide_bvh.cpp, device: scene_build.cu).
+struct DerivedScene {
+    uint64_t n_tris, n_nodes, n_wide_nodes, n_leaf_blocks;
+    size_t wide_bytes, leaf_bytes, shade_bytes;
+    uint32_t max_depth_binary, max_depth_wide, stack_bound;
+};
+// The derived arrays are in place (d_wide / d_leaf / d_shade / d_child_bin / d_leaf_dir): scene info, SceneView, launch
+// geometry, L2 set-up and tail queues for them; the peers of a device group take copies. Clears scene_dirty.
+int install_scene(b2rt_context* ctx, const DerivedScene& d);
+// refit.cu: per-triangle shading records (normals + material) of `tris`
+cudaError_t launch_shade_records(b2rt::ShadeTri* shade, const b2rt::RefTriangle* tris, uint32_t n, cudaStream_t s);
 int render_items(b2rt_context* ctx, const b2rt::GidMap& map, uint64_t n);
 int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any);
 
@@ -129,6 +141,7 @@ int group_execute(b2rt_context* ctx, size_t gid_begin, size_t gid_end);
 int group_trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any);
 int group_finish(b2rt_context* ctx);
 void group_bind_output(b2rt_context* ctx);
+int group_broadcast_buffer(b2rt_context* ctx, b2rt_buffer id);   // the root's contents of buffer `id` to every peer's copy
 const std::vector<b2rt_context*>& group_members(const b2rt_context* ctx);
 
 }  // namespace b2rt_detail

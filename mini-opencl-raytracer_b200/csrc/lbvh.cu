@@ -267,7 +267,26 @@ __global__ void order_kernel(const uint32_t* __restrict__ sorted_group, const ui
     for (uint32_t k = 0; k < n; ++k) order[at + k] = t0 + k;
 }
 
+// out[i] += block_offsets[i / SCAN_BLOCK]: the add-back that completes block_scan_kernel + sums_scan_kernel.
+__global__ void add_block_offsets_kernel(uint32_t* __restrict__ out, uint32_t m, const uint32_t* __restrict__ block_offsets) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < m) out[i] += block_offsets[i / SCAN_BLOCK];
+}
+
 }  // namespace
+
+size_t scan_scratch_words(uint32_t m) { return (m + SCAN_BLOCK - 1) / SCAN_BLOCK + 1; }
+
+cudaError_t scan_exclusive(const uint32_t* d_in, uint32_t m, uint32_t* d_out, uint32_t* d_sums, uint64_t* launches, cudaStream_t st) {
+    if (m == 0) return cudaMemsetAsync(d_sums, 0, 4, st);
+    const uint32_t n_blocks = (m + SCAN_BLOCK - 1) / SCAN_BLOCK;
+    block_scan_kernel<<<n_blocks, SCAN_BLOCK, 0, st>>>(d_in, m, d_out, d_sums);
+    sums_scan_kernel<<<1, SCAN_BLOCK, 0, st>>>(d_sums, n_blocks);
+    add_block_offsets_kernel<<<(m + 255u) / 256u, 256, 0, st>>>(d_out, m, d_sums);
+    if (launches) *launches += 3;
+    // sums_scan_kernel leaves the total in d_sums[n_blocks]; move it to the front for the caller
+    return cudaMemcpyAsync(d_sums, d_sums + n_blocks, 4, cudaMemcpyDeviceToDevice, st);
+}
 
 size_t lbvh_scratch_bytes(uint32_t m) {
     const size_t n_blocks = (m + SCAN_BLOCK - 1) / SCAN_BLOCK;

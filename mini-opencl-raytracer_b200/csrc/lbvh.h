@@ -17,4 +17,9 @@ size_t lbvh_scratch_bytes(uint32_t m);
 cudaError_t lbvh_build(const float* d_group_bounds, const uint32_t* d_first, uint32_t m, const float scene_lo[3], const float scene_hi[3],
                        void* d_scratch, RefNode* d_nodes, uint32_t* d_order, uint64_t* launches, cudaStream_t st);
 
+// Exclusive scan of m uint32 values on `st` (d_in and d_out must not overlap). d_sums: scan_scratch_words(m) words; on return d_sums[0]
+// holds the total.
+size_t scan_scratch_words(uint32_t m);
+cudaError_t scan_exclusive(const uint32_t* d_in, uint32_t m, uint32_t* d_out, uint32_t* d_sums, uint64_t* launches, cudaStream_t st);
+
 }  // namespace b2rt

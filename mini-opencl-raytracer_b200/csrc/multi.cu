@@ -212,6 +212,19 @@ int group_buffer_create(b2rt_context* ctx, uint32_t flags, size_t bytes, const v
     return B2RT_SUCCESS;
 }
 
+int group_broadcast_buffer(b2rt_context* ctx, b2rt_buffer id) {
+    Group* g = ctx->group;
+    Buffer* b = find(ctx, id);
+    if (!b) return fail(ctx, B2RT_INVALID_MEM_OBJECT, "unknown buffer");
+    std::vector<void*> ptrs{ b->d_ptr };
+    for (size_t k = 1; k < g->members.size(); ++k) {
+        Buffer* p = find(g->members[k], id);
+        if (!p || p->bytes != b->bytes) return fail(ctx, B2RT_OUT_OF_RESOURCES, "buffer ids of the device group went out of step");
+        ptrs.push_back(p->d_ptr);
+    }
+    return broadcast(ctx, ptrs.data(), b->bytes);
+}
+
 int group_each(b2rt_context* ctx, int (*fn)(b2rt_context*, void*), void* arg, bool parallel) {
     Group* g = ctx->group;
     if (parallel) return run_members(ctx, [fn, arg](b2rt_context* m, int) { return fn(m, arg); });

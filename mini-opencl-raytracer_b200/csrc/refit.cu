@@ -221,6 +221,13 @@ int refit_each(b2rt_context* ctx, void* arg) {
 
 }  // namespace
 
+namespace b2rt_detail {
+cudaError_t launch_shade_records(ShadeTri* shade, const RefTriangle* tris, uint32_t n, cudaStream_t s) {
+    if (n) refit_shade_kernel<<<(n + 255u) / 256u, 256, 0, s>>>(shade, tris, n);
+    return cudaGetLastError();
+}
+}  // namespace b2rt_detail
+
 extern "C" int b2rt_refit_scene(b2rt_context* ctx, const void* triangles, uint64_t n_triangles) {
     if (!ctx) return B2RT_INVALID_CONTEXT;
     if (!triangles || !n_triangles) return fail(ctx, B2RT_INVALID_VALUE, "refit: null or empty triangle array");

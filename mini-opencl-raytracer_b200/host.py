@@ -37,6 +37,8 @@ def lib():
         "g3d_engine_load_scene_cached": (C.c_int, [vp, cs, C.c_uint, cs, C.POINTER(C.c_int), cs, sz]),
         "g3d_scene_load_triangles": (vp, [cs, cs, sz]),
         "g3d_engine_load_scene_device_bvh": (C.c_int, [vp, cs, cs, sz]),
+        "g3d_engine_scene_from_device": (C.c_int, [vp, vp, C.c_uint64, vp, C.c_uint64, cs, sz]),
+        "g3d_engine_scene_read_back": (C.c_int, [vp, cs, sz]),
         "g3d_scene_from_triangles": (vp, [vp, u64, vp, u64, C.c_uint, cs, sz]),
         "g3d_scene_free": (None, [vp]),
         "g3d_scene_count": (u64, [vp, C.c_int]),
@@ -194,6 +196,18 @@ class Engine:
         """CLOBJloader::Load, then CLBVHScene::CreateBVHTreesDevice: the binary BVH is built on the GPU."""
         e = _err()
         self._ck(self._L.g3d_engine_load_scene_device_bvh(self._h, os.fsencode(obj_path), e, len(e)), e)
+
+    def build_scene_device(self, d_triangles, n, mats):
+        """A new scene from n loader-order CLTriangles at device address d_triangles (CLBVHScene::CreateBVHTreesFromDevice):
+        built on the GPU, nothing read back; scene_arrays() is empty until read_back_scene()."""
+        m = np.ascontiguousarray(mats)
+        e = _err()
+        self._ck(self._L.g3d_engine_scene_from_device(self._h, C.c_void_p(int(d_triangles)), int(n), m.ctypes.data, m.nbytes // 64, e, len(e)), e)
+
+    def read_back_scene(self):
+        """CLBVHScene::ReadBackScene: the device-built triangles and nodes into the host arrays."""
+        e = _err()
+        self._ck(self._L.g3d_engine_scene_read_back(self._h, e, len(e)), e)
 
     def scene_arrays(self):
         h = self._L.g3d_engine_scene(self._h)

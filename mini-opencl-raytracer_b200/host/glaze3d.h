@@ -143,6 +143,8 @@ namespace Glaze3D
         CLBuffer() {}
         // cl::Buffer(context, flags, size, host_ptr, &err)
         CLBuffer(const CLContext& context, uint32_t flags, size_t size, const void* host_ptr, int* err);
+        // New: take ownership of a buffer the library created (e.g. by b2rt_build_scene_device); released like any other
+        static CLBuffer Adopt(const CLContext& context, b2rt_buffer id, size_t size);
         b2rt_buffer id() const { return m_State ? m_State->id : 0; }
         size_t size() const { return m_State ? m_State->bytes : 0; }
     private:
@@ -203,6 +205,12 @@ namespace Glaze3D
         // built on the GPU by b2rt_build_bvh (Morton order + Karras hierarchy) instead of the SAH recursion: a few
         // milliseconds of device time instead of seconds. It is a different tree: hit IDs index THIS order.
         void CreateBVHTreesDevice();
+        // New: the whole scene built on the GPU from n LOADER-order triangles already in device memory of the context's
+        // device (b2rt_build_scene_device): m_Materials are uploaded and bound first, then the tree, the re-ordered
+        // triangles and the compressed wide BVH are made on the device. The re-ordered triangles and the node array stay
+        // there, held by m_TriangleBuffer / m_NodeBuffer; m_Triangles and Nodes() stay empty until ReadBackScene().
+        void CreateBVHTreesFromDevice(const void* d_triangles, size_t n);
+        void ReadBackScene();                                             // m_TriangleBuffer / m_NodeBuffer -> m_Triangles / Nodes()
         // New: the vertices of m_Triangles were changed in place (same count and order): refit the device scene -- node boxes,
         // compressed wide BVH, shading records -- by b2rt_refit_scene instead of building and uploading again, and read the
         // refitted node boxes back into Nodes().

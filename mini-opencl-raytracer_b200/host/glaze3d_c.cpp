@@ -137,6 +137,30 @@ extern "C" int g3d_engine_load_scene_device_bvh(void* engine, const char* objPat
     return 0;
     G3D_CATCH(-1)
 }
+// A new scene whose triangles are already on the device: CLBVHScene::CreateBVHTreesFromDevice with these materials.
+extern "C" int g3d_engine_scene_from_device(void* engine, const void* d_triangles, uint64_t n, const void* materials, uint64_t n_materials,
+                                            char* err, size_t errLen)
+{
+    G3D_TRY
+    auto& e = static_cast<EngineBox*>(engine)->engine;
+    eng = e;
+    auto scene = std::make_shared<CLBVHScene>();
+    const CLMaterial* m = static_cast<const CLMaterial*>(materials);
+    scene->m_Materials.assign(m, m + n_materials);
+    e->render->m_Scene = scene;
+    scene->CreateBVHTreesFromDevice(d_triangles, (size_t)n);
+    return 0;
+    G3D_CATCH(-1)
+}
+extern "C" int g3d_engine_scene_read_back(void* engine, char* err, size_t errLen)
+{
+    G3D_TRY
+    auto& e = static_cast<EngineBox*>(engine)->engine;
+    eng = e;
+    e->render->m_Scene->ReadBackScene();
+    return 0;
+    G3D_CATCH(-1)
+}
 extern "C" int g3d_engine_adopt_scene(void* engine, void* scene, char* err, size_t errLen)
 {
     G3D_TRY

@@ -20,6 +20,13 @@ namespace Glaze3D
         if (st == B2RT_SUCCESS) m_State = std::shared_ptr<State>(new State{ context.GetContext(), id, size });
     }
 
+    CLBuffer CLBuffer::Adopt(const CLContext& context, b2rt_buffer id, size_t size)
+    {
+        CLBuffer b;
+        if (id) b.m_State = std::shared_ptr<State>(new State{ context.GetContext(), id, size });
+        return b;
+    }
+
     // ---- CLContext --------------------------------------------------------------------------------
     CLContext::CLContext(int device) : m_Device(device)
     {

@@ -362,6 +362,44 @@ namespace Glaze3D
         SetupBuffers();
     }
 
+    void CLBVHScene::CreateBVHTreesFromDevice(const void* d_triangles, size_t n)
+    {
+        if (!eng || !eng->render || !eng->render->m_CLContext)
+            throw CLException("CLBVHScene::CreateBVHTreesFromDevice needs eng->render->m_CLContext", B2RT_INVALID_CONTEXT);
+        if (m_Materials.empty()) throw CLException("CLBVHScene::CreateBVHTreesFromDevice needs the scene's materials", B2RT_INVALID_VALUE);
+        const CLContext& ctx = *eng->render->m_CLContext;
+        b2rt_context* c = ctx.GetContext();
+        int err = 0;
+        m_MaterialBuffer = CLBuffer(ctx, B2RT_MEM_READ_ONLY | B2RT_MEM_COPY_HOST_PTR, m_Materials.size() * sizeof(CLMaterial), m_Materials.data(), &err);
+        if (err) throw CLException("Failed to create material buffer", err);
+        eng->render->SetUniform<CLBuffer>((int)RenderKernelArgument_t::BUFFER_MATERIAL, m_MaterialBuffer);
+        b2rt_buffer bt = 0, bn = 0;
+        uint64_t n_nodes = 0;
+        int st = b2rt_build_scene_device(c, d_triangles, n, nullptr, &bt, &bn, &n_nodes, nullptr);
+        if (st) throw CLException(std::string("Failed to build the scene on the device: ") + b2rt_last_error(c), st);
+        // the library has bound both buffers already; binding the same ids again changes nothing
+        m_TriangleBuffer = CLBuffer::Adopt(ctx, bt, n * sizeof(CLTriangle));
+        m_NodeBuffer = CLBuffer::Adopt(ctx, bn, (size_t)n_nodes * sizeof(CLLinearBVHNode));
+        eng->render->SetUniform<CLBuffer>((int)RenderKernelArgument_t::BUFFER_SCENE, m_TriangleBuffer);
+        eng->render->SetUniform<CLBuffer>((int)RenderKernelArgument_t::BUFFER_NODE, m_NodeBuffer);
+        m_Triangles.clear();
+        m_Nodes.clear();
+    }
+
+    void CLBVHScene::ReadBackScene()
+    {
+        if (!eng || !eng->render || !eng->render->m_CLContext)
+            throw CLException("CLBVHScene::ReadBackScene needs eng->render->m_CLContext", B2RT_INVALID_CONTEXT);
+        if (!m_TriangleBuffer.id() || !m_NodeBuffer.id()) throw CLException("CLBVHScene::ReadBackScene needs a scene on the device", B2RT_INVALID_MEM_OBJECT);
+        b2rt_context* c = eng->render->m_CLContext->GetContext();
+        m_Triangles.resize(m_TriangleBuffer.size() / sizeof(CLTriangle));
+        m_Nodes.resize(m_NodeBuffer.size() / sizeof(CLLinearBVHNode));
+        int st = b2rt_read_buffer(c, m_TriangleBuffer.id(), m_Triangles.data(), m_Triangles.size() * sizeof(CLTriangle));
+        if (!st) st = b2rt_read_buffer(c, m_NodeBuffer.id(), m_Nodes.data(), m_Nodes.size() * sizeof(CLLinearBVHNode));
+        if (!st) st = b2rt_finish(c);
+        if (st) throw CLException(std::string("Failed to read the scene back: ") + b2rt_last_error(c), st);
+    }
+
     void CLBVHScene::SetupBuffers()
     {
         if (!eng || !eng->render || !eng->render->m_CLContext)
