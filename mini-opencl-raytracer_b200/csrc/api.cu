@@ -294,11 +294,21 @@ int tail_queue(b2rt_context* ctx, int which, unsigned long long* count, unsigned
     return B2RT_SUCCESS;
 }
 
+// B2RT_OPT_TRAVERSAL=1: the reference-layout walk keeps one stack entry per level of the binary tree, at most 256. A tree
+// that passes the wide walk's check in ensure_scene is never that deep; should one be, it is refused rather than walked
+// with entries dropped.
+static int binary_walk_fits(b2rt_context* ctx) {
+    if (ctx->info.max_depth_binary <= 256) return B2RT_SUCCESS;
+    return fail(ctx, B2RT_OUT_OF_RESOURCES, "BVH too deep for the reference-layout walk's stack (binary depth " + std::to_string(ctx->info.max_depth_binary) + ")");
+}
+
 int trace_device(b2rt_context* ctx, const void* d_rays, uint64_t n, void* d_out, bool any, cudaStream_t st) {
     if (n == 0) return B2RT_SUCCESS;
     if (!d_rays || !d_out) return fail(ctx, B2RT_INVALID_VALUE, "null ray or output pointer");
     if (ctx->opt_traversal == 1) {
-        CK(launch_trace_binary(ctx->view, d_rays, n, d_out, any, st));
+        int fits = binary_walk_fits(ctx);
+        if (fits) return fits;
+        CK(launch_trace_binary(ctx->view, d_rays, n, d_out, any, ctx->info.max_depth_binary, st));
         ctx->launches += 1;
         return B2RT_SUCCESS;
     }
@@ -492,7 +502,7 @@ int render_wavefront(b2rt_context* ctx, const FrameArgs& a, float* d_result, con
     if (st) return st;
     if (a.bounces <= 0) {
         // Render() never enters its loop: radiance 0 for every pixel, which is what the megakernel does without tracing.
-        CK(launch_render_mega(ctx->view, a, d_result, map, n, false, ctx->stack_bound, ctx->stream));
+        CK(launch_render_mega(ctx->view, a, d_result, map, n, false, ctx->stack_bound, ctx->info.max_depth_binary, ctx->stream));
         ctx->launches += 1;
         return B2RT_SUCCESS;
     }
@@ -599,9 +609,11 @@ int render_items(b2rt_context* ctx, const GidMap& map, uint64_t n) {
 int render_with_mode(b2rt_context* ctx, const FrameArgs& a, float* result, const GidMap& map, uint64_t n, int mode) {
     int st = B2RT_SUCCESS;
     if (mode == 1) {
-        st = apply_l2_policy(ctx, ctx->stream);
+        if (ctx->opt_traversal == 1) st = binary_walk_fits(ctx);
+        if (!st) st = apply_l2_policy(ctx, ctx->stream);
         if (st) return st;
-        CK(launch_render_mega(ctx->view, a, result, map, (uint32_t)n, ctx->opt_traversal == 1, ctx->stack_bound, ctx->stream));
+        CK(launch_render_mega(ctx->view, a, result, map, (uint32_t)n, ctx->opt_traversal == 1, ctx->stack_bound, ctx->info.max_depth_binary,
+                              ctx->stream));
         ctx->launches += 1;
         return B2RT_SUCCESS;
     }

@@ -6,7 +6,7 @@
 //      warp-local pool, idle lanes are re-filled from the pool with ballot/popc
 //      compaction, interior-node steps and leaf steps run in separate
 //      warp-uniform loops, all node/leaf fetches are 128-bit __ldg.
-//  trace_binary_kernel<ANY>         one thread per ray over the reference's own
+//  trace_binary_kernel<ANY,CAP>     one thread per ray over the reference's own
 //      48 B / 256 B arrays in the reference's order: the "recompiled reference
 //      kernel" baseline and an on-device cross-check of the wide path.
 //  camera_rays_kernel               CreateRay (kernel_bvh.cl:386-403) as a ray stream.
@@ -508,13 +508,15 @@ trace_persistent(SceneView s, const RayIn* __restrict__ rays, uint64_t n, void* 
 }
 
 // ---------------------------------------------------------------------------------------
-// Reference-layout binary walk (kernel_bvh.cl:171-219 verbatim semantics).
+// Reference-layout binary walk (kernel_bvh.cl:171-219 verbatim semantics), except for the stack: the reference's is
+// int[64] and unchecked, so on a tree deeper than 64 levels it writes past its end. This one has CAP entries, CAP at least
+// the tree's binary depth (the walk holds at most one entry per level of the current path), like the oracle's growing stack.
 // ---------------------------------------------------------------------------------------
-template <bool ANY>
+template <bool ANY, int CAP>
 __device__ __forceinline__ HitX trace_binary(const RefTriangle* __restrict__ tris, const RefNode* __restrict__ nodes,
                                              const RayX& r, float tmax) {
     HitX h; h.t = tmax; h.u = 0.0f; h.v = 0.0f; h.tri = 0xFFFFFFFFu;
-    uint32_t stack[64];
+    uint32_t stack[CAP];
     int sp = 0;
     uint32_t cur = 0;
     for (;;) {
@@ -534,7 +536,8 @@ __device__ __forceinline__ HitX trace_binary(const RefTriangle* __restrict__ tri
             } else {
                 descend = true;
                 bool second_first = (r.sign >> axis) & 1u;
-                if (sp < 64) stack[sp++] = second_first ? cur + 1u : tail.x;
+                if (sp < CAP) stack[sp++] = second_first ? cur + 1u : tail.x;
+                else report_stack_overflow();           // never: the launch picks CAP >= the binary depth (b2rt_counters::stack_overflows)
                 cur = second_first ? tail.x : cur + 1u;
             }
         }
@@ -546,14 +549,14 @@ __device__ __forceinline__ HitX trace_binary(const RefTriangle* __restrict__ tri
     return h;
 }
 
-template <bool ANY>
+template <bool ANY, int CAP>
 __global__ void __launch_bounds__(128)
 trace_binary_kernel(SceneView s, const RayIn* __restrict__ rays, uint64_t n, void* __restrict__ out) {
     uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     RayX r; float tmax;
     load_ray(rays, i, r, tmax);
-    HitX h = trace_binary<ANY>(s.tris, s.nodes, r, tmax);
+    HitX h = trace_binary<ANY, CAP>(s.tris, s.nodes, r, tmax);
     if (ANY) reinterpret_cast<uint32_t*>(out)[i] = (h.tri != 0xFFFFFFFFu) ? 1u : 0u;
     else reinterpret_cast<float4*>(out)[i] = make_float4(h.t, h.u, h.v, __uint_as_float(h.tri));
 }
@@ -618,7 +621,7 @@ render_mega_kernel(SceneView s, FrameArgs a, float* __restrict__ result, GidMap 
     V3 radiance = v3(0.0f, 0.0f, 0.0f), beta = v3(1.0f, 1.0f, 1.0f);
     for (int b = 0; (uint32_t)b < (uint32_t)a.bounces; ++b) {              // Render(), kernel_bvh.cl:349-384
         HitX h;
-        if (BINARY) h = trace_binary<false>(s.tris, s.nodes, r, 100000.0f);
+        if (BINARY) h = trace_binary<false, CAP>(s.tris, s.nodes, r, 100000.0f);
         else h = trace_wide<false, false, CAP>(s.wide, s.leaf, r, 100000.0f, nullptr, nullptr, s.one_bits);
         V3 no, nd;
         if (!path_step(s, a, r, h, radiance, beta, seed, no, nd)) break;
@@ -798,13 +801,25 @@ uint32_t trace_warp_smem_words() { return (B2_TAIL_HELP && B2_TAIL_CODE) ? (uint
 uint32_t tail_frontier_words(uint32_t stack_bound) { uint32_t w = 4u * (stack_bound + 8u); return w < 256u ? 256u : w; }
 uint32_t tail_record_words(uint32_t stack_bound) { return TAIL_HEADER_WORDS + ((stack_bound + 8u + 3u) & ~3u); }
 
-cudaError_t launch_trace_binary(const SceneView& s, const void* d_rays, uint64_t n, void* d_out, bool any, cudaStream_t st) {
+template <int CAP>
+static void launch_binary_cap(bool any, unsigned blocks, cudaStream_t st, const SceneView& s, const RayIn* r, uint64_t n, void* out) {
+    if (any) trace_binary_kernel<true, CAP><<<blocks, 128, 0, st>>>(s, r, n, out);
+    else trace_binary_kernel<false, CAP><<<blocks, 128, 0, st>>>(s, r, n, out);
+}
+
+cudaError_t launch_trace_binary(const SceneView& s, const void* d_rays, uint64_t n, void* d_out, bool any, uint32_t max_depth_binary,
+                                cudaStream_t st) {
     if (n == 0) return cudaSuccess;
     uint64_t blocks = (n + 127) / 128;
     if (blocks > 0x7fffffffull) return cudaErrorInvalidValue;
     const RayIn* r = static_cast<const RayIn*>(d_rays);
-    if (any) trace_binary_kernel<true><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, d_out);
-    else trace_binary_kernel<false><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, d_out);
+    switch (pick_cap(max_depth_binary > 1u ? max_depth_binary : 1u)) {
+        case 32: launch_binary_cap<32>(any, (unsigned)blocks, st, s, r, n, d_out); break;
+        case 64: launch_binary_cap<64>(any, (unsigned)blocks, st, s, r, n, d_out); break;
+        case 128: launch_binary_cap<128>(any, (unsigned)blocks, st, s, r, n, d_out); break;
+        case 256: launch_binary_cap<256>(any, (unsigned)blocks, st, s, r, n, d_out); break;
+        default: return cudaErrorInvalidValue;
+    }
     return cudaGetLastError();
 }
 
@@ -816,16 +831,23 @@ cudaError_t launch_camera_rays(const FrameArgs& a, uint64_t gid0, uint64_t gid1,
     return cudaGetLastError();
 }
 
+template <int CAP>
+static void launch_mega_cap(bool binary, unsigned g, cudaStream_t st, const SceneView& s, const FrameArgs& a, float* d_result, const GidMap& map,
+                            uint32_t n) {
+    if (binary) render_mega_kernel<true, CAP><<<g, 128, 0, st>>>(s, a, d_result, map, n);
+    else render_mega_kernel<false, CAP><<<g, 128, 0, st>>>(s, a, d_result, map, n);
+}
+
 cudaError_t launch_render_mega(const SceneView& s, const FrameArgs& a, float* d_result, const GidMap& map, uint32_t n,
-                               bool binary, uint32_t stack_bound, cudaStream_t st) {
+                               bool binary, uint32_t stack_bound, uint32_t max_depth_binary, cudaStream_t st) {
     if (n == 0) return cudaSuccess;
     unsigned g = (n + 127u) / 128u;
-    if (binary) { render_mega_kernel<true, 32><<<g, 128, 0, st>>>(s, a, d_result, map, n); return cudaGetLastError(); }
-    switch (pick_cap(stack_bound)) {
-        case 32: render_mega_kernel<false, 32><<<g, 128, 0, st>>>(s, a, d_result, map, n); break;
-        case 64: render_mega_kernel<false, 64><<<g, 128, 0, st>>>(s, a, d_result, map, n); break;
-        case 128: render_mega_kernel<false, 128><<<g, 128, 0, st>>>(s, a, d_result, map, n); break;
-        case 256: render_mega_kernel<false, 256><<<g, 128, 0, st>>>(s, a, d_result, map, n); break;
+    // the wide walk holds at most stack_bound entries, the reference-layout walk at most max_depth_binary
+    switch (binary ? pick_cap(max_depth_binary > 1u ? max_depth_binary : 1u) : pick_cap(stack_bound)) {
+        case 32: launch_mega_cap<32>(binary, g, st, s, a, d_result, map, n); break;
+        case 64: launch_mega_cap<64>(binary, g, st, s, a, d_result, map, n); break;
+        case 128: launch_mega_cap<128>(binary, g, st, s, a, d_result, map, n); break;
+        case 256: launch_mega_cap<256>(binary, g, st, s, a, d_result, map, n); break;
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();

@@ -45,12 +45,14 @@ cudaError_t launch_trace_wide(const SceneView& s, const void* d_rays, uint64_t n
                               const unsigned long long* d_n = nullptr,    // d_n != null: ray count read on the device (n = upper bound)
                               const TailQueue* tail = nullptr, int tail_grid = 0,
                               cudaEvent_t between = nullptr);           // recorded between the persistent and the tail kernel (stage timing)
-// One thread per ray over the reference-layout arrays (baseline / cross-check).
-cudaError_t launch_trace_binary(const SceneView& s, const void* d_rays, uint64_t n, void* d_out, bool any, cudaStream_t st);
+// One thread per ray over the reference-layout arrays (baseline / cross-check). Its stack holds max_depth_binary entries
+// (b2rt_scene_info); cudaErrorInvalidValue for a tree deeper than 256 levels.
+cudaError_t launch_trace_binary(const SceneView& s, const void* d_rays, uint64_t n, void* d_out, bool any, uint32_t max_depth_binary,
+                                cudaStream_t st);
 cudaError_t launch_camera_rays(const FrameArgs& a, uint64_t gid0, uint64_t gid1, void* d_rays, cudaStream_t st);
-// KernelEntry for the n pixels map.gid(0..n-1), one thread per pixel.
+// KernelEntry for the n pixels map.gid(0..n-1), one thread per pixel; binary: over the reference-layout arrays.
 cudaError_t launch_render_mega(const SceneView& s, const FrameArgs& a, float* d_result, const GidMap& map, uint32_t n,
-                               bool binary, uint32_t stack_bound, cudaStream_t st);
+                               bool binary, uint32_t stack_bound, uint32_t max_depth_binary, cudaStream_t st);
 // Wavefront stages of the same frame (kernels.cu): camera rays + path state, and the per-bounce shade/compact stage.
 cudaError_t launch_wf_generate(const FrameArgs& a, const GidMap& map, uint32_t n, void* d_rays, void* d_state,
                                unsigned long long* d_queue_count, cudaStream_t st);
