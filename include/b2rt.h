@@ -231,6 +231,41 @@ int b2rt_build_scene_device(b2rt_context* ctx, const void* d_triangles, uint64_t
  * Fails (rebuild instead) when two triangles that were the loader's copies of one face no longer are. Synchronous. */
 int b2rt_refit_scene(b2rt_context* ctx, const void* triangles, uint64_t n_triangles);
 
+/* Refit from device memory (new): the same contract as b2rt_refit_scene (same topology, order and hit IDs; results equal
+ * the reference's walk over the new triangles and the refitted nodes), but the new vertex data is already on this
+ * handle's device and nothing crosses PCIe -- e.g. the animation loop "simulate (torch) -> refit -> trace / render" on one
+ * stream without a host round trip.
+ *  d_triangles: CLTriangle records, 16-byte aligned, device or managed memory of the handle's (root) device.
+ *  d_order == NULL: d_triangles holds the n scene-order triangles. It may be the bound triangle buffer itself (in place).
+ *  d_order != NULL: device uint32[n]; scene triangle k is d_triangles[d_order[k]]. This is exactly the d_order_out of
+ *                   b2rt_build_scene_device (or b2rt_build_bvh's order_out), so loader-order data can be passed as is.
+ *  d_status: device uint32, required. The call sets it to 0 on the stream, then ORs in B2RT_REFIT_* bits.
+ *  Ordered after the work already enqueued on cuda_stream (NULL = the context's stream) and on the context's stream
+ *  (which frames in flight on the wavefront path join). Work enqueued after the call on either stream sees the refitted
+ *  scene; work on any third stream is the caller's to order. On a single-device handle the call returns without waiting
+ *  for the device (only the first call after binding a new scene derives it, which waits). On a b2rt_create_multi handle
+ *  the root gathers, the peers receive copies and every device refits its own; the call is synchronous there and d_status
+ *  holds the OR of every device's bits when it returns.
+ * Returns B2RT_INVALID_CONTEXT for a NULL handle, B2RT_INVALID_KERNEL_ARGS when no built scene is bound, B2RT_INVALID_VALUE
+ * for a NULL or empty input or a NULL d_status, n_triangles different from the bound scene's count, a pointer that is not
+ * device or managed memory of the right device, d_triangles not 16-byte or d_order / d_status not 4-byte aligned, and
+ * d_triangles overlapping the bound triangle buffer when d_order is given (a gather cannot run in place) or overlapping it
+ * without being exactly it. Nothing of the scene is touched before these checks pass.
+ * A non-zero status leaves a scene that is safe to traverse but whose hits are undefined: topology and all indices are
+ * unchanged, only positions and boxes are stale or wrong. A later refit with valid data restores the scene completely,
+ * because a refit is a pure function of (topology, triangles). */
+int b2rt_refit_scene_device(b2rt_context* ctx, const void* d_triangles, uint64_t n_triangles, const uint32_t* d_order,
+                            uint32_t* d_status, void* cuda_stream);
+/* Status bits of b2rt_refit_scene_device. b2rt_refit_scene reports these conditions as B2RT_INVALID_ARG_VALUE, except that
+ * it checks vertices for non-finite values only through the boxes they produce. */
+enum {
+    B2RT_REFIT_NONFINITE = 1,      /* a non-finite vertex coordinate (every vertex is checked)                       */
+    B2RT_REFIT_DUPLICATE = 2,      /* two triangles that were the loader's copies of one face no longer are: rebuild */
+    B2RT_REFIT_RANGE = 4,          /* bounds too large to quantise                                                   */
+    B2RT_REFIT_LEAF_BOX = 8,       /* a leaf block without a stored box no longer matches its vertices               */
+    B2RT_REFIT_ORDER = 16          /* some d_order[k] >= n: scene triangle k was left as it was                      */
+};
+
 /* ---- ray-stream path (new) ----------------------------------------------------------- */
 /* Host buffers: H2D copy, trace, D2H copy, synchronous on return.
  * closest: hits[i] = {t,u,v,tri} of Intersect() (kernel_bvh.cl:171-219), tri = B2RT_MISS and

@@ -29,8 +29,10 @@ SYMBOLS = [
     "b2rt_get_counters", "b2rt_reset_counters", "b2rt_launch_count", "b2rt_device_count",
     "b2rt_create_multi", "b2rt_group_size", "b2rt_group_info", "b2rt_comm_unique_id", "b2rt_comm_init", "b2rt_comm_share_output",
     "b2rt_execute_shard", "b2rt_shard_bands", "b2rt_refit_scene", "b2rt_stage_times",
-    "b2rt_build_scene_device",
+    "b2rt_build_scene_device", "b2rt_refit_scene_device",
 ]
+# status bits of b2rt_refit_scene_device
+REFIT_NONFINITE, REFIT_DUPLICATE, REFIT_RANGE, REFIT_LEAF_BOX, REFIT_ORDER = 1, 2, 4, 8, 16
 
 
 class SceneInfo(C.Structure):
@@ -106,6 +108,7 @@ def lib():
         "b2rt_device_count": (C.c_int, []),
         "b2rt_refit_scene": (C.c_int, [vp, vp, u64]),
         "b2rt_build_scene_device": (C.c_int, [vp, vp, u64, vp, C.POINTER(u64), C.POINTER(u64), C.POINTER(u64), vp]),
+        "b2rt_refit_scene_device": (C.c_int, [vp, vp, u64, vp, vp, vp]),
         "b2rt_stage_times": (C.c_int, [vp, C.POINTER(u32), C.POINTER(C.c_float), u32, C.POINTER(u32)]),
         "b2rt_create_multi": (C.c_int, [C.POINTER(C.c_int), C.c_int, C.POINTER(vp)]),
         "b2rt_group_size": (C.c_int, [vp]),
@@ -279,6 +282,14 @@ class Context:
                                                  C.byref(nn), C.c_void_p(int(stream))))
         self.last_build_seconds = time.perf_counter() - t0
         return bt.value, bn.value, nn.value
+
+    def refit_scene_device(self, d_triangles, n, d_status, d_order=0, stream=0):
+        """b2rt_refit_scene_device: refit the bound scene from n CLTriangles at device address d_triangles -- scene order,
+        or loader order gathered through d_order (the build's device order). d_status: device uint32 that receives the
+        REFIT_* bits on the stream. Enqueued behind the work on `stream` (0 = the context's stream) and the context's
+        stream; does not wait for the device on a single-device handle."""
+        self._ck(self._L.b2rt_refit_scene_device(self._h, C.c_void_p(int(d_triangles)), int(n), C.c_void_p(int(d_order)),
+                                                 C.c_void_p(int(d_status)), C.c_void_p(int(stream))))
 
     def read_scene(self):
         """The bound triangle (slot 1) and node (slot 2) buffers read back: ((n, 256) uint8, (m, 48) uint8)."""

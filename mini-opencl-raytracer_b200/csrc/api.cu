@@ -706,8 +706,10 @@ extern "C" int b2rt_create(int device_id, b2rt_context** out) {
         if ((e = cudaEventCreateWithFlags(&ctx->ev_wf_join[i], cudaEventDisableTiming)) != cudaSuccess) return bail(e, "cudaEventCreate");
     }
     if ((e = cudaEventCreateWithFlags(&ctx->ev_wf_fork, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "cudaEventCreate");
-    for (int i = 0; i < 2; ++i)
+    for (int i = 0; i < 2; ++i) {
         if ((e = cudaEventCreate(&ctx->ev_tune[i])) != cudaSuccess) return bail(e, "cudaEventCreate");
+        if ((e = cudaEventCreateWithFlags(&ctx->ev_refit[i], cudaEventDisableTiming)) != cudaSuccess) return bail(e, "cudaEventCreate");
+    }
     {   // stream-ordered allocations (b2rt_build_bvh) stay mapped between calls up to 256 MB
         cudaMemPool_t pool = nullptr;
         if (cudaDeviceGetDefaultMemPool(&pool, device_id) == cudaSuccess) {
@@ -754,7 +756,10 @@ extern "C" void b2rt_destroy(b2rt_context* ctx) {
         if (ctx->ev_wf_join[i]) cudaEventDestroy(ctx->ev_wf_join[i]);
     }
     if (ctx->ev_wf_fork) cudaEventDestroy(ctx->ev_wf_fork);
-    for (int i = 0; i < 2; ++i) if (ctx->ev_tune[i]) cudaEventDestroy(ctx->ev_tune[i]);
+    for (int i = 0; i < 2; ++i) {
+        if (ctx->ev_tune[i]) cudaEventDestroy(ctx->ev_tune[i]);
+        if (ctx->ev_refit[i]) cudaEventDestroy(ctx->ev_refit[i]);
+    }
     for (cudaEvent_t ev : ctx->stage_events) cudaEventDestroy(ev);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
     if (ctx->stream_in) cudaStreamDestroy(ctx->stream_in);

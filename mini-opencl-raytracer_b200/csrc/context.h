@@ -81,6 +81,7 @@ struct b2rt_context {
     std::pair<uint64_t, int> tune_pending_key;
     int tune_pending_mode = -1;
     cudaEvent_t ev_tune[2] = { nullptr, nullptr };
+    cudaEvent_t ev_refit[2] = { nullptr, nullptr };   // b2rt_refit_scene_device: caller's stream -> context's stream and back
     void* d_rgba8 = nullptr;            // 8-bit read-back staging
     uint64_t rgba8_capacity = 0;
     cudaEvent_t ev_in[2] = { nullptr, nullptr }, ev_comp[2] = { nullptr, nullptr }, ev_out[2] = { nullptr, nullptr };

@@ -14,7 +14,9 @@ _LIB = None
 
 
 class HostError(RuntimeError):
-    pass
+    def __init__(self, text, status=None):
+        super().__init__(text)
+        self.status = status                # the C++ CLException's code where the call reports it, else None
 
 
 def lib_path():
@@ -39,6 +41,7 @@ def lib():
         "g3d_engine_load_scene_device_bvh": (C.c_int, [vp, cs, cs, sz]),
         "g3d_engine_scene_from_device": (C.c_int, [vp, vp, C.c_uint64, vp, C.c_uint64, cs, sz]),
         "g3d_engine_scene_read_back": (C.c_int, [vp, cs, sz]),
+        "g3d_engine_scene_refit_device": (C.c_int, [vp, vp, C.c_uint64, cs, sz]),
         "g3d_scene_from_triangles": (vp, [vp, u64, vp, u64, C.c_uint, cs, sz]),
         "g3d_scene_free": (None, [vp]),
         "g3d_scene_count": (u64, [vp, C.c_int]),
@@ -208,6 +211,15 @@ class Engine:
         """CLBVHScene::ReadBackScene: the device-built triangles and nodes into the host arrays."""
         e = _err()
         self._ck(self._L.g3d_engine_scene_read_back(self._h, e, len(e)), e)
+
+    def refit_scene_device(self, d_triangles, n):
+        """CLBVHScene::RefitFromDevice: new vertex data for the device scene from n CLTriangles at device address d_triangles,
+        in loader order for a scene made by build_scene_device, else in scene order. Raises HostError (with .status) on
+        failure, status -50 (CL_INVALID_ARG_VALUE) when the refit reported bad data."""
+        e = _err()
+        rc = self._L.g3d_engine_scene_refit_device(self._h, C.c_void_p(int(d_triangles)), int(n), e, len(e))
+        if rc:
+            raise HostError(e.value.decode(), rc)
 
     def scene_arrays(self):
         h = self._L.g3d_engine_scene(self._h)

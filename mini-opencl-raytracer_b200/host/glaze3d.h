@@ -208,13 +208,20 @@ namespace Glaze3D
         // New: the whole scene built on the GPU from n LOADER-order triangles already in device memory of the context's
         // device (b2rt_build_scene_device): m_Materials are uploaded and bound first, then the tree, the re-ordered
         // triangles and the compressed wide BVH are made on the device. The re-ordered triangles and the node array stay
-        // there, held by m_TriangleBuffer / m_NodeBuffer; m_Triangles and Nodes() stay empty until ReadBackScene().
+        // there, held by m_TriangleBuffer / m_NodeBuffer; m_Triangles and Nodes() stay empty until ReadBackScene(). The
+        // triangle order of the build stays on the device too (m_OrderBuffer), for RefitFromDevice.
         void CreateBVHTreesFromDevice(const void* d_triangles, size_t n);
         void ReadBackScene();                                             // m_TriangleBuffer / m_NodeBuffer -> m_Triangles / Nodes()
         // New: the vertices of m_Triangles were changed in place (same count and order): refit the device scene -- node boxes,
         // compressed wide BVH, shading records -- by b2rt_refit_scene instead of building and uploading again, and read the
         // refitted node boxes back into Nodes().
         void Refit();
+        // New: refit the device scene from n triangles already in device memory of the context's device
+        // (b2rt_refit_scene_device): in LOADER order for a scene made by CreateBVHTreesFromDevice (gathered through
+        // m_OrderBuffer), in scene order for a scene built or uploaded from the host. Synchronous; a status bit set by the
+        // refit throws CLException(B2RT_INVALID_ARG_VALUE) naming it. m_Triangles / Nodes() are left as they are (stale);
+        // ReadBackScene() refreshes them.
+        void RefitFromDevice(const void* d_triangles, size_t n);
         const std::vector<CLLinearBVHNode>& Nodes() const { return m_Nodes; }
         void SetupBuffers();                                              // CLBVHnode.cpp:209-236
 
@@ -226,6 +233,8 @@ namespace Glaze3D
     private:
         std::vector<CLLinearBVHNode> m_Nodes;
         CLBuffer m_TriangleBuffer, m_NodeBuffer, m_MaterialBuffer;
+        CLBuffer m_OrderBuffer;           // uint32 per triangle: loader index of scene triangle k (device-built scenes only)
+        CLBuffer m_RefitStatusBuffer;     // uint32: RefitFromDevice's status word, made on its first call
     };
 
     class CLOBJloader

@@ -161,6 +161,26 @@ extern "C" int g3d_engine_scene_read_back(void* engine, char* err, size_t errLen
     return 0;
     G3D_CATCH(-1)
 }
+// CLBVHScene::RefitFromDevice: new vertex data already on the device (loader order for a device-built scene). Returns the
+// CLException's status (e.g. B2RT_INVALID_ARG_VALUE for a refit status bit), -1 for any other failure.
+extern "C" int g3d_engine_scene_refit_device(void* engine, const void* d_triangles, uint64_t n, char* err, size_t errLen)
+{
+    try {
+        auto& e = static_cast<EngineBox*>(engine)->engine;
+        eng = e;
+        e->render->m_Scene->RefitFromDevice(d_triangles, (size_t)n);
+        return 0;
+    } catch (const CLException& x) {
+        setError(err, errLen, x.what());
+        return x.code ? x.code : -1;
+    } catch (const std::exception& x) {
+        setError(err, errLen, x.what());
+        return -1;
+    } catch (...) {
+        setError(err, errLen, "unknown exception");
+        return -1;
+    }
+}
 extern "C" int g3d_engine_adopt_scene(void* engine, void* scene, char* err, size_t errLen)
 {
     G3D_TRY

@@ -373,10 +373,16 @@ namespace Glaze3D
         m_MaterialBuffer = CLBuffer(ctx, B2RT_MEM_READ_ONLY | B2RT_MEM_COPY_HOST_PTR, m_Materials.size() * sizeof(CLMaterial), m_Materials.data(), &err);
         if (err) throw CLException("Failed to create material buffer", err);
         eng->render->SetUniform<CLBuffer>((int)RenderKernelArgument_t::BUFFER_MATERIAL, m_MaterialBuffer);
+        CLBuffer order(ctx, 0, n * sizeof(uint32_t), nullptr, &err);
+        if (err) throw CLException("Failed to create triangle order buffer", err);
+        void* d_order = nullptr;
+        err = b2rt_device_pointer(c, order.id(), &d_order, nullptr);
+        if (err) throw CLException("Failed to find the triangle order buffer", err);
         b2rt_buffer bt = 0, bn = 0;
         uint64_t n_nodes = 0;
-        int st = b2rt_build_scene_device(c, d_triangles, n, nullptr, &bt, &bn, &n_nodes, nullptr);
+        int st = b2rt_build_scene_device(c, d_triangles, n, static_cast<uint32_t*>(d_order), &bt, &bn, &n_nodes, nullptr);
         if (st) throw CLException(std::string("Failed to build the scene on the device: ") + b2rt_last_error(c), st);
+        m_OrderBuffer = order;
         // the library has bound both buffers already; binding the same ids again changes nothing
         m_TriangleBuffer = CLBuffer::Adopt(ctx, bt, n * sizeof(CLTriangle));
         m_NodeBuffer = CLBuffer::Adopt(ctx, bn, (size_t)n_nodes * sizeof(CLLinearBVHNode));
@@ -415,6 +421,7 @@ namespace Glaze3D
         m_MaterialBuffer = CLBuffer(ctx, B2RT_MEM_READ_ONLY | B2RT_MEM_COPY_HOST_PTR, m_Materials.size() * sizeof(CLMaterial), m_Materials.data(), &err);
         if (err) throw CLException("Failed to create material buffer", err);
         eng->render->SetUniform<CLBuffer>((int)RenderKernelArgument_t::BUFFER_MATERIAL, m_MaterialBuffer);
+        m_OrderBuffer = CLBuffer();                                    // the triangles uploaded here are in scene order
     }
 
     void CLBVHScene::Refit()
@@ -428,5 +435,39 @@ namespace Glaze3D
         st = b2rt_read_buffer(c, m_NodeBuffer.id(), m_Nodes.data(), m_Nodes.size() * sizeof(CLLinearBVHNode));
         if (!st) st = b2rt_finish(c);
         if (st) throw CLException(std::string("Failed to read refitted nodes: ") + b2rt_last_error(c), st);
+    }
+
+    void CLBVHScene::RefitFromDevice(const void* d_triangles, size_t n)
+    {
+        if (!eng || !eng->render || !eng->render->m_CLContext)
+            throw CLException("CLBVHScene::RefitFromDevice needs eng->render->m_CLContext", B2RT_INVALID_CONTEXT);
+        if (!m_TriangleBuffer.id() || !m_NodeBuffer.id()) throw CLException("CLBVHScene::RefitFromDevice needs a scene on the device", B2RT_INVALID_MEM_OBJECT);
+        const CLContext& ctx = *eng->render->m_CLContext;
+        b2rt_context* c = ctx.GetContext();
+        int err = 0;
+        if (!m_RefitStatusBuffer.id()) {
+            m_RefitStatusBuffer = CLBuffer(ctx, 0, sizeof(uint32_t), nullptr, &err);
+            if (err) throw CLException("Failed to create refit status buffer", err);
+        }
+        const CLBuffer& status = m_RefitStatusBuffer;
+        void *d_status = nullptr, *d_order = nullptr;
+        err = b2rt_device_pointer(c, status.id(), &d_status, nullptr);
+        if (!err && m_OrderBuffer.id()) err = b2rt_device_pointer(c, m_OrderBuffer.id(), &d_order, nullptr);
+        if (err) throw CLException("Failed to find the refit buffers", err);
+        int st = b2rt_refit_scene_device(c, d_triangles, n, static_cast<const uint32_t*>(d_order), static_cast<uint32_t*>(d_status), nullptr);
+        if (st) throw CLException(std::string("Failed to refit scene: ") + b2rt_last_error(c), st);
+        uint32_t bits = 0;
+        st = b2rt_read_buffer(c, status.id(), &bits, sizeof(bits));
+        if (!st) st = b2rt_finish(c);
+        if (st) throw CLException(std::string("Failed to read the refit status: ") + b2rt_last_error(c), st);
+        if (bits) {
+            static const char* names[] = { "non-finite vertex positions", "a loader duplicate pair was broken (rebuild instead)",
+                                           "bounds too large to quantise", "a leaf box no longer matches its vertices",
+                                           "a triangle order entry out of range" };
+            std::string what;
+            for (int b = 0; b < 5; ++b)
+                if (bits & (1u << b)) what += (what.empty() ? "" : "; ") + std::string(names[b]);
+            throw CLException("Failed to refit scene: " + what, B2RT_INVALID_ARG_VALUE);
+        }
     }
 }
