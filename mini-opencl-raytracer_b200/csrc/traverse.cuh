@@ -10,7 +10,8 @@
 //    reference's fp32 operation order with one IEEE rounding per operation
 //    (no FMA contraction): InitRay kernel_bvh.cl:42-55, RayBounds :156-169,
 //    RayTriangle :98-153. On the device every such op is an explicit
-//    __f*_rn intrinsic, which nvcc never contracts.
+//    __f*_rn intrinsic, which nvcc never contracts, or a packed .rn.f32x2
+//    op used under the rule at "packed fp32 pairs" below.
 //  * leaves are entered in exactly the reference's DFS order (near child first
 //    by sign[axis], kernel_bvh.cl:200-207) and a leaf's triangles are tested iff
 //    the leaf's exact fp32 box passes RayBounds on [0, best]. Because a parent
@@ -188,6 +189,30 @@ extern unsigned long long g_emu_culling_violations;
 B2_HD void report_stack_overflow() { ++g_emu_stack_overflows; }
 #endif
 
+// ---- packed fp32 pairs ----------------------------------------------------------------
+// sm_100 evaluates add/sub/mul.rn.f32x2 as one FADD2 / FMUL2: two IEEE operations, each rounded on its own, in one issue
+// slot. The exact leaf path (box_gate_exact, tri_eval_exact) runs on such pairs.
+// HAZARD: ptxas contracts a mul.rn.f32x2 that feeds an add/sub.rn.f32x2 into one FFMA2 (one rounding instead of two) even
+// under -fmad=false. So the halves of a packed product are only ever combined by scalar xadd / xsub (__fadd_rn /
+// __fsub_rn, which are not contracted); packed sums may feed packed products. tests/test_packed_fp32_sass.py checks the SASS.
+#if defined(__CUDACC__)
+struct F2 { unsigned long long v; };      // one 64-bit register pair: half 0 in the low register
+B2_HD F2 pack2(float a, float b) { F2 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r.v) : "f"(a), "f"(b)); return r; }
+B2_HD float lo2(F2 p) { float a; asm("mov.b64 {%0, _}, %1;" : "=f"(a) : "l"(p.v)); return a; }
+B2_HD float hi2(F2 p) { float b; asm("mov.b64 {_, %0}, %1;" : "=f"(b) : "l"(p.v)); return b; }
+B2_HD F2 sub2(F2 a, F2 b) { F2 r; asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r.v) : "l"(a.v), "l"(b.v)); return r; }
+B2_HD F2 mul2(F2 a, F2 b) { F2 r; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r.v) : "l"(a.v), "l"(b.v)); return r; }
+#else
+// Host emulation: two scalar operations (the emulation cannot see a contraction; the SASS test does).
+struct F2 { float a, b; };
+B2_HD F2 pack2(float a, float b) { F2 r; r.a = a; r.b = b; return r; }
+B2_HD float lo2(F2 p) { return p.a; }
+B2_HD float hi2(F2 p) { return p.b; }
+B2_HD F2 sub2(F2 x, F2 y) { return pack2(xsub(x.a, y.a), xsub(x.b, y.b)); }
+B2_HD F2 mul2(F2 x, F2 y) { return pack2(xmul(x.a, y.a), xmul(x.b, y.b)); }
+#endif
+B2_HD F2 both2(float v) { return pack2(v, v); }
+
 // OpenCL max()/min() as worded by the spec ("y if x < y, otherwise x"), the
 // convention the oracle pins for NaN operands (oracle/ref_build/cl_shim.hpp).
 B2_HD float max_cl(float x, float y) { return x < y ? y : x; }
@@ -226,15 +251,16 @@ struct TravCounters { uint32_t wide_nodes, leaf_blocks, leaf_pass, tri_tests, wo
 
 // RayBounds, kernel_bvh.cl:156-169, on an exact fp32 box.
 B2_HD bool box_gate_exact(const RayX& r, float lox, float loy, float loz, float hix, float hiy, float hiz, float best) {
-    float nx = (r.sign & 1u) ? hix : lox, fx = (r.sign & 1u) ? lox : hix;
-    float ny = (r.sign & 2u) ? hiy : loy, fy = (r.sign & 2u) ? loy : hiy;
-    float nz = (r.sign & 4u) ? hiz : loz, fz = (r.sign & 4u) ? loz : hiz;
-    float t0 = max_cl(0.0f, xmul(xsub(nx, r.ox), r.ix));
-    float t1 = min_cl(best, xmul(xsub(fx, r.ox), r.ix));
-    t0 = max_cl(t0, xmul(xsub(ny, r.oy), r.iy));
-    t1 = min_cl(t1, xmul(xsub(fy, r.oy), r.iy));
-    t0 = max_cl(t0, xmul(xsub(nz, r.oz), r.iz));
-    t1 = min_cl(t1, xmul(xsub(fz, r.oz), r.iz));
+    // (near, far) planes of an axis as one pair: a packed difference feeding a packed product is not contracted
+    const F2 sx = mul2(sub2(pack2((r.sign & 1u) ? hix : lox, (r.sign & 1u) ? lox : hix), both2(r.ox)), both2(r.ix));
+    const F2 sy = mul2(sub2(pack2((r.sign & 2u) ? hiy : loy, (r.sign & 2u) ? loy : hiy), both2(r.oy)), both2(r.iy));
+    const F2 sz = mul2(sub2(pack2((r.sign & 4u) ? hiz : loz, (r.sign & 4u) ? loz : hiz), both2(r.oz)), both2(r.iz));
+    float t0 = max_cl(0.0f, lo2(sx));
+    float t1 = min_cl(best, hi2(sx));
+    t0 = max_cl(t0, lo2(sy));
+    t1 = min_cl(t1, hi2(sy));
+    t0 = max_cl(t0, lo2(sz));
+    t1 = min_cl(t1, hi2(sz));
     return t1 >= t0;
 }
 
@@ -245,23 +271,31 @@ B2_HD bool box_gate_exact(const RayX& r, float lox, float loy, float loz, float 
 // comparison is the negation the reference tests, in its order) without divergent exits.
 B2_HD bool tri_eval_exact(const RayX& r, float ax, float ay, float az, float bx, float by, float bz,
                           float cx, float cy, float cz, float& t, float& u, float& v) {
-    float e1x = xsub(bx, ax), e1y = xsub(by, ay), e1z = xsub(bz, az);
-    float e2x = xsub(cx, ax), e2y = xsub(cy, ay), e2z = xsub(cz, az);
-    float px = xsub(xmul(r.dy, e2z), xmul(r.dz, e2y));
-    float py = xsub(xmul(r.dz, e2x), xmul(r.dx, e2z));
-    float pz = xsub(xmul(r.dx, e2y), xmul(r.dy, e2x));
-    float det = xadd(xadd(xmul(e1x, px), xmul(e1y, py)), xmul(e1z, pz));
+    // x and y of every vector form one pair (a vertex's x, y arrive adjacent from one 128-bit load), z stays scalar;
+    // cross and dot products are FMUL2 whose halves are combined by scalar adds (see HAZARD)
+    const F2 a = pack2(ax, ay), d = pack2(r.dx, r.dy);
+    const F2 e1 = sub2(pack2(bx, by), a), e2 = sub2(pack2(cx, cy), a);
+    const float e1z = xsub(bz, az), e2z = xsub(cz, az);
+    const F2 m1 = mul2(d, both2(e2z)), m2 = mul2(e2, both2(r.dz)), m3 = mul2(d, pack2(hi2(e2), lo2(e2)));
+    const F2 p = pack2(xsub(hi2(m1), hi2(m2)), xsub(lo2(m2), lo2(m1)));     // px = dy e2z - dz e2y, py = dz e2x - dx e2z
+    const float pz = xsub(lo2(m3), hi2(m3));                                  // dx e2y - dy e2x
+    const F2 m4 = mul2(e1, p);
+    const float det = xadd(xadd(lo2(m4), hi2(m4)), xmul(e1z, pz));
     bool ok = !(det < 1.0e-8f) && !(-det > 1.0e-8f);                                   // :116
-    float inv = xdiv(1.0f, det);
-    float tx = xsub(r.ox, ax), ty = xsub(r.oy, ay), tz = xsub(r.oz, az);
-    u = xmul(xadd(xadd(xmul(tx, px), xmul(ty, py)), xmul(tz, pz)), inv);
+    const float inv = xdiv(1.0f, det);
+    const F2 s = sub2(pack2(r.ox, r.oy), a);
+    const float sz = xsub(r.oz, az);
+    const F2 m5 = mul2(s, p);
+    u = xmul(xadd(xadd(lo2(m5), hi2(m5)), xmul(sz, pz)), inv);
     ok = ok && !(u < 0.0f) && !(u > 1.0f);                                             // :125
-    float qx = xsub(xmul(ty, e1z), xmul(tz, e1y));
-    float qy = xsub(xmul(tz, e1x), xmul(tx, e1z));
-    float qz = xsub(xmul(tx, e1y), xmul(ty, e1x));
-    v = xmul(xadd(xadd(xmul(r.dx, qx), xmul(r.dy, qy)), xmul(r.dz, qz)), inv);
+    const F2 m6 = mul2(s, both2(e1z)), m7 = mul2(e1, both2(sz)), m8 = mul2(s, pack2(hi2(e1), lo2(e1)));
+    const F2 q = pack2(xsub(hi2(m6), hi2(m7)), xsub(lo2(m7), lo2(m6)));     // qx = sy e1z - sz e1y, qy = sz e1x - sx e1z
+    const float qz = xsub(lo2(m8), hi2(m8));                                  // sx e1y - sy e1x
+    const F2 m9 = mul2(d, q);
+    v = xmul(xadd(xadd(lo2(m9), hi2(m9)), xmul(r.dz, qz)), inv);
     ok = ok && !(v < 0.0f) && !(xadd(u, v) > 1.0f);                                    // :132
-    t = xmul(xadd(xadd(xmul(e2x, qx), xmul(e2y, qy)), xmul(e2z, qz)), inv);
+    const F2 m10 = mul2(e2, q);
+    t = xmul(xadd(xadd(lo2(m10), hi2(m10)), xmul(e2z, qz)), inv);
     return ok;
 }
 B2_HD void tri_test_exact(const RayX& r, float ax, float ay, float az, float bx, float by, float bz,
