@@ -130,7 +130,8 @@ enum {
     B2RT_OPT_RESUME_MAX = 11,   /* two-step tail: a dry warp with at most this many live rays suspends them; a second persistent launch
                                    re-packs all suspended rays 32 to a warp and walks on at full width, and only what that pass
                                    leaves (B2RT_OPT_COOP_MAX per warp) goes to the cooperative kernel. 0 = off (default, also -1) .. 16.
-                                   Only used while larger than the cooperative threshold. Results do not depend on it. */
+                                   Only used while larger than the cooperative threshold. Results do not depend on it. Ignored by
+                                   b2rt_trace_multi[_device]. */
     B2RT_OPT_TAIL_HELP = 12,    /* 1 (default) / 0: in a library built with -DB2_TAIL_HELP=1, warps of a persistent traversal launch that have
                                    finished or handed over their own rays serve the cooperative tail queue inside the same launch; the
                                    tail kernel takes what is left. The default build compiles this out (measured slower on frame shares,
@@ -142,7 +143,7 @@ enum {
     B2RT_OPT_COOP_MAX = 7       /* tail mode of the persistent kernels: a warp whose ray pool is dry and that has at most this many
                                    rays alive hands them to the cooperative tail kernel, 32 lanes per ray (0 = off .. 16; default -1 = 8, but off for scenes
                                    of fewer than ~1000 nodes, whose rays are too short to gain). Results do not
-                                   depend on it. */
+                                   depend on it. Ignored by b2rt_trace_multi[_device], whose launches have no cooperative tail. */
 };
 
 /* ---- lifetime ---------------------------------------------------------------------- */
@@ -280,6 +281,30 @@ int b2rt_trace_any(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, uint32_t
  * queue of the stream that has not launched for longest. */
 int b2rt_trace_closest_device(b2rt_context* ctx, const b2rt_ray* d_rays, uint64_t n, b2rt_hit* d_hits, void* cuda_stream);
 int b2rt_trace_any_device(b2rt_context* ctx, const b2rt_ray* d_rays, uint64_t n, uint32_t* d_occluded, void* cuda_stream);
+
+/* The k nearest hits per ray (new). Intersect() (kernel_bvh.cl:171-219) with isect replaced by a list of at most k hits:
+ *  - the walk is the reference's depth-first order; a leaf is entered iff its exact fp32 box passes RayBounds on
+ *    [0, bound], where bound = tmax while the list holds fewer than k hits and the t of its k-th entry once it is full;
+ *  - a triangle is accepted iff RayTriangle accepts it with t < bound: the acceptance rule of b2rt_trace_closest (no lower
+ *    bound on t, tmin ignored, front faces only). The bound is updated after every insertion, also between the triangles
+ *    of one leaf;
+ *  - an accepted hit is inserted after every entry with t <= its own (equal t keeps visiting order, like the reference's
+ *    strict <); a full list drops its last entry;
+ *  - the ray ends when bound < 0 (no later box can pass);
+ *  - row i of the output is hits[i*k .. i*k+k), sorted by t; unused slots are {t = tmax, u = 0, v = 0, tri = B2RT_MISS}.
+ * Every triangle of the scene array is its own hit: the loader's two copies of a face (SURVEY.md A-6) appear as two hits,
+ * usually at the same t. With k = 1 every row is bit-identical to what b2rt_trace_closest returns, misses included.
+ * k = 0 or k > B2RT_MULTI_MAX_HITS, or a NULL pointer with n > 0, returns B2RT_INVALID_VALUE and writes nothing; n = 0
+ * succeeds and does nothing.
+ * b2rt_trace_multi: host buffers, synchronous (pipelined in chunks like b2rt_trace_closest; a chunk holds fewer rays for
+ * larger k). On a b2rt_create_multi handle the rays are cut into contiguous ranges, one per device.
+ * b2rt_trace_multi_device: device buffers (d_hits = b2rt_hit[n * k]), asynchronous on cuda_stream with the stream rules of
+ * b2rt_trace_closest_device; on a b2rt_create_multi handle it runs on the root.
+ * B2RT_OPT_TRAVERSAL = 1 runs the query through the reference-layout walk, B2RT_OPT_COUNTERS = 1 through the counting
+ * build. These launches have no cooperative tail: B2RT_OPT_COOP_MAX and B2RT_OPT_RESUME_MAX are accepted and ignored. */
+#define B2RT_MULTI_MAX_HITS 64
+int b2rt_trace_multi(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, uint32_t k, b2rt_hit* hits);
+int b2rt_trace_multi_device(b2rt_context* ctx, const b2rt_ray* d_rays, uint64_t n, uint32_t k, b2rt_hit* d_hits, void* cuda_stream);
 /* CreateRay (kernel_bvh.cl:386-403) for gid in [gid_begin, gid_end) with the currently bound
  * WIDTH/HEIGHT/FRAME_COUNT/CAMERA_* arguments, written to device memory as b2rt_ray. */
 int b2rt_camera_rays_device(b2rt_context* ctx, size_t gid_begin, size_t gid_end, b2rt_ray* d_rays, void* cuda_stream);
@@ -293,7 +318,7 @@ int b2rt_camera_rays_device(b2rt_context* ctx, size_t gid_begin, size_t gid_end,
  *    devices; each device keeps the running average of ITS pixels and stores every finished pixel through to the root's
  *    image over a peer mapping, so b2rt_read_buffer / b2rt_read_pixels after it return the complete frame (the root's
  *    stream waits for all devices);
- *  - b2rt_trace_closest / b2rt_trace_any cut the host ray stream into contiguous ranges, one per device;
+ *  - b2rt_trace_closest / b2rt_trace_any / b2rt_trace_multi cut the host ray stream into contiguous ranges, one per device;
  *  - the *_device entry points, b2rt_build_bvh and b2rt_execute_bands address one device: the root
  *    (b2rt_build_scene_device builds there and copies the scene to every device).
  * n_devices == 1 gives an ordinary handle. CLRaytracer code written against the single-device calls runs unchanged. */

@@ -29,8 +29,9 @@ SYMBOLS = [
     "b2rt_get_counters", "b2rt_reset_counters", "b2rt_launch_count", "b2rt_device_count",
     "b2rt_create_multi", "b2rt_group_size", "b2rt_group_info", "b2rt_comm_unique_id", "b2rt_comm_init", "b2rt_comm_share_output",
     "b2rt_execute_shard", "b2rt_shard_bands", "b2rt_refit_scene", "b2rt_stage_times",
-    "b2rt_build_scene_device", "b2rt_refit_scene_device",
+    "b2rt_build_scene_device", "b2rt_refit_scene_device", "b2rt_trace_multi", "b2rt_trace_multi_device",
 ]
+MULTI_MAX_HITS = 64          # B2RT_MULTI_MAX_HITS: largest k of b2rt_trace_multi
 # status bits of b2rt_refit_scene_device
 REFIT_NONFINITE, REFIT_DUPLICATE, REFIT_RANGE, REFIT_LEAF_BOX, REFIT_ORDER = 1, 2, 4, 8, 16
 
@@ -97,6 +98,8 @@ def lib():
         "b2rt_trace_any": (C.c_int, [vp, vp, u64, vp]),
         "b2rt_trace_closest_device": (C.c_int, [vp, vp, u64, vp, vp]),
         "b2rt_trace_any_device": (C.c_int, [vp, vp, u64, vp, vp]),
+        "b2rt_trace_multi": (C.c_int, [vp, vp, u64, u32, vp]),
+        "b2rt_trace_multi_device": (C.c_int, [vp, vp, u64, u32, vp, vp]),
         "b2rt_camera_rays_device": (C.c_int, [vp, sz, sz, vp, vp]),
         "b2rt_device_pointer": (C.c_int, [vp, u64, C.POINTER(vp), C.POINTER(sz)]),
         "b2rt_bound_buffer": (C.c_int, [vp, u32, C.POINTER(u64)]),
@@ -400,6 +403,19 @@ class Context:
             occluded = np.empty(rays.shape[0], dtype=np.uint32)
         self._ck(self._L.b2rt_trace_any(self._h, _ptr(rays), rays.shape[0], _ptr(occluded)))
         return occluded
+
+    def trace_multi(self, rays, k):
+        """The k nearest hits of every ray (b2rt_trace_multi): an (n, k) HIT_DTYPE array, each row sorted by t and
+        padded with {tmax, 0, 0, MISS}."""
+        rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
+        hits = np.empty((rays.shape[0], max(int(k), 0)), dtype=HIT_DTYPE)
+        self._ck(self._L.b2rt_trace_multi(self._h, _ptr(rays), rays.shape[0], int(k), _ptr(hits)))
+        return hits
+
+    def trace_multi_device(self, d_rays, n, k, d_hits, stream=0):
+        """b2rt_trace_multi_device: d_hits holds n * k records of 16 bytes."""
+        self._ck(self._L.b2rt_trace_multi_device(self._h, C.c_void_p(int(d_rays)), int(n), int(k), C.c_void_p(int(d_hits)),
+                                                 C.c_void_p(int(stream))))
 
     def trace_closest_device(self, d_rays, n, d_hits, stream=0):
         self._ck(self._L.b2rt_trace_closest_device(self._h, C.c_void_p(int(d_rays)), int(n), C.c_void_p(int(d_hits)),

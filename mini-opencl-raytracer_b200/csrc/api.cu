@@ -302,17 +302,19 @@ static int binary_walk_fits(b2rt_context* ctx) {
     return fail(ctx, B2RT_OUT_OF_RESOURCES, "BVH too deep for the reference-layout walk's stack (binary depth " + std::to_string(ctx->info.max_depth_binary) + ")");
 }
 
-int trace_device(b2rt_context* ctx, const void* d_rays, uint64_t n, void* d_out, bool any, cudaStream_t st) {
+// k > 0: the k nearest hits per ray (b2rt_trace_multi), d_out = b2rt_hit[n * k]; `any` is then ignored.
+int trace_device(b2rt_context* ctx, const void* d_rays, uint64_t n, void* d_out, bool any, cudaStream_t st, uint32_t k = 0) {
     if (n == 0) return B2RT_SUCCESS;
     if (!d_rays || !d_out) return fail(ctx, B2RT_INVALID_VALUE, "null ray or output pointer");
     if (ctx->opt_traversal == 1) {
         int fits = binary_walk_fits(ctx);
         if (fits) return fits;
-        CK(launch_trace_binary(ctx->view, d_rays, n, d_out, any, ctx->info.max_depth_binary, st));
+        if (k) CK(launch_trace_binary_multi(ctx->view, d_rays, n, k, d_out, ctx->info.max_depth_binary, st));
+        else CK(launch_trace_binary(ctx->view, d_rays, n, d_out, any, ctx->info.max_depth_binary, st));
         ctx->launches += 1;
         return B2RT_SUCCESS;
     }
-    int grid = any ? ctx->grid_any : ctx->grid_closest;
+    int grid = (any && !k) ? ctx->grid_any : ctx->grid_closest;
     if (ctx->opt_blocks_per_sm > 0) grid = ctx->sm_count * (int)ctx->opt_blocks_per_sm;
     uint64_t warps_needed = (n + 31) / 32, blocks_needed = (warps_needed * 32 + trace_block_threads() - 1) / trace_block_threads();
     if ((uint64_t)grid > blocks_needed) grid = (int)blocks_needed;
@@ -322,6 +324,14 @@ int trace_device(b2rt_context* ctx, const void* d_rays, uint64_t n, void* d_out,
     if (st_pol) return st_pol;
     const uint64_t seq = ctx->next_seq++;
     unsigned long long* next = ctx->d_next + 8 * (seq % NEXT_RING);
+    if (k) {
+        // no cooperative tail: the tail hand-over would need the row list in its record (B2RT_OPT_COOP_MAX and
+        // B2RT_OPT_RESUME_MAX do not apply)
+        CK(launch_trace_multi(ctx->view, d_rays, n, k, d_out, ctx->opt_counters != 0, ctx->stack_bound, grid, next, ctx->d_counters,
+                              (uint32_t)ctx->opt_refill_min, (uint32_t)(ctx->opt_leaf_bias ? ctx->opt_leaf_bias : 32), st));
+        ctx->launches += 1;
+        return B2RT_SUCCESS;
+    }
     // Tail queues go with the STREAM: launches on one stream are ordered, so they share a queue (allocated by the first of
     // them -- r2: round robin made each of a handle's first four launches pay a 100 MB cudaMalloc, two of them inside a timed
     // region of bench.py); launches on up to TAIL_RING different streams may overlap (documented in b2rt.h), a further
@@ -346,25 +356,29 @@ int trace_device(b2rt_context* ctx, const void* d_rays, uint64_t n, void* d_out,
     return B2RT_SUCCESS;
 }
 
-int ensure_staging(b2rt_context* ctx, uint64_t chunk) {
-    if (ctx->stage_capacity >= chunk) return B2RT_SUCCESS;
+int ensure_staging(b2rt_context* ctx, uint64_t chunk, size_t out_bytes) {
+    if (ctx->stage_capacity >= chunk && ctx->stage_out_bytes >= out_bytes) return B2RT_SUCCESS;
+    chunk = std::max(chunk, ctx->stage_capacity);
+    out_bytes = std::max(out_bytes, ctx->stage_out_bytes);
     for (int i = 0; i < 2; ++i) {
         if (ctx->d_stage_rays[i]) cudaFree(ctx->d_stage_rays[i]);
         if (ctx->d_stage_out[i]) cudaFree(ctx->d_stage_out[i]);
         ctx->d_stage_rays[i] = ctx->d_stage_out[i] = nullptr;
     }
     ctx->stage_capacity = 0;
+    ctx->stage_out_bytes = 0;
     for (int i = 0; i < 2; ++i) {
         CK(cudaMalloc(&ctx->d_stage_rays[i], chunk * sizeof(b2rt_ray)));
-        CK(cudaMalloc(&ctx->d_stage_out[i], chunk * sizeof(b2rt_hit)));
+        CK(cudaMalloc(&ctx->d_stage_out[i], out_bytes));
     }
     ctx->stage_capacity = chunk;
+    ctx->stage_out_bytes = out_bytes;
     return B2RT_SUCCESS;
 }
 
 // Host-buffer ray stream: chunks are copied in, traced and copied out on three streams so
-// that PCIe transfers overlap the traversal kernels.
-int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any) {
+// that PCIe transfers overlap the traversal kernels. k > 0: k hits per ray (see trace_device).
+int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any, uint32_t k) {
     int st = use_device(ctx);
     if (st) return st;
     st = ensure_scene(ctx);
@@ -373,26 +387,28 @@ int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, b
     if (!rays || !out) return fail(ctx, B2RT_INVALID_VALUE, "null ray or output pointer");
     uint64_t chunk_rays = STREAM_CHUNK;
     if (const char* env = getenv("B2RT_STREAM_CHUNK")) { long long v = atoll(env); if (v >= 1024) chunk_rays = (uint64_t)v; }   // tuning aid
+    // k hits per ray: the chunk shrinks with k, so that the output staging stays that of a closest-hit chunk
+    if (k > 1) chunk_rays = std::max<uint64_t>(chunk_rays / k, 1024);
     uint64_t chunk = std::min<uint64_t>(n, chunk_rays);
-    st = ensure_staging(ctx, chunk);
+    const size_t out_elem = k ? (size_t)k * sizeof(b2rt_hit) : (any ? sizeof(uint32_t) : sizeof(b2rt_hit));
+    st = ensure_staging(ctx, chunk, chunk * std::max(out_elem, sizeof(b2rt_hit)));
     if (st) return st;
-    const size_t out_elem = any ? sizeof(uint32_t) : sizeof(b2rt_hit);
     // Chunk sizes ramp up from `ramp` to `chunk` and back down at the end: the first copy-in and the last kernel +
     // copy-out are the only parts of the pipeline that nothing overlaps, so they are kept short.
     const uint64_t ramp = std::min<uint64_t>(chunk, 1ull << 19);
-    uint64_t k = 0, m = 0;
-    for (uint64_t off = 0; off < n; off += m, ++k) {
-        int s = (int)(k & 1);
+    uint64_t c = 0, m = 0;
+    for (uint64_t off = 0; off < n; off += m, ++c) {
+        int s = (int)(c & 1);
         const uint64_t left = n - off;
-        m = std::min<uint64_t>(chunk, ramp << std::min<uint64_t>(k, 16));                              // ramp up
+        m = std::min<uint64_t>(chunk, ramp << std::min<uint64_t>(c, 16));                              // ramp up
         if (left <= ramp) m = left;
         else m = std::min<uint64_t>(m, std::max<uint64_t>(ramp, (left / 2 + 31) & ~31ull));            // ramp down: at most half of what is left
-        if (k >= 2) CK(cudaStreamWaitEvent(ctx->stream_in, ctx->ev_comp[s], 0));     // rays[s] free again
+        if (c >= 2) CK(cudaStreamWaitEvent(ctx->stream_in, ctx->ev_comp[s], 0));     // rays[s] free again
         CK(cudaMemcpyAsync(ctx->d_stage_rays[s], rays + off, m * sizeof(b2rt_ray), cudaMemcpyHostToDevice, ctx->stream_in));
         CK(cudaEventRecord(ctx->ev_in[s], ctx->stream_in));
         CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[s], 0));
-        if (k >= 2) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[s], 0));         // out[s] drained
-        st = trace_device(ctx, ctx->d_stage_rays[s], m, ctx->d_stage_out[s], any, ctx->stream);
+        if (c >= 2) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[s], 0));         // out[s] drained
+        st = trace_device(ctx, ctx->d_stage_rays[s], m, ctx->d_stage_out[s], any, ctx->stream, k);
         if (st) return st;
         CK(cudaEventRecord(ctx->ev_comp[s], ctx->stream));
         CK(cudaStreamWaitEvent(ctx->stream_out, ctx->ev_comp[s], 0));
@@ -1170,6 +1186,30 @@ extern "C" int b2rt_trace_any_device(b2rt_context* ctx, const b2rt_ray* d_rays, 
     st = ensure_scene(ctx);
     if (st) return st;
     return trace_device(ctx, d_rays, n, d_occluded, true, cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream);
+}
+// k nearest hits: k in [1, B2RT_MULTI_MAX_HITS] and no NULL pointer with n > 0, checked before anything is touched.
+static int multi_args(b2rt_context* ctx, const void* rays, uint64_t n, uint32_t k, const void* hits) {
+    if (k == 0 || k > B2RT_MULTI_MAX_HITS) return fail(ctx, B2RT_INVALID_VALUE, "k must be 1.." + std::to_string(B2RT_MULTI_MAX_HITS));
+    if (n && (!rays || !hits)) return fail(ctx, B2RT_INVALID_VALUE, "null ray or output pointer");
+    if (n > (1ull << 56) / k) return fail(ctx, B2RT_INVALID_VALUE, "ray count too large");
+    return B2RT_SUCCESS;
+}
+extern "C" int b2rt_trace_multi(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, uint32_t k, b2rt_hit* hits) {
+    if (!ctx) return B2RT_INVALID_CONTEXT;
+    int st = multi_args(ctx, rays, n, k, hits);
+    if (st) return st;
+    if (ctx->group) return group_trace_host(ctx, rays, n, hits, false, k);   // contiguous ranges, one per device
+    return trace_host(ctx, rays, n, hits, false, k);
+}
+extern "C" int b2rt_trace_multi_device(b2rt_context* ctx, const b2rt_ray* d_rays, uint64_t n, uint32_t k, b2rt_hit* d_hits, void* cuda_stream) {
+    if (!ctx) return B2RT_INVALID_CONTEXT;
+    int st = multi_args(ctx, d_rays, n, k, d_hits);
+    if (st) return st;
+    st = use_device(ctx);
+    if (st) return st;
+    st = ensure_scene(ctx);
+    if (st) return st;
+    return trace_device(ctx, d_rays, n, d_hits, false, cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream, k);
 }
 extern "C" int b2rt_camera_rays_device(b2rt_context* ctx, size_t gid_begin, size_t gid_end, b2rt_ray* d_rays, void* cuda_stream) {
     if (!ctx) return B2RT_INVALID_CONTEXT;

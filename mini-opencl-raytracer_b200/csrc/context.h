@@ -69,7 +69,8 @@ struct b2rt_context {
     unsigned long long* d_counters = nullptr;
     void* d_stage_rays[2] = { nullptr, nullptr };
     void* d_stage_out[2] = { nullptr, nullptr };
-    uint64_t stage_capacity = 0;
+    uint64_t stage_capacity = 0;               // rays per staging buffer ...
+    size_t stage_out_bytes = 0;                // ... and bytes per output staging buffer
     // wavefront frame path: two ray queues, hits, per-path state, three rotating queue counters
     void* d_wf_rays[2] = { nullptr, nullptr };
     void *d_wf_hits = nullptr, *d_wf_state = nullptr;
@@ -130,7 +131,7 @@ int install_scene(b2rt_context* ctx, const DerivedScene& d);
 // refit.cu: per-triangle shading records (normals + material) of `tris`
 cudaError_t launch_shade_records(b2rt::ShadeTri* shade, const b2rt::RefTriangle* tris, uint32_t n, cudaStream_t s);
 int render_items(b2rt_context* ctx, const b2rt::GidMap& map, uint64_t n);
-int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any);
+int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any, uint32_t k = 0);   // k > 0: k hits per ray
 
 // multi.cu
 void group_destroy(b2rt_context* ctx);
@@ -139,7 +140,7 @@ int group_buffer_create(b2rt_context* ctx, uint32_t flags, size_t bytes, const v
 int group_each(b2rt_context* ctx, int (*fn)(b2rt_context*, void*), void* arg, bool parallel);
 int group_adopt_scene(b2rt_context* root);
 int group_execute(b2rt_context* ctx, size_t gid_begin, size_t gid_end);
-int group_trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any);
+int group_trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any, uint32_t hits_per_ray = 0);   // > 0: b2rt_trace_multi
 int group_finish(b2rt_context* ctx);
 void group_bind_output(b2rt_context* ctx);
 int group_broadcast_buffer(b2rt_context* ctx, b2rt_buffer id);   // the root's contents of buffer `id` to every peer's copy

@@ -1,14 +1,16 @@
 // kernels.cu -- hand-written sm_100a kernels behind libb2rt.so.
 //
-//  trace_persistent<ANY,COUNT,CAP>  persistent-thread while-while traversal of the
+//  trace_persistent<P,COUNT,CAP>    persistent-thread while-while traversal of the
 //      compressed wide BVH for a ray stream: one grid of (SMs x blocks/SM) CTAs,
 //      every warp pulls chunks of rays from a global atomic counter into a
 //      warp-local pool, idle lanes are re-filled from the pool with ballot/popc
 //      compaction, interior-node steps and leaf steps run in separate
-//      warp-uniform loops, all node/leaf fetches are 128-bit __ldg.
+//      warp-uniform loops, all node/leaf fetches are 128-bit __ldg. P is the hit policy
+//      (traverse.cuh): closest hit, any hit, or the k nearest hits per ray.
 //  trace_binary_kernel<ANY,CAP>     one thread per ray over the reference's own
 //      48 B / 256 B arrays in the reference's order: the "recompiled reference
-//      kernel" baseline and an on-device cross-check of the wide path.
+//      kernel" baseline and an on-device cross-check of the wide path;
+//      trace_binary_multi_kernel<CAP> the same walk keeping the k nearest hits.
 //  camera_rays_kernel               CreateRay (kernel_bvh.cl:386-403) as a ray stream.
 //  wf_generate_kernel / wf_shade_kernel   KernelEntry (kernel_bvh.cl:415-456) as a wavefront:
 //      camera rays + path state, then per bounce trace_persistent over the live ray queue and
@@ -78,6 +80,13 @@ __device__ __forceinline__ void write_result(void* __restrict__ out, uint64_t i,
     if (ANY) reinterpret_cast<uint32_t*>(out)[i] = (h.tri != 0xFFFFFFFFu) ? 1u : 0u;
     else reinterpret_cast<float4*>(out)[i] = make_float4(h.t, h.u, h.v, __uint_as_float(h.tri));
 #endif
+}
+
+// A finished ray of a trace_persistent<P> launch: its hit, occlusion flag, or (HIT_MULTI) the padding of its row of k hits.
+template <int P>
+__device__ __forceinline__ void finish_ray(void* __restrict__ out, uint64_t i, const HitX& h, uint32_t k) {
+    if (P == HIT_MULTI) pad_row(reinterpret_cast<HitX*>(out) + i * k, k, h);
+    else write_result<P == HIT_ANY>(out, i, h);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -238,13 +247,16 @@ enum { WARP_SMEM_WORDS = (B2_SMEM_STACK + (B2_STAGE_RAYS ? STAGE_WORDS : 0)) * 3
 // issued instructions have many active lanes even though rays are incoherent. Finished lanes are
 // re-filled from a warp-local pool of ray indices (ballot + popc compaction) that is topped up
 // from one global atomic counter, `chunk` rays at a time.
+// HIT_MULTI (k hits per ray, out = HitX[n * k]): each lane keeps its ray's list in the ray's own output row; such launches
+// have no cooperative tail and no two-step resume (a dry warp stays until every lane is idle), k is a launch argument.
 // ---------------------------------------------------------------------------------------
-template <bool ANY, bool COUNT, int CAP>
+template <int P, bool COUNT, int CAP>
 __global__ void __launch_bounds__(TRACE_BLOCK, B2_MIN_BLOCKS)
 trace_persistent(SceneView s, const RayIn* __restrict__ rays, uint64_t n, void* __restrict__ out,
                  unsigned long long* __restrict__ next, unsigned long long* __restrict__ counters, uint32_t chunk,
                  uint32_t refill_min, uint32_t leaf_bias, const unsigned long long* __restrict__ n_dev, TailQueue tail,
-                 const uint32_t* __restrict__ resume) {
+                 const uint32_t* __restrict__ resume, uint32_t k) {
+    constexpr bool ANY = P == HIT_ANY, MULTI = P == HIT_MULTI;
     // resume != null: the "rays" of this launch are the hand-over records of a previous one (n_dev = their count): every
     // lane picks a suspended ray up where its first owner left it
     const unsigned lane = threadIdx.x & 31u;
@@ -258,7 +270,7 @@ trace_persistent(SceneView s, const RayIn* __restrict__ rays, uint64_t n, void* 
 #if B2_TAIL_CODE && B2_TAIL_HELP
     if (tail.help_fcap && lane == 0) atomicAdd(tail.handed + 1, 1ull);           // "started", see the helping epilogue
 #endif
-    Lane<ANY, COUNT, CAP> L;
+    Lane<P, COUNT, CAP> L;
     uint32_t local_stack[CAP];
     // One contiguous piece of shared memory per warp: [stack entry][lane] columns, then the staged rays; the whole piece is
     // the frontier of a helping warp once its own rays are done (epilogue).
@@ -306,12 +318,12 @@ trace_persistent(SceneView s, const RayIn* __restrict__ rays, uint64_t n, void* 
             // ---- refill idle lanes from the warp pool -------------------------------------------
             // Finished rays are written here, several lanes at a time, instead of one lane at a time when they finish.
             const unsigned idle = ~busy;
-            if (has_out) { write_result<ANY>(out, my_index, L.h); has_out = 0; }
+            if (has_out) { finish_ray<P>(out, my_index, L.h, k); has_out = 0; }
             if (pool_left == 0u) {
                 unsigned long long base = 0;
                 if (lane == 0) base = atomicAdd(next, (unsigned long long)chunk);
                 base = __shfl_sync(FULL, base, 0);
-                if (base >= n) { pool_left = POOL_DRY; leave_at = B2_TAIL_CODE ? 32u - (tail.coop_max < 31u ? tail.coop_max : 31u) : 32u; continue; }
+                if (base >= n) { pool_left = POOL_DRY; leave_at = (B2_TAIL_CODE && !MULTI) ? 32u - (tail.coop_max < 31u ? tail.coop_max : 31u) : 32u; continue; }
                 pool_next = base;
                 pool_left = (base + chunk < n) ? chunk : (uint32_t)(n - base);
             }
@@ -367,7 +379,7 @@ trace_persistent(SceneView s, const RayIn* __restrict__ rays, uint64_t n, void* 
                         load_ray(rays, my_index, r, tmax);
                         L.start(r, tmax);
                         if (resume) {
-                            const ResumeState o = resume_fetch<Lane<ANY, COUNT, CAP>>(local_stack, rec);
+                            const ResumeState o = resume_fetch<Lane<P, COUNT, CAP>>(local_stack, rec);
                             L.h.t = o.t; L.h.u = o.u; L.h.v = o.v; L.h.tri = o.tri;
                             L.cur = o.cur; L.leaf0 = o.leaf0; L.leaf1 = o.leaf1; L.top = o.top; L.sp = o.sp;
 #if B2_SMEM_STACK
@@ -411,7 +423,7 @@ trace_persistent(SceneView s, const RayIn* __restrict__ rays, uint64_t n, void* 
         } else {
             if (COUNT) { ph_leaf++; ph_leaf_lanes += __popc(vl); }
             stepped = L.wants_leaf();
-            if (stepped) L.leaf_step(s.leaf, stack);
+            if (stepped) L.leaf_step(s.leaf, stack, MULTI ? reinterpret_cast<HitX*>(out) + my_index * k : nullptr, k);
         }
 #if B2_TOUCH
         if (stepped) {
@@ -425,9 +437,9 @@ trace_persistent(SceneView s, const RayIn* __restrict__ rays, uint64_t n, void* 
             if (COUNT) { traced++; max_ray_steps = max_ray_steps > ray_steps ? max_ray_steps : ray_steps; ray_steps = 0; }
         }
     }
-    if (has_out) write_result<ANY>(out, my_index, L.h);       // rays that finished after the last refill
+    if (has_out) finish_ray<P>(out, my_index, L.h, k);       // rays that finished after the last refill
     // at most coop_max lanes per warp get here, and the queue holds coop_max records per warp of the grid
-    if (B2_TAIL_CODE && tail.coop_max && !L.done()) {
+    if (B2_TAIL_CODE && !MULTI && tail.coop_max && !L.done()) {
 #if B2_SMEM_STACK
         for (int i = 0; i < L.sp && i < B2_SMEM_STACK; ++i) local_stack[i] = stk_get(stack, i);      // the record wants one plain array
 #endif
@@ -441,7 +453,7 @@ trace_persistent(SceneView s, const RayIn* __restrict__ rays, uint64_t n, void* 
     // work, started while the queue is still filling. It leaves when every warp of the grid is past its hand-over and the
     // queue is empty, or after B2_HELP_POLLS empty polls: no unbounded wait, so nothing depends on the whole grid being
     // resident; whatever is left in the queue is the tail kernel's, as before.
-    if (tail.coop_max && tail.help_fcap) {
+    if (!MULTI && tail.coop_max && tail.help_fcap) {
         __syncwarp();
         TailStats ts;
         tail_stats_clear(ts);
@@ -511,11 +523,14 @@ trace_persistent(SceneView s, const RayIn* __restrict__ rays, uint64_t n, void* 
 // Reference-layout binary walk (kernel_bvh.cl:171-219 verbatim semantics), except for the stack: the reference's is
 // int[64] and unchecked, so on a tree deeper than 64 levels it writes past its end. This one has CAP entries, CAP at least
 // the tree's binary depth (the walk holds at most one entry per level of the current path), like the oracle's growing stack.
+// P = HIT_MULTI: the k nearest hits go to `row` (h holds the list's state, traverse.cuh); the caller pads the row.
 // ---------------------------------------------------------------------------------------
-template <bool ANY, int CAP>
+template <int P, int CAP>
 __device__ __forceinline__ HitX trace_binary(const RefTriangle* __restrict__ tris, const RefNode* __restrict__ nodes,
-                                             const RayX& r, float tmax) {
+                                             const RayX& r, float tmax, HitX* row = nullptr, uint32_t k = 0) {
+    constexpr bool ANY = P == HIT_ANY;
     HitX h; h.t = tmax; h.u = 0.0f; h.v = 0.0f; h.tri = 0xFFFFFFFFu;
+    if (P == HIT_MULTI) { h.u = tmax; h.tri = 0u; }
     uint32_t stack[CAP];
     int sp = 0;
     uint32_t cur = 0;
@@ -530,7 +545,8 @@ __device__ __forceinline__ HitX trace_binary(const RefTriangle* __restrict__ tri
                 for (uint32_t i = 0; i < nprim; ++i) {
                     const float4* tp = reinterpret_cast<const float4*>(tris + tail.x + i);
                     float4 a = __ldg(tp), b = __ldg(tp + 5), c = __ldg(tp + 10);   // positions at +0, +80, +160 B
-                    tri_test_exact(r, a.x, a.y, a.z, b.x, b.y, b.z, c.x, c.y, c.z, tail.x + i, h);
+                    if (P == HIT_MULTI) tri_test_multi(r, a.x, a.y, a.z, b.x, b.y, b.z, c.x, c.y, c.z, tail.x + i, h, row, k);
+                    else tri_test_exact(r, a.x, a.y, a.z, b.x, b.y, b.z, c.x, c.y, c.z, tail.x + i, h);
                 }
                 if (ANY && h.tri != 0xFFFFFFFFu) break;
             } else {
@@ -559,6 +575,17 @@ trace_binary_kernel(SceneView s, const RayIn* __restrict__ rays, uint64_t n, voi
     HitX h = trace_binary<ANY, CAP>(s.tris, s.nodes, r, tmax);
     if (ANY) reinterpret_cast<uint32_t*>(out)[i] = (h.tri != 0xFFFFFFFFu) ? 1u : 0u;
     else reinterpret_cast<float4*>(out)[i] = make_float4(h.t, h.u, h.v, __uint_as_float(h.tri));
+}
+
+template <int CAP>
+__global__ void __launch_bounds__(128)
+trace_binary_multi_kernel(SceneView s, const RayIn* __restrict__ rays, uint64_t n, HitX* __restrict__ out, uint32_t k) {
+    uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    RayX r; float tmax;
+    load_ray(rays, i, r, tmax);
+    HitX* row = out + i * k;
+    pad_row(row, k, trace_binary<HIT_MULTI, CAP>(s.tris, s.nodes, r, tmax, row, k));
 }
 
 // ---------------------------------------------------------------------------------------
@@ -729,21 +756,21 @@ tonemap_rgba8_kernel(const float4* __restrict__ image, uchar4* __restrict__ out,
 // ---------------------------------------------------------------------------------------
 static int pick_cap(uint32_t bound) { return bound <= 32 ? 32 : (bound <= 64 ? 64 : (bound <= 128 ? 128 : (bound <= 256 ? 256 : 0))); }
 
-template <bool ANY, bool COUNT>
+template <int P, bool COUNT>
 static cudaError_t launch_persistent_cap(int cap, int grid, cudaStream_t st, const SceneView& s, const void* rays,
                                          uint64_t n, void* out, unsigned long long* next, unsigned long long* counters,
                                          uint32_t refill_min, uint32_t leaf_bias, const unsigned long long* n_dev, const TailQueue& tail,
-                                         const uint32_t* resume = nullptr) {
+                                         const uint32_t* resume = nullptr, uint32_t k = 0) {
     const RayIn* r = static_cast<const RayIn*>(rays);
     // rays per pool top-up: about 1/8 of a warp's fair share, a multiple of 32 in [32, 512]
     uint64_t warps = (uint64_t)grid * (TRACE_BLOCK / 32);
     uint64_t c = n / (warps * 8u + 1u);
     uint32_t chunk = (uint32_t)(c < 32 ? 32 : (c > 512 ? 512 : (c & ~31ull)));
     switch (cap) {
-        case 32: trace_persistent<ANY, COUNT, 32><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume); break;
-        case 64: trace_persistent<ANY, COUNT, 64><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume); break;
-        case 128: trace_persistent<ANY, COUNT, 128><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume); break;
-        case 256: trace_persistent<ANY, COUNT, 256><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume); break;
+        case 32: trace_persistent<P, COUNT, 32><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume, k); break;
+        case 64: trace_persistent<P, COUNT, 64><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume, k); break;
+        case 128: trace_persistent<P, COUNT, 128><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume, k); break;
+        case 256: trace_persistent<P, COUNT, 256><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume, k); break;
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();
@@ -776,10 +803,10 @@ cudaError_t launch_trace_wide(const SceneView& s, const void* d_rays, uint64_t n
     TailQueue q2 = tail;
     if (two_step) { q2.count = tail.count2; q2.next = tail.next2; q2.records = tail.records2; }
     auto pass = [&](const unsigned long long* n_dev, unsigned long long* next, const TailQueue& q, const uint32_t* resume) -> cudaError_t {
-        if (any) return count ? launch_persistent_cap<true, true>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume)
-                              : launch_persistent_cap<true, false>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume);
-        return count ? launch_persistent_cap<false, true>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume)
-                     : launch_persistent_cap<false, false>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume);
+        if (any) return count ? launch_persistent_cap<HIT_ANY, true>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume)
+                              : launch_persistent_cap<HIT_ANY, false>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume);
+        return count ? launch_persistent_cap<HIT_CLOSEST, true>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume)
+                     : launch_persistent_cap<HIT_CLOSEST, false>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume);
     };
     cudaError_t e = pass(d_n, d_next, q1, nullptr);
     // second pass: the suspended rays are its ray stream (count and read position = queue 1's counters)
@@ -795,6 +822,20 @@ cudaError_t launch_trace_wide(const SceneView& s, const void* d_rays, uint64_t n
     else { if (count) trace_tail_kernel<false, true><<<tail_grid, TAIL_BLOCK, smem, st>>>(s, r, d_out, q2, d_counters, fcap, wide_limit);
            else trace_tail_kernel<false, false><<<tail_grid, TAIL_BLOCK, smem, st>>>(s, r, d_out, q2, d_counters, fcap, wide_limit); }
     return cudaGetLastError();
+}
+
+cudaError_t launch_trace_multi(const SceneView& s, const void* d_rays, uint64_t n, uint32_t k, void* d_out, bool count,
+                               uint32_t stack_bound, int grid_blocks, unsigned long long* d_next, unsigned long long* d_counters,
+                               uint32_t refill_min, uint32_t leaf_bias, cudaStream_t st) {
+    const int cap = pick_cap(stack_bound);
+    if (!cap || k == 0) return cudaErrorInvalidValue;
+    cudaError_t e = cudaMemsetAsync(d_next, 0, 8 * sizeof(unsigned long long), st);
+    if (e != cudaSuccess) return e;
+    if (refill_min < 1 || refill_min > 32) refill_min = 8;
+    if (leaf_bias < 1 || leaf_bias > 512) leaf_bias = 16;
+    const TailQueue none = { nullptr, nullptr, nullptr, 0, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0, 0 };
+    return count ? launch_persistent_cap<HIT_MULTI, true>(cap, grid_blocks, st, s, d_rays, n, d_out, d_next, d_counters, refill_min, leaf_bias, nullptr, none, nullptr, k)
+                 : launch_persistent_cap<HIT_MULTI, false>(cap, grid_blocks, st, s, d_rays, n, d_out, d_next, d_counters, refill_min, leaf_bias, nullptr, none, nullptr, k);
 }
 
 uint32_t trace_warp_smem_words() { return (B2_TAIL_HELP && B2_TAIL_CODE) ? (uint32_t)WARP_SMEM_WORDS : 0u; }
@@ -818,6 +859,23 @@ cudaError_t launch_trace_binary(const SceneView& s, const void* d_rays, uint64_t
         case 64: launch_binary_cap<64>(any, (unsigned)blocks, st, s, r, n, d_out); break;
         case 128: launch_binary_cap<128>(any, (unsigned)blocks, st, s, r, n, d_out); break;
         case 256: launch_binary_cap<256>(any, (unsigned)blocks, st, s, r, n, d_out); break;
+        default: return cudaErrorInvalidValue;
+    }
+    return cudaGetLastError();
+}
+
+cudaError_t launch_trace_binary_multi(const SceneView& s, const void* d_rays, uint64_t n, uint32_t k, void* d_out, uint32_t max_depth_binary,
+                                      cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    uint64_t blocks = (n + 127) / 128;
+    if (blocks > 0x7fffffffull || k == 0) return cudaErrorInvalidValue;
+    const RayIn* r = static_cast<const RayIn*>(d_rays);
+    HitX* out = static_cast<HitX*>(d_out);
+    switch (pick_cap(max_depth_binary > 1u ? max_depth_binary : 1u)) {
+        case 32: trace_binary_multi_kernel<32><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, out, k); break;
+        case 64: trace_binary_multi_kernel<64><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, out, k); break;
+        case 128: trace_binary_multi_kernel<128><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, out, k); break;
+        case 256: trace_binary_multi_kernel<256><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, out, k); break;
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();
@@ -897,10 +955,10 @@ cudaError_t trace_occupancy(bool any, uint32_t stack_bound, int* blocks_per_sm) 
     int cap = pick_cap(stack_bound);
     const void* fn = nullptr;
     switch (cap) {
-        case 32: fn = any ? (const void*)trace_persistent<true, false, 32> : (const void*)trace_persistent<false, false, 32>; break;
-        case 64: fn = any ? (const void*)trace_persistent<true, false, 64> : (const void*)trace_persistent<false, false, 64>; break;
-        case 128: fn = any ? (const void*)trace_persistent<true, false, 128> : (const void*)trace_persistent<false, false, 128>; break;
-        case 256: fn = any ? (const void*)trace_persistent<true, false, 256> : (const void*)trace_persistent<false, false, 256>; break;
+        case 32: fn = any ? (const void*)trace_persistent<HIT_ANY, false, 32> : (const void*)trace_persistent<HIT_CLOSEST, false, 32>; break;
+        case 64: fn = any ? (const void*)trace_persistent<HIT_ANY, false, 64> : (const void*)trace_persistent<HIT_CLOSEST, false, 64>; break;
+        case 128: fn = any ? (const void*)trace_persistent<HIT_ANY, false, 128> : (const void*)trace_persistent<HIT_CLOSEST, false, 128>; break;
+        case 256: fn = any ? (const void*)trace_persistent<HIT_ANY, false, 256> : (const void*)trace_persistent<HIT_CLOSEST, false, 256>; break;
         default: return cudaErrorInvalidValue;
     }
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, fn, TRACE_BLOCK, 0);

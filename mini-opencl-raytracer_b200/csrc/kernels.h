@@ -49,6 +49,14 @@ cudaError_t launch_trace_wide(const SceneView& s, const void* d_rays, uint64_t n
 // (b2rt_scene_info); cudaErrorInvalidValue for a tree deeper than 256 levels.
 cudaError_t launch_trace_binary(const SceneView& s, const void* d_rays, uint64_t n, void* d_out, bool any, uint32_t max_depth_binary,
                                 cudaStream_t st);
+// The k nearest hits per ray (1 <= k): d_out is b2rt_hit[n * k], row i sorted by t and padded with misses. The persistent
+// kernel with the HIT_MULTI policy, without a cooperative tail (d_next: eight 64-bit scratch counters, reset here) ...
+cudaError_t launch_trace_multi(const SceneView& s, const void* d_rays, uint64_t n, uint32_t k, void* d_out, bool count,
+                               uint32_t stack_bound, int grid_blocks, unsigned long long* d_next, unsigned long long* d_counters,
+                               uint32_t refill_min, uint32_t leaf_bias, cudaStream_t st);
+// ... and the same over the reference-layout arrays, one thread per ray.
+cudaError_t launch_trace_binary_multi(const SceneView& s, const void* d_rays, uint64_t n, uint32_t k, void* d_out, uint32_t max_depth_binary,
+                                      cudaStream_t st);
 cudaError_t launch_camera_rays(const FrameArgs& a, uint64_t gid0, uint64_t gid1, void* d_rays, cudaStream_t st);
 // KernelEntry for the n pixels map.gid(0..n-1), one thread per pixel; binary: over the reference-layout arrays.
 cudaError_t launch_render_mega(const SceneView& s, const FrameArgs& a, float* d_result, const GidMap& map, uint32_t n,

@@ -305,14 +305,64 @@ B2_HD void tri_test_exact(const RayX& r, float ax, float ay, float az, float bx,
     if (ok && t < h.t) { h.t = t; h.u = u; h.v = v; h.tri = tri; }                      // :140
 }
 
+// ---- hit policies ------------------------------------------------------------------------
+// HIT_CLOSEST: h is the nearest accepted hit. HIT_ANY: the walk ends at the first accepted hit.
+// HIT_MULTI: the k nearest accepted hits, kept sorted by t in the ray's own output row (global memory, k records of 16 B);
+// h then holds the list's state, so that the policy needs no register beyond the other two:
+//     h.t   = bound: the ray's tmax while the row holds fewer than k hits, else the t of its k-th entry
+//     h.u   = the ray's tmax (the value unused slots are padded with)
+//     h.tri = the number of entries in the row
+// A triangle is accepted iff RayTriangle accepts it with t < bound -- the closest-hit rule with `best` replaced by the
+// bound, which never grows during the walk: the leaf gate on [0, bound] and every culling argument above carry over.
+enum : int { HIT_CLOSEST = 0, HIT_ANY = 1, HIT_MULTI = 2 };
+#if defined(__CUDACC__)
+// The row is read back with an explicit coherent load: the same thread wrote it earlier in this launch, so the read-only
+// path (ld.global.nc / __ldg) must not be used for it; the memory clobber keeps the load behind the stores before it.
+B2_HD HitX ld_hit(const HitX* p) {
+    HitX h; uint32_t t, u, v;
+    asm volatile("ld.global.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(t), "=r"(u), "=r"(v), "=r"(h.tri) : "l"(p) : "memory");
+    h.t = __uint_as_float(t); h.u = __uint_as_float(u); h.v = __uint_as_float(v);
+    return h;
+}
+B2_HD void st_hit(HitX* p, float t, float u, float v, uint32_t tri) { *reinterpret_cast<float4*>(p) = make_float4(t, u, v, __uint_as_float(tri)); }
+#else
+B2_HD HitX ld_hit(const HitX* p) { return *p; }
+B2_HD void st_hit(HitX* p, float t, float u, float v, uint32_t tri) { p->t = t; p->u = u; p->v = v; p->tri = tri; }
+#endif
+// Insert an accepted hit (t < h.t) into the row: after every entry with t' <= t, so equal t keeps visiting order like the
+// reference's strict `<`; a full row drops its last entry. Entries only move here.
+B2_HD void list_insert(HitX* row, uint32_t k, HitX& h, float t, float u, float v, uint32_t tri) {
+    uint32_t j = h.tri < k ? h.tri : k - 1u;          // the slot that becomes occupied
+    float last = t;                                    // what ends up in slot k - 1 (the new bound once the row is full)
+    for (; j > 0u; --j) {
+        const HitX p = ld_hit(row + j - 1u);
+        if (!(p.t > t)) break;
+        st_hit(row + j, p.t, p.u, p.v, p.tri);
+        if (j == k - 1u) last = p.t;
+    }
+    st_hit(row + j, t, u, v, tri);
+    if (h.tri < k) ++h.tri;
+    if (h.tri == k) h.t = last;
+}
+B2_HD void tri_test_multi(const RayX& r, float ax, float ay, float az, float bx, float by, float bz,
+                          float cx, float cy, float cz, uint32_t tri, HitX& h, HitX* row, uint32_t k) {
+    float t, u, v;
+    const bool ok = tri_eval_exact(r, ax, ay, az, bx, by, bz, cx, cy, cz, t, u, v);
+    if (ok && t < h.t) list_insert(row, k, h, t, u, v, tri);
+}
+// A finished HIT_MULTI ray: slots [h.tri, k) of its row become {tmax, 0, 0, B2RT_MISS}.
+B2_HD void pad_row(HitX* row, uint32_t k, const HitX& h) {
+    for (uint32_t i = h.tri; i < k; ++i) st_hit(row + i, h.u, 0.0f, 0.0f, 0xFFFFFFFFu);
+}
+
 // ---- leaf block ----------------------------------------------------------------------
 // The exact fp32 box of a one-record block: component-wise min / max of its vertices (exact operations; see b2rt_types.h).
 B2_HD float min3_nn(float a, float b, float c) { return min_nn(min_nn(a, b), c); }
 B2_HD float max3_nn(float a, float b, float c) { return max_nn(max_nn(a, b), c); }
 
-// Returns true when at least one triangle was accepted by this call.
-template <bool COUNT>
-B2_HD bool visit_leaf(const U4* leaf, uint32_t offset, const RayX& r, HitX& h, TravCounters* c) {
+// Returns true when at least one triangle was accepted by this call. MULTI: accepted hits go into `row` (HIT_MULTI).
+template <bool COUNT, bool MULTI = false>
+B2_HD bool visit_leaf(const U4* leaf, uint32_t offset, const RayX& r, HitX& h, TravCounters* c, HitX* row = nullptr, uint32_t row_len = 0) {
     const U4* p = leaf + offset;
     U4 a = ld128(p), b = ld128(p + 1), cc = ld128(p + 2);       // every block has >= 1 record
     const uint32_t nrec = (a.w >> LEAF_NREC_SHIFT) & LEAF_NREC_MASK;
@@ -338,14 +388,18 @@ B2_HD bool visit_leaf(const U4* leaf, uint32_t offset, const RayX& r, HitX& h, T
         float v2x = bits2f(b.x), v2y = bits2f(b.y), v2z = bits2f(b.z);
         float v3x = bits2f(cc.x), v3y = bits2f(cc.y), v3z = bits2f(cc.z);
         uint32_t flags = a.w & REC_FLAG_MASK;
-        tri_test_exact(r, v1x, v1y, v1z, v2x, v2y, v2z, v3x, v3y, v3z, id, h);
+        if (MULTI) tri_test_multi(r, v1x, v1y, v1z, v2x, v2y, v2z, v3x, v3y, v3z, id, h, row, row_len);
+        else tri_test_exact(r, v1x, v1y, v1z, v2x, v2y, v2z, v3x, v3y, v3z, id, h);
         if (COUNT) c->tri_tests++;
         if (flags) {
             // the loader's second copy of the same triangle, rotated left (v2,v3,v1) or right (v3,v1,v2)
             const bool left = flags == REC_ROT_LEFT;
-            tri_test_exact(r, left ? v2x : v3x, left ? v2y : v3y, left ? v2z : v3z,
-                           left ? v3x : v1x, left ? v3y : v1y, left ? v3z : v1z,
-                           left ? v1x : v2x, left ? v1y : v2y, left ? v1z : v2z, id + 1, h);
+            if (MULTI) tri_test_multi(r, left ? v2x : v3x, left ? v2y : v3y, left ? v2z : v3z,
+                                      left ? v3x : v1x, left ? v3y : v1y, left ? v3z : v1z,
+                                      left ? v1x : v2x, left ? v1y : v2y, left ? v1z : v2z, id + 1, h, row, row_len);
+            else tri_test_exact(r, left ? v2x : v3x, left ? v2y : v3y, left ? v2z : v3z,
+                                left ? v3x : v1x, left ? v3y : v1y, left ? v3z : v1z,
+                                left ? v1x : v2x, left ? v1y : v2y, left ? v1z : v2z, id + 1, h);
             if (COUNT) c->tri_tests++;
         }
         id += flags ? 2u : 1u;
@@ -608,8 +662,10 @@ template <int DEPTH, int STRIDE> B2_HD void stk_set(HybridStack<DEPTH, STRIDE> s
 // whichever step more lanes are waiting for.
 // The short stack of child references lives OUTSIDE this struct (a plain local array owned by the
 // caller): with the array inside, the compiler keeps every scalar of the struct in local memory too.
-template <bool ANY, bool COUNT, int CAP>
+// P: hit policy (HIT_CLOSEST, HIT_ANY, HIT_MULTI).
+template <int P, bool COUNT, int CAP>
 struct Lane {
+    static constexpr bool ANY = P == HIT_ANY, MULTI = P == HIT_MULTI;
     RayX r;
     HitX h;
     uint32_t cur;          // wide node to test next, a leaf waiting for a queue slot, or REF_EMPTY
@@ -625,6 +681,7 @@ struct Lane {
     B2_HD void start(const RayX& ray, float tmax) {
         r = ray;
         h.t = tmax; h.u = 0.0f; h.v = 0.0f; h.tri = 0xFFFFFFFFu;
+        if (MULTI) { h.u = tmax; h.tri = 0u; }        // empty list (see HIT_MULTI)
         cur = 0; leaf0 = leaf1 = top = REF_EMPTY; sp = 0; overflow = false;
 #if B2_LEAF_QUEUE == 3
         leaf2 = REF_EMPTY;
@@ -716,9 +773,10 @@ struct Lane {
         settle(stack);
     }
     // Returns true when the ray is finished by this leaf (any-hit accept, or best < 0: every later
-    // box test of the reference fails, SURVEY.md Appendix A-5).
-    template <class S> B2_HD bool leaf_step(const U4* leaf, S stack) {
-        bool got = visit_leaf<COUNT>(leaf, leaf0 & ~REF_LEAF_BIT, r, h, COUNT ? &tc : nullptr);
+    // box test of the reference fails, SURVEY.md Appendix A-5; for HIT_MULTI the bound < 0).
+    // row, k: the ray's output row and its length (HIT_MULTI only).
+    template <class S> B2_HD bool leaf_step(const U4* leaf, S stack, HitX* row = nullptr, uint32_t k = 0) {
+        bool got = visit_leaf<COUNT, MULTI>(leaf, leaf0 & ~REF_LEAF_BIT, r, h, COUNT ? &tc : nullptr, row, k);
 #if B2_LEAF_QUEUE == 3
         leaf0 = leaf1; leaf1 = leaf2; leaf2 = REF_EMPTY;
 #else
@@ -733,10 +791,11 @@ struct Lane {
 // ---- simple per-ray driver (one thread = one ray; also the host emulation) -------------
 // `schedule` != 0 makes the emulation pick node/leaf steps pseudo-randomly whenever both are
 // allowed, to exercise every interleaving the warp-vote kernels can produce.
-template <bool ANY, bool COUNT, int CAP>
+// HIT_MULTI: the hits go to row[0, k), padded when the ray is finished.
+template <int P, bool COUNT, int CAP>
 B2_HD HitX trace_wide(const U4* wide, const U4* leaf, const RayX& r, float tmax, TravCounters* c, bool* overflow,
-                      uint32_t one, uint32_t schedule = 0) {
-    Lane<ANY, COUNT, CAP> L;
+                      uint32_t one, uint32_t schedule = 0, HitX* row = nullptr, uint32_t k = 0) {
+    Lane<P, COUNT, CAP> L;
     uint32_t stack[CAP];
     L.tc.wide_nodes = L.tc.leaf_blocks = L.tc.leaf_pass = L.tc.tri_tests = L.tc.words = L.tc.max_stack = L.tc.rounds = 0;
     L.start(r, tmax);
@@ -744,9 +803,10 @@ B2_HD HitX trace_wide(const U4* wide, const U4* leaf, const RayX& r, float tmax,
         const bool node = L.wants_node(), lf = L.wants_leaf();
         bool do_leaf = lf;                                  // default: consume pending leaves first (no speculation)
         if (node && lf && schedule) { schedule = schedule * 1664525u + 1013904223u; do_leaf = (schedule >> 16) & 1u; }
-        if (do_leaf) { if (L.leaf_step(leaf, stack)) break; }
+        if (do_leaf) { if (L.leaf_step(leaf, stack, row, k)) break; }
         else L.node_step(wide, stack, one);
     }
+    if (P == HIT_MULTI) pad_row(row, k, L.h);
     if (COUNT && c) *c = L.tc;
     if (overflow) *overflow = L.overflow;
     return L.h;

@@ -62,6 +62,7 @@ def lib():
         "g3d_engine_scene": (vp, [vp]),
         "g3d_engine_trace_closest": (C.c_int, [vp, vp, u64, vp, cs, sz]),
         "g3d_engine_trace_any": (C.c_int, [vp, vp, u64, vp, cs, sz]),
+        "g3d_engine_trace_multi": (C.c_int, [vp, vp, u64, C.c_uint32, vp, cs, sz]),
         "g3d_write_icosphere_obj": (C.c_longlong, [cs, C.c_int, C.c_double, C.c_double, C.c_ulonglong]),
         "g3d_write_scattered_obj": (C.c_longlong, [cs, C.c_longlong, C.c_double, C.c_double, C.c_double, C.c_ulonglong]),
     }
@@ -274,3 +275,11 @@ class Engine:
         e = _err()
         self._ck(self._L.g3d_engine_trace_any(self._h, rays.ctypes.data, rays.shape[0], occluded.ctypes.data, e, len(e)), e)
         return occluded
+
+    def trace_multi(self, rays, k):
+        """CLRaytracer::TraceMulti: the k nearest hits of every ray as an (n, k) HIT_DTYPE array."""
+        rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
+        hits = np.empty((rays.shape[0], max(int(k), 0)), dtype=HIT_DTYPE)
+        e = _err()
+        self._ck(self._L.g3d_engine_trace_multi(self._h, rays.ctypes.data, rays.shape[0], int(k), hits.ctypes.data, e, len(e)), e)
+        return hits

@@ -14,7 +14,7 @@
 //   CLOBJloader ........................... CLOBJloader.h, CLOBJloader.cpp:10-176
 //   CLRaytracer ........................... CLRaytracer.h:16-40, CLRaytracer.cpp:12-148
 //   CLui (state only) / CLEngineBase ...... CLui.h:17-40, CLEngineBase.h:13-93, CLEngineBase.cpp:141-211
-// New (the reference has no ray-stream API): CLRaytracer::TraceClosest / TraceAny.
+// New (the reference has no ray-stream API): CLRaytracer::TraceClosest / TraceAny / TraceMulti.
 #pragma once
 #include <cstddef>
 #include <cstdint>
@@ -261,6 +261,8 @@ namespace Glaze3D
         // New: ray streams through the same scene. hits[i].tri == B2RT_MISS on a miss.
         void TraceClosest(const b2rt_ray* rays, uint64_t n, b2rt_hit* hits);
         void TraceAny(const b2rt_ray* rays, uint64_t n, uint32_t* occluded);
+        // The k nearest hits per ray (b2rt_trace_multi): hits[i*k .. i*k+k) sorted by t, unused slots {tmax, 0, 0, B2RT_MISS}.
+        void TraceMulti(const b2rt_ray* rays, uint64_t n, uint32_t k, b2rt_hit* hits);
 
         std::shared_ptr<CLContext> m_CLContext = nullptr;
         std::shared_ptr<CLKernel> m_RenderKernel = nullptr;

@@ -245,3 +245,10 @@ extern "C" int g3d_engine_trace_any(void* engine, const b2rt_ray* rays, uint64_t
     return 0;
     G3D_CATCH(-1)
 }
+extern "C" int g3d_engine_trace_multi(void* engine, const b2rt_ray* rays, uint64_t n, uint32_t k, b2rt_hit* hits, char* err, size_t errLen)
+{
+    G3D_TRY
+    static_cast<EngineBox*>(engine)->engine->render->TraceMulti(rays, n, k, hits);
+    return 0;
+    G3D_CATCH(-1)
+}

@@ -162,6 +162,11 @@ namespace Glaze3D
         int st = b2rt_trace_any(m_CLContext->GetContext(), rays, n, occluded);
         if (st) throw CLException(std::string("Failed to trace rays: ") + b2rt_last_error(m_CLContext->GetContext()), st);
     }
+    void CLRaytracer::TraceMulti(const b2rt_ray* rays, uint64_t n, uint32_t k, b2rt_hit* hits)
+    {
+        int st = b2rt_trace_multi(m_CLContext->GetContext(), rays, n, k, hits);
+        if (st) throw CLException(std::string("Failed to trace rays: ") + b2rt_last_error(m_CLContext->GetContext()), st);
+    }
 
     // ---- CLEngineBase (headless) -------------------------------------------------------------------
     CLEngineBase::CLEngineBase()

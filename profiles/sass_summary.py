@@ -12,9 +12,11 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "mini-opencl-raytracer_b200", "libb2rt.so")
+# the hit policy of trace_persistent is its first template argument: 0 closest, 1 any-hit, 2 multi (traverse.cuh HIT_*)
 KERNELS = {
-    "trace_persistent<closest, no counters, CAP 64>": "trace_persistentILb0ELb0ELi64E",
-    "trace_persistent<any-hit, no counters, CAP 64>": "trace_persistentILb1ELb0ELi64E",
+    "trace_persistent<closest, no counters, CAP 64>": "trace_persistentILi0ELb0ELi64E",
+    "trace_persistent<any-hit, no counters, CAP 64>": "trace_persistentILi1ELb0ELi64E",
+    "trace_persistent<multi, no counters, CAP 64>": "trace_persistentILi2ELb0ELi64E",
     "trace_tail_kernel<closest, no counters>": "trace_tail_kernelILb0ELb0E",
     "wf_shade_kernel": "wf_shade_kernel",
     "wf_generate_kernel": "wf_generate_kernel",
