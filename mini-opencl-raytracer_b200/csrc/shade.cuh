@@ -1,10 +1,11 @@
 // shade.cuh -- device re-statement of the per-pixel driver around the traversal:
 // RNG, camera, BRDF sampling, lighting and accumulation of kernel_bvh.cl:57-96,
-// 221-456. Needed only so that rendered frames match the reference (PSNR), it is
-// not the optimisation target. Every fp32 operation replays the reference's
-// operation order with one rounding per op; pow/sin/cos are evaluated in fp64 and
-// rounded once, which reproduces glibc's (nearly always correctly rounded) powf/
-// sinf/cosf used by the CPU oracle to within 1 ulp.
+// 221-456. Not the optimisation target. Every fp32 operation replays the
+// reference's operation order with one rounding per op; pow/sin/cos are evaluated
+// in fp64 and rounded once, which reproduces glibc's (nearly always correctly
+// rounded) powf/sinf/cosf used by the CPU oracle to within 1 ulp. Frames equal,
+// bit for bit, the oracle built with these three functions in place of glibc's
+// (tests/frame_oracle/oracle_devlibm.c, tests/test_gpu_frame_exact.py).
 #pragma once
 #include "traverse.cuh"
 
@@ -28,9 +29,15 @@ __device__ __forceinline__ V3 ldv(const RefVec& p) { return v3(p.x, p.y, p.z); }
 // powf as glibc evaluates it for the CPU oracle (correctly rounded except very near rounding boundaries): a double result
 // good to ~1e-14 relative, rounded once to float. exp2(b * log2(a)) in fp64 delivers that at half the cost of CUDA's
 // full double-precision pow(); the square (pow(x, 2.0), used twice by SampleBrdf) is exact in fp64 and also correct for
-// negative x, where the logarithm route would give NaN. Special values follow powf for the exponents the kernel uses
-// (2.0, 2.2, 0.4545.., 1/(alpha+1)): pow(0, b>0) = 0, pow(x<0, non-integer) = NaN, pow(inf, b>0) = inf, NaN propagates.
+// negative x, where the logarithm route would give NaN. The logarithm route gives NaN where C99 powf returns 1 -- pow(x, 0)
+// for x = 0, inf or NaN (0 * -inf, 0 * inf, 0 * NaN) and pow(1, y) for y = +-inf or NaN (inf * 0, NaN * 0) -- so those two
+// cases return 1 first. SampleBrdf reaches both: roughness 0 gives the exponent 1/(alpha+1) = 0, roughness sqrt(2) gives
+// alpha = -1 and the exponent inf, and rnd() returns exactly 0 or 1 for some seeds. For the bases the kernel passes
+// (rnd() in [0, 1], pixel values >= 0 or NaN, any value squared) the other special values follow powf by themselves:
+// pow(0, b>0) = 0, pow(0, b<0) = inf, pow(inf, b>0) = inf, pow(x<1, inf) = 0, NaN propagates. A negative base with an
+// integer exponent other than 2 would not (NaN instead of +-|a|^b); no caller passes one.
 __device__ __forceinline__ float pow_cr(float a, float b) {
+    if (b == 0.0f || (a == 1.0f && !(fabsf(b) < INFINITY))) return 1.0f;   // folds away for a constant finite b
     if (b == 2.0f) return (float)((double)a * (double)a);
     return (float)exp2((double)b * log2((double)a));
 }
