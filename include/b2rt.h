@@ -305,6 +305,49 @@ int b2rt_trace_any_device(b2rt_context* ctx, const b2rt_ray* d_rays, uint64_t n,
 #define B2RT_MULTI_MAX_HITS 64
 int b2rt_trace_multi(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, uint32_t k, b2rt_hit* hits);
 int b2rt_trace_multi_device(b2rt_context* ctx, const b2rt_ray* d_rays, uint64_t n, uint32_t k, b2rt_hit* d_hits, void* cuda_stream);
+
+/* ---- closest point (new) ------------------------------------------------------------------ */
+/* Nearest surface point of the bound scene to each query point, and its squared distance (collision and contact, snapping
+ * onto a surface, distance-field sampling, attribute transfer).
+ *  Candidates: every triangle k of the bound scene array, (a, b, c) = (v1, v2, v3).position.xyz of its CLTriangle. The
+ *    loader's two copies of a face are two candidates (the second one's vertices rotated as stored).
+ *  Distance: cp(p, a, b, c) -> (d2, u, v) is Ericson's region test ("Real-Time Collision Detection" 5.1.5), every operation
+ *    one IEEE fp32 operation rounded to nearest, no contraction, in this order: ab = b-a, ac = c-a, ap = p-a, d1 = ab.ap,
+ *    d2' = ac.ap (x.y = (x0*y0 + x1*y1) + x2*y2); bp = p-b, cp = p-c, d3 = ab.bp, d4 = ac.bp, d5 = ab.cp, d6 = ac.cp,
+ *    vc = d1*d4 - d3*d2', vb = d5*d2' - d1*d6, va = d3*d6 - d5*d4. The first region (Ericson's order and conditions) that
+ *    holds is taken (an edge region also needs its denominator > 0, which only a zero-length edge fails: without it a
+ *    repeated vertex would take that edge's branch with t = 0/0):
+ *      vertex a   d1 <= 0 && d2' <= 0                         (u, v) = (0, 0), point a
+ *      vertex b   d3 >= 0 && d4 <= d3                         (1, 0), point b
+ *      edge ab    vc <= 0 && d1 >= 0 && d3 <= 0 && d1-d3 > 0                      (t, 0), t = d1/(d1-d3), point a + ab*t
+ *      vertex c   d6 >= 0 && d5 <= d6                                              (0, 1), point c
+ *      edge ac    vb <= 0 && d2' >= 0 && d6 <= 0 && d2'-d6 > 0                    (0, t), t = d2'/(d2'-d6), point a + ac*t
+ *      edge bc    va <= 0 && (d4-d3) >= 0 && (d5-d6) >= 0 && (d4-d3)+(d5-d6) > 0
+ *                                                                (1-t, t), t = (d4-d3)/((d4-d3)+(d5-d6)), point b + (c-b)*t
+ *      interior   (va+vb)+vc > 0: denom = 1/((va+vb)+vc), (u, v) = (vb*denom, vc*denom), point (a + ab*u) + ac*v
+ *      otherwise (degenerate): the edges ab, ac, bc in this order from their origins a, a, b, each with
+ *        t = clamp01((o->p).e / e.e) (clamp01 maps NaN to 0), point o + e*t, clamped and measured as below; the smallest
+ *        d2 wins, ties to the earlier edge; (u, v) = (t, 0), (0, t) or (1-t, t).
+ *    The point is clamped per axis into the triangle's vertex box [min(a,b,c), max(a,b,c)] (fminf(fmaxf(q, lo), hi): NaN
+ *    becomes lo), then d2 = ((px-qx)^2 + (py-qy)^2) + (pz-qz)^2. (u, v) are the branch's parameters in the reference's
+ *    barycentric convention, point = (1-u-v) v1 + u v2 + v v3.
+ *  Result: among the candidates with d2 <= max_d2, the smallest d2, ties to the smallest triangle index:
+ *    out[i] = {d2, u, v, tri}; when none qualifies {max_d2, 0, 0, B2RT_MISS}. max_d2 = +inf searches the whole scene; a
+ *    negative or NaN max_d2, or a NaN coordinate, always misses. The result does not depend on the tree or visiting order.
+ *  Outside the contract: scenes with non-finite vertices (the device build and refit reject them) and caller-supplied trees
+ *    whose node boxes do not contain their triangles (every builder here produces boxes that do).
+ * n = 0 succeeds; a NULL pointer with n > 0 returns B2RT_INVALID_VALUE and writes nothing.
+ * b2rt_closest_point: host buffers, synchronous, pipelined in chunks like b2rt_trace_closest; on a b2rt_create_multi handle
+ * the queries are cut into contiguous ranges, one per device.
+ * b2rt_closest_point_device: device buffers, asynchronous on cuda_stream with the stream rules of b2rt_trace_closest_device;
+ * on a b2rt_create_multi handle it runs on the root.
+ * B2RT_OPT_TRAVERSAL = 1 runs the reference-layout walk, B2RT_OPT_COUNTERS = 1 the counting build (rays = queries,
+ * tri_tests = distance evaluations). B2RT_OPT_COOP_MAX, B2RT_OPT_RESUME_MAX and B2RT_OPT_TAIL_HELP are ignored. */
+typedef struct { float x, y, z, max_d2; } b2rt_point_query;      /* 16 B */
+typedef struct { float d2, u, v; uint32_t tri; } b2rt_point_hit;   /* 16 B */
+int b2rt_closest_point(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out);
+int b2rt_closest_point_device(b2rt_context* ctx, const b2rt_point_query* d_q, uint64_t n, b2rt_point_hit* d_out, void* cuda_stream);
+
 /* CreateRay (kernel_bvh.cl:386-403) for gid in [gid_begin, gid_end) with the currently bound
  * WIDTH/HEIGHT/FRAME_COUNT/CAMERA_* arguments, written to device memory as b2rt_ray. */
 int b2rt_camera_rays_device(b2rt_context* ctx, size_t gid_begin, size_t gid_end, b2rt_ray* d_rays, void* cuda_stream);
@@ -318,7 +361,8 @@ int b2rt_camera_rays_device(b2rt_context* ctx, size_t gid_begin, size_t gid_end,
  *    devices; each device keeps the running average of ITS pixels and stores every finished pixel through to the root's
  *    image over a peer mapping, so b2rt_read_buffer / b2rt_read_pixels after it return the complete frame (the root's
  *    stream waits for all devices);
- *  - b2rt_trace_closest / b2rt_trace_any / b2rt_trace_multi cut the host ray stream into contiguous ranges, one per device;
+ *  - b2rt_trace_closest / b2rt_trace_any / b2rt_trace_multi cut the host ray stream into contiguous ranges, one per device,
+ *    and b2rt_closest_point its queries likewise;
  *  - the *_device entry points, b2rt_build_bvh and b2rt_execute_bands address one device: the root
  *    (b2rt_build_scene_device builds there and copies the scene to every device).
  * n_devices == 1 gives an ordinary handle. CLRaytracer code written against the single-device calls runs unchanged. */

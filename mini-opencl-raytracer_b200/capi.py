@@ -6,7 +6,7 @@ import time
 
 import numpy as np
 
-from .layouts import HIT_DTYPE, MAT_BYTES, NODE_BYTES, RAY_DTYPE, TRI_BYTES
+from .layouts import HIT_DTYPE, MAT_BYTES, NODE_BYTES, POINT_HIT_DTYPE, POINT_QUERY_DTYPE, RAY_DTYPE, TRI_BYTES
 
 MISS = 0xFFFFFFFF
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -30,6 +30,7 @@ SYMBOLS = [
     "b2rt_create_multi", "b2rt_group_size", "b2rt_group_info", "b2rt_comm_unique_id", "b2rt_comm_init", "b2rt_comm_share_output",
     "b2rt_execute_shard", "b2rt_shard_bands", "b2rt_refit_scene", "b2rt_stage_times",
     "b2rt_build_scene_device", "b2rt_refit_scene_device", "b2rt_trace_multi", "b2rt_trace_multi_device",
+    "b2rt_closest_point", "b2rt_closest_point_device",
 ]
 MULTI_MAX_HITS = 64          # B2RT_MULTI_MAX_HITS: largest k of b2rt_trace_multi
 # status bits of b2rt_refit_scene_device
@@ -100,6 +101,8 @@ def lib():
         "b2rt_trace_any_device": (C.c_int, [vp, vp, u64, vp, vp]),
         "b2rt_trace_multi": (C.c_int, [vp, vp, u64, u32, vp]),
         "b2rt_trace_multi_device": (C.c_int, [vp, vp, u64, u32, vp, vp]),
+        "b2rt_closest_point": (C.c_int, [vp, vp, u64, vp]),
+        "b2rt_closest_point_device": (C.c_int, [vp, vp, u64, vp, vp]),
         "b2rt_camera_rays_device": (C.c_int, [vp, sz, sz, vp, vp]),
         "b2rt_device_pointer": (C.c_int, [vp, u64, C.POINTER(vp), C.POINTER(sz)]),
         "b2rt_bound_buffer": (C.c_int, [vp, u32, C.POINTER(u64)]),
@@ -416,6 +419,19 @@ class Context:
         """b2rt_trace_multi_device: d_hits holds n * k records of 16 bytes."""
         self._ck(self._L.b2rt_trace_multi_device(self._h, C.c_void_p(int(d_rays)), int(n), int(k), C.c_void_p(int(d_hits)),
                                                  C.c_void_p(int(stream))))
+
+    def closest_point(self, queries):
+        """The nearest surface point of the scene to every query (b2rt_closest_point): a POINT_HIT_DTYPE array of
+        {d2, u, v, tri}; {max_d2, 0, 0, MISS} where no triangle lies within max_d2."""
+        queries = np.ascontiguousarray(queries, dtype=POINT_QUERY_DTYPE)
+        out = np.empty(queries.shape[0], dtype=POINT_HIT_DTYPE)
+        self._ck(self._L.b2rt_closest_point(self._h, _ptr(queries), queries.shape[0], _ptr(out)))
+        return out
+
+    def closest_point_device(self, d_queries, n, d_out, stream=0):
+        """b2rt_closest_point_device: n query and n result records of 16 bytes in device memory."""
+        self._ck(self._L.b2rt_closest_point_device(self._h, C.c_void_p(int(d_queries)), int(n), C.c_void_p(int(d_out)),
+                                                   C.c_void_p(int(stream))))
 
     def trace_closest_device(self, d_rays, n, d_hits, stream=0):
         self._ck(self._L.b2rt_trace_closest_device(self._h, C.c_void_p(int(d_rays)), int(n), C.c_void_p(int(d_hits)),

@@ -356,6 +356,30 @@ int trace_device(b2rt_context* ctx, const void* d_rays, uint64_t n, void* d_out,
     return B2RT_SUCCESS;
 }
 
+// Closest point per query (b2rt_closest_point_device): d_q = b2rt_point_query[n], d_out = b2rt_point_hit[n].
+int point_device(b2rt_context* ctx, const void* d_q, uint64_t n, void* d_out, cudaStream_t st) {
+    if (n == 0) return B2RT_SUCCESS;
+    if (!d_q || !d_out) return fail(ctx, B2RT_INVALID_VALUE, "null query or output pointer");
+    if (ctx->opt_traversal == 1) {
+        int fits = binary_walk_fits(ctx);
+        if (fits) return fits;
+        CK(launch_closest_point_binary(ctx->view, d_q, n, d_out, ctx->info.max_depth_binary, st));
+        ctx->launches += 1;
+        return B2RT_SUCCESS;
+    }
+    int grid = ctx->grid_closest;
+    if (ctx->opt_blocks_per_sm > 0) grid = ctx->sm_count * (int)ctx->opt_blocks_per_sm;
+    const uint64_t blocks_needed = ((n + 31) / 32 * 32 + trace_block_threads() - 1) / trace_block_threads();
+    if ((uint64_t)grid > blocks_needed) grid = (int)blocks_needed;
+    int st_pol = apply_l2_policy(ctx, st);
+    if (st_pol) return st_pol;
+    unsigned long long* next = ctx->d_next + 8 * (ctx->next_seq++ % NEXT_RING);     // a counter of its own, as for rays
+    CK(launch_closest_point(ctx->view, d_q, n, d_out, ctx->opt_counters != 0, ctx->stack_bound, grid, next, ctx->d_counters,
+                            (uint32_t)ctx->opt_refill_min, st));
+    ctx->launches += 1;
+    return B2RT_SUCCESS;
+}
+
 int ensure_staging(b2rt_context* ctx, uint64_t chunk, size_t out_bytes) {
     if (ctx->stage_capacity >= chunk && ctx->stage_out_bytes >= out_bytes) return B2RT_SUCCESS;
     chunk = std::max(chunk, ctx->stage_capacity);
@@ -414,6 +438,45 @@ int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, b
         CK(cudaStreamWaitEvent(ctx->stream_out, ctx->ev_comp[s], 0));
         CK(cudaMemcpyAsync(static_cast<char*>(out) + off * out_elem, ctx->d_stage_out[s], m * out_elem,
                            cudaMemcpyDeviceToHost, ctx->stream_out));
+        CK(cudaEventRecord(ctx->ev_out[s], ctx->stream_out));
+    }
+    CK(cudaStreamSynchronize(ctx->stream_out));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return B2RT_SUCCESS;
+}
+
+// Host-buffer closest-point queries: the pipeline of trace_host with 16-byte queries and records (a staging buffer sized
+// for a chunk of rays holds a chunk of queries).
+int point_host(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out) {
+    int st = use_device(ctx);
+    if (st) return st;
+    st = ensure_scene(ctx);
+    if (st) return st;
+    if (n == 0) return B2RT_SUCCESS;
+    if (!q || !out) return fail(ctx, B2RT_INVALID_VALUE, "null query or output pointer");
+    uint64_t chunk_q = STREAM_CHUNK;
+    if (const char* env = getenv("B2RT_STREAM_CHUNK")) { long long v = atoll(env); if (v >= 1024) chunk_q = (uint64_t)v; }
+    const uint64_t chunk = std::min<uint64_t>(n, chunk_q);
+    st = ensure_staging(ctx, chunk, chunk * sizeof(b2rt_point_hit));
+    if (st) return st;
+    const uint64_t ramp = std::min<uint64_t>(chunk, 1ull << 19);
+    uint64_t c = 0, m = 0;
+    for (uint64_t off = 0; off < n; off += m, ++c) {
+        const int s = (int)(c & 1);
+        const uint64_t left = n - off;
+        m = std::min<uint64_t>(chunk, ramp << std::min<uint64_t>(c, 16));
+        if (left <= ramp) m = left;
+        else m = std::min<uint64_t>(m, std::max<uint64_t>(ramp, (left / 2 + 31) & ~31ull));
+        if (c >= 2) CK(cudaStreamWaitEvent(ctx->stream_in, ctx->ev_comp[s], 0));
+        CK(cudaMemcpyAsync(ctx->d_stage_rays[s], q + off, m * sizeof(b2rt_point_query), cudaMemcpyHostToDevice, ctx->stream_in));
+        CK(cudaEventRecord(ctx->ev_in[s], ctx->stream_in));
+        CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[s], 0));
+        if (c >= 2) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[s], 0));
+        st = point_device(ctx, ctx->d_stage_rays[s], m, ctx->d_stage_out[s], ctx->stream);
+        if (st) return st;
+        CK(cudaEventRecord(ctx->ev_comp[s], ctx->stream));
+        CK(cudaStreamWaitEvent(ctx->stream_out, ctx->ev_comp[s], 0));
+        CK(cudaMemcpyAsync(out + off, ctx->d_stage_out[s], m * sizeof(b2rt_point_hit), cudaMemcpyDeviceToHost, ctx->stream_out));
         CK(cudaEventRecord(ctx->ev_out[s], ctx->stream_out));
     }
     CK(cudaStreamSynchronize(ctx->stream_out));
@@ -1210,6 +1273,22 @@ extern "C" int b2rt_trace_multi_device(b2rt_context* ctx, const b2rt_ray* d_rays
     st = ensure_scene(ctx);
     if (st) return st;
     return trace_device(ctx, d_rays, n, d_hits, false, cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream, k);
+}
+// ---- closest point ----------------------------------------------------------------------------
+extern "C" int b2rt_closest_point(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out) {
+    if (!ctx) return B2RT_INVALID_CONTEXT;
+    if (n && (!q || !out)) return fail(ctx, B2RT_INVALID_VALUE, "null query or output pointer");
+    if (ctx->group) return group_point_host(ctx, q, n, out);                 // contiguous ranges, one per device
+    return point_host(ctx, q, n, out);
+}
+extern "C" int b2rt_closest_point_device(b2rt_context* ctx, const b2rt_point_query* d_q, uint64_t n, b2rt_point_hit* d_out, void* cuda_stream) {
+    if (!ctx) return B2RT_INVALID_CONTEXT;
+    if (n && (!d_q || !d_out)) return fail(ctx, B2RT_INVALID_VALUE, "null query or output pointer");
+    int st = use_device(ctx);
+    if (st) return st;
+    st = ensure_scene(ctx);
+    if (st) return st;
+    return point_device(ctx, d_q, n, d_out, cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream);
 }
 extern "C" int b2rt_camera_rays_device(b2rt_context* ctx, size_t gid_begin, size_t gid_end, b2rt_ray* d_rays, void* cuda_stream) {
     if (!ctx) return B2RT_INVALID_CONTEXT;

@@ -18,6 +18,8 @@
 //  render_mega_kernel               KernelEntry as one launch: one thread per pixel, path loop
 //      around the same traversal primitives (bit-identical to the wavefront).
 //  tonemap_rgba8_kernel             accumulation image -> clamped 8-bit RGBA for display read-back.
+//  point_persistent<COUNT,CAP>      closest point on the scene per query point (point_query.cuh), persistent like
+//      trace_persistent; point_binary_kernel<CAP> the same over the reference-layout arrays, one thread per query.
 //
 // No tensor cores: the path is pointer chasing + fp32 slab/triangle tests, not a
 // contraction (BASELINE.json north_star). Compile with -fmad=false; all
@@ -28,6 +30,7 @@
 #include "kernels.h"
 #include "shade.cuh"
 #include "coop.cuh"
+#include "point_query.cuh"
 
 namespace b2rt {
 
@@ -752,6 +755,124 @@ tonemap_rgba8_kernel(const float4* __restrict__ image, uchar4* __restrict__ out,
 }
 
 // ---------------------------------------------------------------------------------------
+// Closest point (b2rt_closest_point). Every lane owns one query (PointLane, point_query.cuh); warps pull chunks of queries
+// from a global atomic counter into a warp-local pool and refill idle lanes from it (ballot + popc compaction), like
+// trace_persistent. Per round the warp votes: the lanes that want a wide-node step or those that want a leaf step, by
+// majority. The result does not depend on the schedule: it is the minimum of the total order (d2, tri).
+// ---------------------------------------------------------------------------------------
+static constexpr int POINT_BLOCK = 128;
+
+__device__ __forceinline__ void write_point(float4* __restrict__ out, uint64_t i, const PointHit& h) {
+    __stcs(out + i, make_float4(h.d2, h.u, h.v, __uint_as_float(h.tri)));
+}
+
+template <bool COUNT, int CAP>
+__global__ void __launch_bounds__(POINT_BLOCK, B2_MIN_BLOCKS)
+point_persistent(SceneView s, const float4* __restrict__ queries, uint64_t n, float4* __restrict__ out,
+                 unsigned long long* __restrict__ next, unsigned long long* __restrict__ counters, uint32_t chunk, uint32_t refill_min) {
+    const unsigned lane = threadIdx.x & 31u;
+    PointLane<COUNT, CAP> L;
+    PointEntry stack[CAP];
+    L.cur = REF_EMPTY; L.sp = 0; L.overflow = false;
+    L.tc.wide_nodes = L.tc.leaf_blocks = L.tc.tri_tests = L.tc.words = L.tc.max_stack = 0;
+    uint64_t my_index = 0, pool_next = 0;
+    uint32_t pool_left = 0, started = 0;
+    bool dry = false;                        // warp-uniform: the global counter has run past n
+    for (;;) {
+        const unsigned vn = __ballot_sync(FULL, L.wants_node());
+        const unsigned vl = __ballot_sync(FULL, L.wants_leaf());
+        const unsigned busy = vn | vl;
+        if (32u - (unsigned)__popc(busy) >= (dry ? 32u : refill_min)) {
+            if (dry) break;
+            if (pool_left == 0u) {
+                unsigned long long base = 0;
+                if (lane == 0) base = atomicAdd(next, (unsigned long long)chunk);
+                base = __shfl_sync(FULL, base, 0);
+                if (base >= n) { dry = true; continue; }
+                pool_next = base;
+                pool_left = (base + chunk < n) ? chunk : (uint32_t)(n - base);
+            }
+            const unsigned idle = ~busy;
+            const unsigned rank = __popc(idle & ((1u << lane) - 1u));
+            if (((idle >> lane) & 1u) && rank < pool_left) {
+                my_index = pool_next + rank;
+                const float4 q = __ldcs(queries + my_index);
+                if (!L.start(q.x, q.y, q.z, q.w)) write_point(out, my_index, L.best);      // misses without a walk
+                if (COUNT) started++;
+            }
+            const unsigned taken = __popc(idle), used = taken < pool_left ? taken : pool_left;
+            pool_next += used;
+            pool_left -= used;
+            continue;
+        }
+        bool stepped;
+        if (__popc(vn) >= __popc(vl)) { stepped = L.wants_node(); if (stepped) L.node_step(s.wide, stack); }
+        else { stepped = L.wants_leaf(); if (stepped) L.leaf_step(s.leaf, stack); }
+        if (stepped && L.done()) write_point(out, my_index, L.best);
+    }
+    if (COUNT) {
+        if (L.overflow) report_stack_overflow();
+        // the ray counters' slots: [0] queries, [1] wide-node visits, [2] leaf blocks, [4] distance evaluations, [5] words
+        unsigned long long v[5] = { started, L.tc.wide_nodes, L.tc.leaf_blocks, L.tc.tri_tests, L.tc.words };
+        const int slot[5] = { 0, 1, 2, 4, 5 };
+#pragma unroll
+        for (int i = 0; i < 5; ++i) {
+            unsigned long long x = v[i];
+            for (int o = 16; o; o >>= 1) x += __shfl_xor_sync(FULL, x, o);
+            if (lane == 0 && x) atomicAdd(&counters[slot[i]], x);
+        }
+    }
+}
+
+// The same query over the reference's CLLinearBVHNode / CLTriangle arrays, one thread per query: a node is entered iff the
+// lb of its exact fp32 box is <= the best so far; the child on the point's side of the box's middle goes first. The stack
+// holds one entry per level (CAP >= max_depth_binary, as for trace_binary).
+template <int CAP>
+__global__ void __launch_bounds__(128)
+point_binary_kernel(SceneView s, const float4* __restrict__ queries, uint64_t n, float4* __restrict__ out) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float4 q = __ldg(queries + i);
+    PointHit best; best.d2 = q.w; best.u = 0.0f; best.v = 0.0f; best.tri = 0xFFFFFFFFu;
+    if (q.x == q.x && q.y == q.y && q.z == q.z && q.w >= 0.0f) {
+        uint32_t stack[CAP];
+        int sp = 0;
+        uint32_t cur = 0;
+        for (;;) {
+            const float4* np = reinterpret_cast<const float4*>(s.nodes + cur);
+            const float4 lo = __ldg(np), hi = __ldg(np + 1);
+            const uint4 tail = __ldg(reinterpret_cast<const uint4*>(np + 2));
+            const uint32_t nprim = tail.y & 0xffffu, axis = (tail.y >> 16) & 0xffu;
+            bool descend = false;
+            if (box_lb(q.x, q.y, q.z, lo.x, lo.y, lo.z, hi.x, hi.y, hi.z) <= best.d2) {
+                if (nprim > 0) {
+                    for (uint32_t k = 0; k < nprim; ++k) {
+                        const float4* tp = reinterpret_cast<const float4*>(s.tris + tail.x + k);
+                        const float4 a = __ldg(tp), b = __ldg(tp + 5), c = __ldg(tp + 10);   // positions at +0, +80, +160 B
+                        float d2, u, v;
+                        closest_on_triangle(q.x, q.y, q.z, a.x, a.y, a.z, b.x, b.y, b.z, c.x, c.y, c.z, d2, u, v);
+                        point_take(best, d2, u, v, tail.x + k);
+                    }
+                } else {
+                    descend = true;
+                    const float pa = axis == 0 ? q.x : (axis == 1 ? q.y : q.z);
+                    const float mid = axis == 0 ? xadd(lo.x, hi.x) : (axis == 1 ? xadd(lo.y, hi.y) : xadd(lo.z, hi.z));
+                    const bool second_first = xadd(pa, pa) > mid;
+                    if (sp < CAP) stack[sp++] = second_first ? cur + 1u : tail.x;
+                    else report_stack_overflow();
+                    cur = second_first ? tail.x : cur + 1u;
+                }
+            }
+            if (!descend) {
+                if (sp == 0) break;
+                cur = stack[--sp];
+            }
+        }
+    }
+    out[i] = make_float4(best.d2, best.u, best.v, __uint_as_float(best.tri));
+}
+
+// ---------------------------------------------------------------------------------------
 // Launch wrappers (host).
 // ---------------------------------------------------------------------------------------
 static int pick_cap(uint32_t bound) { return bound <= 32 ? 32 : (bound <= 64 ? 64 : (bound <= 128 ? 128 : (bound <= 256 ? 256 : 0))); }
@@ -934,6 +1055,49 @@ cudaError_t launch_tonemap_rgba8(const void* d_image, void* d_out, uint64_t n, c
     uint64_t blocks = (n + 255) / 256;
     if (blocks > 0x7fffffffull) return cudaErrorInvalidValue;
     tonemap_rgba8_kernel<<<(unsigned)blocks, 256, 0, st>>>(static_cast<const float4*>(d_image), static_cast<uchar4*>(d_out), n);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_closest_point(const SceneView& s, const void* d_queries, uint64_t n, void* d_out, bool count, uint32_t stack_bound,
+                                 int grid_blocks, unsigned long long* d_next, unsigned long long* d_counters, uint32_t refill_min,
+                                 cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    const int cap = pick_cap(stack_bound);
+    if (!cap || grid_blocks < 1) return cudaErrorInvalidValue;
+    cudaError_t e = cudaMemsetAsync(d_next, 0, sizeof(unsigned long long), st);
+    if (e != cudaSuccess) return e;
+    if (refill_min < 1 || refill_min > 32) refill_min = 8;
+    const uint64_t warps = (uint64_t)grid_blocks * (POINT_BLOCK / 32), c = n / (warps * 8u + 1u);
+    const uint32_t chunk = (uint32_t)(c < 32 ? 32 : (c > 512 ? 512 : (c & ~31ull)));
+    const float4* q = static_cast<const float4*>(d_queries);
+    float4* out = static_cast<float4*>(d_out);
+#define B2_POINT_LAUNCH(C) (count ? point_persistent<true, C><<<grid_blocks, POINT_BLOCK, 0, st>>>(s, q, n, out, d_next, d_counters, chunk, refill_min) \
+                                  : point_persistent<false, C><<<grid_blocks, POINT_BLOCK, 0, st>>>(s, q, n, out, d_next, d_counters, chunk, refill_min))
+    switch (cap) {
+        case 32: B2_POINT_LAUNCH(32); break;
+        case 64: B2_POINT_LAUNCH(64); break;
+        case 128: B2_POINT_LAUNCH(128); break;
+        case 256: B2_POINT_LAUNCH(256); break;
+        default: return cudaErrorInvalidValue;
+    }
+#undef B2_POINT_LAUNCH
+    return cudaGetLastError();
+}
+
+cudaError_t launch_closest_point_binary(const SceneView& s, const void* d_queries, uint64_t n, void* d_out, uint32_t max_depth_binary,
+                                        cudaStream_t st) {
+    if (n == 0) return cudaSuccess;
+    const uint64_t blocks = (n + 127) / 128;
+    if (blocks > 0x7fffffffull) return cudaErrorInvalidValue;
+    const float4* q = static_cast<const float4*>(d_queries);
+    float4* out = static_cast<float4*>(d_out);
+    switch (pick_cap(max_depth_binary > 1u ? max_depth_binary : 1u)) {
+        case 32: point_binary_kernel<32><<<(unsigned)blocks, 128, 0, st>>>(s, q, n, out); break;
+        case 64: point_binary_kernel<64><<<(unsigned)blocks, 128, 0, st>>>(s, q, n, out); break;
+        case 128: point_binary_kernel<128><<<(unsigned)blocks, 128, 0, st>>>(s, q, n, out); break;
+        case 256: point_binary_kernel<256><<<(unsigned)blocks, 128, 0, st>>>(s, q, n, out); break;
+        default: return cudaErrorInvalidValue;
+    }
     return cudaGetLastError();
 }
 

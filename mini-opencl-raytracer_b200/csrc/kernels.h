@@ -57,6 +57,14 @@ cudaError_t launch_trace_multi(const SceneView& s, const void* d_rays, uint64_t 
 // ... and the same over the reference-layout arrays, one thread per ray.
 cudaError_t launch_trace_binary_multi(const SceneView& s, const void* d_rays, uint64_t n, uint32_t k, void* d_out, uint32_t max_depth_binary,
                                       cudaStream_t st);
+// Closest point per query (b2rt_closest_point): d_queries = b2rt_point_query[n], d_out = b2rt_point_hit[n]. The persistent
+// kernel over the compressed wide BVH (d_next: one 64-bit scratch counter, reset here) ...
+cudaError_t launch_closest_point(const SceneView& s, const void* d_queries, uint64_t n, void* d_out, bool count, uint32_t stack_bound,
+                                 int grid_blocks, unsigned long long* d_next, unsigned long long* d_counters, uint32_t refill_min,
+                                 cudaStream_t st);
+// ... and the same over the reference-layout arrays, one thread per query.
+cudaError_t launch_closest_point_binary(const SceneView& s, const void* d_queries, uint64_t n, void* d_out, uint32_t max_depth_binary,
+                                        cudaStream_t st);
 cudaError_t launch_camera_rays(const FrameArgs& a, uint64_t gid0, uint64_t gid1, void* d_rays, cudaStream_t st);
 // KernelEntry for the n pixels map.gid(0..n-1), one thread per pixel; binary: over the reference-layout arrays.
 cudaError_t launch_render_mega(const SceneView& s, const FrameArgs& a, float* d_result, const GidMap& map, uint32_t n,

@@ -354,6 +354,20 @@ int group_trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* 
     });
 }
 
+int group_point_host(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out) {
+    Group* g = ctx->group;
+    int st = use_device(ctx);
+    if (st) return st;
+    st = ensure_scene(ctx);
+    if (st) return st;
+    const uint64_t world = g->members.size();
+    return run_members(ctx, [&](b2rt_context* m, int k) {
+        const uint64_t lo = n * (uint64_t)k / world, hi = n * (uint64_t)(k + 1) / world;     // contiguous ranges, as for rays
+        if (hi == lo) return (int)B2RT_SUCCESS;
+        return point_host(m, q + lo, hi - lo, out + lo);
+    });
+}
+
 const std::vector<b2rt_context*>& group_members(const b2rt_context* ctx) { return ctx->group->members; }
 
 int group_finish(b2rt_context* ctx) {

@@ -7,7 +7,7 @@ import os
 import numpy as np
 
 from . import capi
-from .layouts import HIT_DTYPE, RAY_DTYPE
+from .layouts import HIT_DTYPE, POINT_HIT_DTYPE, POINT_QUERY_DTYPE, RAY_DTYPE
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
@@ -63,6 +63,7 @@ def lib():
         "g3d_engine_trace_closest": (C.c_int, [vp, vp, u64, vp, cs, sz]),
         "g3d_engine_trace_any": (C.c_int, [vp, vp, u64, vp, cs, sz]),
         "g3d_engine_trace_multi": (C.c_int, [vp, vp, u64, C.c_uint32, vp, cs, sz]),
+        "g3d_engine_closest_point": (C.c_int, [vp, vp, u64, vp, cs, sz]),
         "g3d_write_icosphere_obj": (C.c_longlong, [cs, C.c_int, C.c_double, C.c_double, C.c_ulonglong]),
         "g3d_write_scattered_obj": (C.c_longlong, [cs, C.c_longlong, C.c_double, C.c_double, C.c_double, C.c_ulonglong]),
     }
@@ -283,3 +284,11 @@ class Engine:
         e = _err()
         self._ck(self._L.g3d_engine_trace_multi(self._h, rays.ctypes.data, rays.shape[0], int(k), hits.ctypes.data, e, len(e)), e)
         return hits
+
+    def closest_point(self, queries):
+        """CLRaytracer::ClosestPoint: the nearest surface point of the scene to every query as a POINT_HIT_DTYPE array."""
+        queries = np.ascontiguousarray(queries, dtype=POINT_QUERY_DTYPE)
+        out = np.empty(queries.shape[0], dtype=POINT_HIT_DTYPE)
+        e = _err()
+        self._ck(self._L.g3d_engine_closest_point(self._h, queries.ctypes.data, queries.shape[0], out.ctypes.data, e, len(e)), e)
+        return out

@@ -252,3 +252,10 @@ extern "C" int g3d_engine_trace_multi(void* engine, const b2rt_ray* rays, uint64
     return 0;
     G3D_CATCH(-1)
 }
+extern "C" int g3d_engine_closest_point(void* engine, const b2rt_point_query* queries, uint64_t n, b2rt_point_hit* out, char* err, size_t errLen)
+{
+    G3D_TRY
+    static_cast<EngineBox*>(engine)->engine->render->ClosestPoint(queries, n, out);
+    return 0;
+    G3D_CATCH(-1)
+}

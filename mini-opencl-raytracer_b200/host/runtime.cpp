@@ -167,6 +167,11 @@ namespace Glaze3D
         int st = b2rt_trace_multi(m_CLContext->GetContext(), rays, n, k, hits);
         if (st) throw CLException(std::string("Failed to trace rays: ") + b2rt_last_error(m_CLContext->GetContext()), st);
     }
+    void CLRaytracer::ClosestPoint(const b2rt_point_query* queries, uint64_t n, b2rt_point_hit* out)
+    {
+        int st = b2rt_closest_point(m_CLContext->GetContext(), queries, n, out);
+        if (st) throw CLException(std::string("Failed to query closest points: ") + b2rt_last_error(m_CLContext->GetContext()), st);
+    }
 
     // ---- CLEngineBase (headless) -------------------------------------------------------------------
     CLEngineBase::CLEngineBase()

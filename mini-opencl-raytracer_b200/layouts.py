@@ -8,6 +8,10 @@ RAY_DTYPE = np.dtype([("ox", "<f4"), ("oy", "<f4"), ("oz", "<f4"), ("tmin", "<f4
                       ("dx", "<f4"), ("dy", "<f4"), ("dz", "<f4"), ("tmax", "<f4")])
 HIT_DTYPE = np.dtype([("t", "<f4"), ("u", "<f4"), ("v", "<f4"), ("tri", "<u4")])
 assert RAY_DTYPE.itemsize == 32 and HIT_DTYPE.itemsize == 16
+# b2rt_closest_point records: a query point with its search radius squared, and the nearest surface point found
+POINT_QUERY_DTYPE = np.dtype([("x", "<f4"), ("y", "<f4"), ("z", "<f4"), ("max_d2", "<f4")])
+POINT_HIT_DTYPE = np.dtype([("d2", "<f4"), ("u", "<f4"), ("v", "<f4"), ("tri", "<u4")])
+assert POINT_QUERY_DTYPE.itemsize == 16 and POINT_HIT_DTYPE.itemsize == 16
 
 # CLLinearBVHNode, 48 B
 NODE_DTYPE = np.dtype({"names": ["bmin", "bmax", "offset", "nPrimitives", "axis"],

@@ -21,6 +21,8 @@ KERNELS = {
     "wf_shade_kernel": "wf_shade_kernel",
     "wf_generate_kernel": "wf_generate_kernel",
     "render_mega_kernel<wide, CAP 64>": "render_mega_kernelILb0ELi64E",
+    "point_persistent<no counters, CAP 64>": "point_persistentILb0ELi64E",
+    "point_binary_kernel<CAP 64>": "point_binary_kernelILi64E",
 }
 
 
