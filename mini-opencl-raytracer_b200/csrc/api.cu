@@ -302,6 +302,23 @@ static int binary_walk_fits(b2rt_context* ctx) {
     return fail(ctx, B2RT_OUT_OF_RESOURCES, "BVH too deep for the reference-layout walk's stack (binary depth " + std::to_string(ctx->info.max_depth_binary) + ")");
 }
 
+// Grid of a persistent launch over n items: the scene's occupancy grid `base`, or B2RT_OPT_BLOCKS_PER_SM blocks per SM when
+// set; `share` wavefronts running side by side each take their part of it (whole CTAs per SM); never more blocks than the
+// n items fill.
+static int persistent_grid(b2rt_context* ctx, int base, uint64_t n, int share = 1) {
+    int grid = ctx->opt_blocks_per_sm > 0 ? ctx->sm_count * (int)ctx->opt_blocks_per_sm : base;
+    if (share > 1) grid = ctx->sm_count * std::max(1, grid / ctx->sm_count / share);
+    const uint64_t blocks_needed = (n + trace_block_threads() - 1) / trace_block_threads();
+    return (uint64_t)grid > blocks_needed ? (int)blocks_needed : grid;
+}
+
+// B2RT_OPT_LEAF_BIAS, or the default measured for the hit policy
+static uint32_t leaf_bias(const b2rt_context* ctx, bool any) { return (uint32_t)(ctx->opt_leaf_bias ? ctx->opt_leaf_bias : (any ? 48 : 32)); }
+
+// Every launch pulls its items from its OWN counter block (a ring of NEXT_RING): launches on different caller streams may
+// overlap, and a shared counter would be reset under a running kernel. Counts the launch in next_seq.
+static unsigned long long* take_next(b2rt_context* ctx) { return ctx->d_next + 8 * (ctx->next_seq++ % NEXT_RING); }
+
 // k > 0: the k nearest hits per ray (b2rt_trace_multi), d_out = b2rt_hit[n * k]; `any` is then ignored.
 int trace_device(b2rt_context* ctx, const void* d_rays, uint64_t n, void* d_out, bool any, cudaStream_t st, uint32_t k = 0) {
     if (n == 0) return B2RT_SUCCESS;
@@ -314,21 +331,15 @@ int trace_device(b2rt_context* ctx, const void* d_rays, uint64_t n, void* d_out,
         ctx->launches += 1;
         return B2RT_SUCCESS;
     }
-    int grid = (any && !k) ? ctx->grid_any : ctx->grid_closest;
-    if (ctx->opt_blocks_per_sm > 0) grid = ctx->sm_count * (int)ctx->opt_blocks_per_sm;
-    uint64_t warps_needed = (n + 31) / 32, blocks_needed = (warps_needed * 32 + trace_block_threads() - 1) / trace_block_threads();
-    if ((uint64_t)grid > blocks_needed) grid = (int)blocks_needed;
-    // every launch pulls rays from its OWN counter (a ring of NEXT_RING slots): launches on different caller streams may
-    // overlap, and a shared counter would be reset under a running kernel
+    const int grid = persistent_grid(ctx, (any && !k) ? ctx->grid_any : ctx->grid_closest, n);
     int st_pol = apply_l2_policy(ctx, st);
     if (st_pol) return st_pol;
-    const uint64_t seq = ctx->next_seq++;
-    unsigned long long* next = ctx->d_next + 8 * (seq % NEXT_RING);
+    unsigned long long* next = take_next(ctx);
     if (k) {
         // no cooperative tail: the tail hand-over would need the row list in its record (B2RT_OPT_COOP_MAX and
         // B2RT_OPT_RESUME_MAX do not apply)
         CK(launch_trace_multi(ctx->view, d_rays, n, k, d_out, ctx->opt_counters != 0, ctx->stack_bound, grid, next, ctx->d_counters,
-                              (uint32_t)ctx->opt_refill_min, (uint32_t)(ctx->opt_leaf_bias ? ctx->opt_leaf_bias : 32), st));
+                              (uint32_t)ctx->opt_refill_min, leaf_bias(ctx, false), st));
         ctx->launches += 1;
         return B2RT_SUCCESS;
     }
@@ -346,12 +357,12 @@ int trace_device(b2rt_context* ctx, const void* d_rays, uint64_t n, void* d_out,
         for (int i = 1; i < TAIL_RING; ++i) if (ctx->tail_slot_used[i] < ctx->tail_slot_used[slot]) slot = i;
         ctx->tail_slot_stream[slot] = sid;
     }
-    ctx->tail_slot_used[slot] = seq + 1;
+    ctx->tail_slot_used[slot] = ctx->next_seq;                 // this launch's number + 1 (take_next counted it)
     TailQueue tail;
     int st_tail = tail_queue(ctx, slot, next + 1, next + 2, tail);
     if (st_tail) return st_tail;
     CK(launch_trace_wide(ctx->view, d_rays, n, d_out, any, ctx->opt_counters != 0, ctx->stack_bound, grid, next,
-                         ctx->d_counters, (uint32_t)ctx->opt_refill_min, (uint32_t)(ctx->opt_leaf_bias ? ctx->opt_leaf_bias : (any ? 48 : 32)), st, nullptr, &tail, ctx->grid_tail));
+                         ctx->d_counters, (uint32_t)ctx->opt_refill_min, leaf_bias(ctx, any), st, nullptr, &tail, ctx->grid_tail));
     ctx->launches += tail.coop_max ? (tail.resume_max ? 3 : 2) : 1;
     return B2RT_SUCCESS;
 }
@@ -367,13 +378,10 @@ int point_device(b2rt_context* ctx, const void* d_q, uint64_t n, void* d_out, cu
         ctx->launches += 1;
         return B2RT_SUCCESS;
     }
-    int grid = ctx->grid_closest;
-    if (ctx->opt_blocks_per_sm > 0) grid = ctx->sm_count * (int)ctx->opt_blocks_per_sm;
-    const uint64_t blocks_needed = ((n + 31) / 32 * 32 + trace_block_threads() - 1) / trace_block_threads();
-    if ((uint64_t)grid > blocks_needed) grid = (int)blocks_needed;
+    const int grid = persistent_grid(ctx, ctx->grid_closest, n);
     int st_pol = apply_l2_policy(ctx, st);
     if (st_pol) return st_pol;
-    unsigned long long* next = ctx->d_next + 8 * (ctx->next_seq++ % NEXT_RING);     // a counter of its own, as for rays
+    unsigned long long* next = take_next(ctx);
     CK(launch_closest_point(ctx->view, d_q, n, d_out, ctx->opt_counters != 0, ctx->stack_bound, grid, next, ctx->d_counters,
                             (uint32_t)ctx->opt_refill_min, st));
     ctx->launches += 1;
@@ -400,21 +408,26 @@ int ensure_staging(b2rt_context* ctx, uint64_t chunk, size_t out_bytes) {
     return B2RT_SUCCESS;
 }
 
-// Host-buffer ray stream: chunks are copied in, traced and copied out on three streams so
-// that PCIe transfers overlap the traversal kernels. k > 0: k hits per ray (see trace_device).
-int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any, uint32_t k) {
+// Items per pipelined chunk of the host-buffer entries; B2RT_STREAM_CHUNK (at least 1024) overrides it as a tuning aid.
+static uint64_t stream_chunk() {
+    if (const char* env = getenv("B2RT_STREAM_CHUNK")) { long long v = atoll(env); if (v >= 1024) return (uint64_t)v; }
+    return STREAM_CHUNK;
+}
+
+// Host-buffer query stream: chunks of at most `chunk_cap` records of `in_elem` bytes (at most a b2rt_ray) are copied in,
+// run through launch(d_in, m, d_out, stream) and their `out_elem`-byte results copied out, on three streams so that PCIe
+// transfers overlap the kernels. The output staging holds at least a chunk of b2rt_hit, so that every query kind fits the
+// same staging buffers without reallocating. `what` names the input in the NULL-pointer error.
+template <class Launch>
+static int host_pipeline(b2rt_context* ctx, const void* in, size_t in_elem, uint64_t n, void* out, size_t out_elem, uint64_t chunk_cap,
+                         const char* what, Launch&& launch) {
     int st = use_device(ctx);
     if (st) return st;
     st = ensure_scene(ctx);
     if (st) return st;
     if (n == 0) return B2RT_SUCCESS;
-    if (!rays || !out) return fail(ctx, B2RT_INVALID_VALUE, "null ray or output pointer");
-    uint64_t chunk_rays = STREAM_CHUNK;
-    if (const char* env = getenv("B2RT_STREAM_CHUNK")) { long long v = atoll(env); if (v >= 1024) chunk_rays = (uint64_t)v; }   // tuning aid
-    // k hits per ray: the chunk shrinks with k, so that the output staging stays that of a closest-hit chunk
-    if (k > 1) chunk_rays = std::max<uint64_t>(chunk_rays / k, 1024);
-    uint64_t chunk = std::min<uint64_t>(n, chunk_rays);
-    const size_t out_elem = k ? (size_t)k * sizeof(b2rt_hit) : (any ? sizeof(uint32_t) : sizeof(b2rt_hit));
+    if (!in || !out) return fail(ctx, B2RT_INVALID_VALUE, std::string("null ") + what + " or output pointer");
+    const uint64_t chunk = std::min<uint64_t>(n, chunk_cap);
     st = ensure_staging(ctx, chunk, chunk * std::max(out_elem, sizeof(b2rt_hit)));
     if (st) return st;
     // Chunk sizes ramp up from `ramp` to `chunk` and back down at the end: the first copy-in and the last kernel +
@@ -422,22 +435,21 @@ int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, b
     const uint64_t ramp = std::min<uint64_t>(chunk, 1ull << 19);
     uint64_t c = 0, m = 0;
     for (uint64_t off = 0; off < n; off += m, ++c) {
-        int s = (int)(c & 1);
+        const int s = (int)(c & 1);
         const uint64_t left = n - off;
         m = std::min<uint64_t>(chunk, ramp << std::min<uint64_t>(c, 16));                              // ramp up
         if (left <= ramp) m = left;
         else m = std::min<uint64_t>(m, std::max<uint64_t>(ramp, (left / 2 + 31) & ~31ull));            // ramp down: at most half of what is left
-        if (c >= 2) CK(cudaStreamWaitEvent(ctx->stream_in, ctx->ev_comp[s], 0));     // rays[s] free again
-        CK(cudaMemcpyAsync(ctx->d_stage_rays[s], rays + off, m * sizeof(b2rt_ray), cudaMemcpyHostToDevice, ctx->stream_in));
+        if (c >= 2) CK(cudaStreamWaitEvent(ctx->stream_in, ctx->ev_comp[s], 0));     // in[s] free again
+        CK(cudaMemcpyAsync(ctx->d_stage_rays[s], static_cast<const char*>(in) + off * in_elem, m * in_elem, cudaMemcpyHostToDevice, ctx->stream_in));
         CK(cudaEventRecord(ctx->ev_in[s], ctx->stream_in));
         CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[s], 0));
         if (c >= 2) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[s], 0));         // out[s] drained
-        st = trace_device(ctx, ctx->d_stage_rays[s], m, ctx->d_stage_out[s], any, ctx->stream, k);
+        st = launch(ctx->d_stage_rays[s], m, ctx->d_stage_out[s], ctx->stream);
         if (st) return st;
         CK(cudaEventRecord(ctx->ev_comp[s], ctx->stream));
         CK(cudaStreamWaitEvent(ctx->stream_out, ctx->ev_comp[s], 0));
-        CK(cudaMemcpyAsync(static_cast<char*>(out) + off * out_elem, ctx->d_stage_out[s], m * out_elem,
-                           cudaMemcpyDeviceToHost, ctx->stream_out));
+        CK(cudaMemcpyAsync(static_cast<char*>(out) + off * out_elem, ctx->d_stage_out[s], m * out_elem, cudaMemcpyDeviceToHost, ctx->stream_out));
         CK(cudaEventRecord(ctx->ev_out[s], ctx->stream_out));
     }
     CK(cudaStreamSynchronize(ctx->stream_out));
@@ -445,43 +457,21 @@ int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, b
     return B2RT_SUCCESS;
 }
 
-// Host-buffer closest-point queries: the pipeline of trace_host with 16-byte queries and records (a staging buffer sized
-// for a chunk of rays holds a chunk of queries).
-int point_host(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out) {
-    int st = use_device(ctx);
-    if (st) return st;
-    st = ensure_scene(ctx);
-    if (st) return st;
-    if (n == 0) return B2RT_SUCCESS;
-    if (!q || !out) return fail(ctx, B2RT_INVALID_VALUE, "null query or output pointer");
-    uint64_t chunk_q = STREAM_CHUNK;
-    if (const char* env = getenv("B2RT_STREAM_CHUNK")) { long long v = atoll(env); if (v >= 1024) chunk_q = (uint64_t)v; }
-    const uint64_t chunk = std::min<uint64_t>(n, chunk_q);
-    st = ensure_staging(ctx, chunk, chunk * sizeof(b2rt_point_hit));
-    if (st) return st;
-    const uint64_t ramp = std::min<uint64_t>(chunk, 1ull << 19);
-    uint64_t c = 0, m = 0;
-    for (uint64_t off = 0; off < n; off += m, ++c) {
-        const int s = (int)(c & 1);
-        const uint64_t left = n - off;
-        m = std::min<uint64_t>(chunk, ramp << std::min<uint64_t>(c, 16));
-        if (left <= ramp) m = left;
-        else m = std::min<uint64_t>(m, std::max<uint64_t>(ramp, (left / 2 + 31) & ~31ull));
-        if (c >= 2) CK(cudaStreamWaitEvent(ctx->stream_in, ctx->ev_comp[s], 0));
-        CK(cudaMemcpyAsync(ctx->d_stage_rays[s], q + off, m * sizeof(b2rt_point_query), cudaMemcpyHostToDevice, ctx->stream_in));
-        CK(cudaEventRecord(ctx->ev_in[s], ctx->stream_in));
-        CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[s], 0));
-        if (c >= 2) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[s], 0));
-        st = point_device(ctx, ctx->d_stage_rays[s], m, ctx->d_stage_out[s], ctx->stream);
-        if (st) return st;
-        CK(cudaEventRecord(ctx->ev_comp[s], ctx->stream));
-        CK(cudaStreamWaitEvent(ctx->stream_out, ctx->ev_comp[s], 0));
-        CK(cudaMemcpyAsync(out + off, ctx->d_stage_out[s], m * sizeof(b2rt_point_hit), cudaMemcpyDeviceToHost, ctx->stream_out));
-        CK(cudaEventRecord(ctx->ev_out[s], ctx->stream_out));
-    }
-    CK(cudaStreamSynchronize(ctx->stream_out));
-    CK(cudaStreamSynchronize(ctx->stream));
-    return B2RT_SUCCESS;
+// Host-buffer ray stream on one device. k > 0: k hits per ray (see trace_device); the chunk then shrinks with k, so that
+// the output staging stays that of a closest-hit chunk.
+static int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any, uint32_t k = 0) {
+    uint64_t chunk = stream_chunk();
+    if (k > 1) chunk = std::max<uint64_t>(chunk / k, 1024);
+    const size_t out_elem = k ? (size_t)k * sizeof(b2rt_hit) : (any ? sizeof(uint32_t) : sizeof(b2rt_hit));
+    return host_pipeline(ctx, rays, sizeof(b2rt_ray), n, out, out_elem, chunk, "ray", [&](const void* d_in, uint64_t m, void* d_out, cudaStream_t s) {
+        return trace_device(ctx, d_in, m, d_out, any, s, k);
+    });
+}
+
+// Host-buffer closest-point queries on one device.
+static int point_host(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out) {
+    return host_pipeline(ctx, q, sizeof(b2rt_point_query), n, out, sizeof(b2rt_point_hit), stream_chunk(), "query",
+                         [&](const void* d_in, uint64_t m, void* d_out, cudaStream_t s) { return point_device(ctx, d_in, m, d_out, s); });
 }
 
 int frame_args(b2rt_context* ctx, FrameArgs& a);
@@ -543,16 +533,10 @@ int wavefront_lane(b2rt_context* ctx, const FrameArgs& a, float* d_result, const
     CK(launch_wf_generate(a, map, n, rays[0], state, cnt, s));        // also resets the lane's four counters
     ctx->launches += 1;
     STAGE(B2RT_STAGE_GENERATE);
-    int grid = ctx->grid_closest;
-    if (ctx->opt_blocks_per_sm > 0) grid = ctx->sm_count * (int)ctx->opt_blocks_per_sm;
     // `share` wavefronts run side by side: each takes its part of the CTA slots (whole CTAs per SM)
+    const int grid = persistent_grid(ctx, ctx->grid_closest, n, share);
     int tail_grid = ctx->grid_tail;
-    if (share > 1) {
-        grid = ctx->sm_count * std::max(1, grid / ctx->sm_count / share);
-        tail_grid = ctx->sm_count * std::max(1, tail_grid / ctx->sm_count / share);
-    }
-    uint64_t blocks_needed = ((uint64_t)n + trace_block_threads() - 1) / trace_block_threads();
-    if ((uint64_t)grid > blocks_needed) grid = (int)blocks_needed;
+    if (share > 1) tail_grid = ctx->sm_count * std::max(1, tail_grid / ctx->sm_count / share);
     TailQueue tail;
     int tq = tail_queue(ctx, TAIL_RING + lane, cnt + 4, cnt + 5, tail);
     if (tq) return tq;
@@ -561,7 +545,7 @@ int wavefront_lane(b2rt_context* ctx, const FrameArgs& a, float* d_result, const
         unsigned long long *n_in = cnt + (b % 3), *n_out = cnt + ((b + 1) % 3), *n_clear = cnt + ((b + 2) % 3);
         if (b) tail.tag = tail_tag(ctx);
         CK(launch_trace_wide(ctx->view, rays[in], n, hits, false, ctx->opt_counters != 0, ctx->stack_bound, grid,
-                             cnt + 3, ctx->d_counters, (uint32_t)ctx->opt_refill_min, (uint32_t)(ctx->opt_leaf_bias ? ctx->opt_leaf_bias : 32), s, n_in, &tail, tail_grid,
+                             cnt + 3, ctx->d_counters, (uint32_t)ctx->opt_refill_min, leaf_bias(ctx, false), s, n_in, &tail, tail_grid,
                              stage_mark(ctx, timed, B2RT_STAGE_TRACE, s)));
         STAGE(B2RT_STAGE_TAIL);
         // the shade stage also clears the counter the NEXT shade stage appends to and the traversal kernels' three counters
@@ -725,13 +709,18 @@ int render_with_mode(b2rt_context* ctx, const FrameArgs& a, float* result, const
     return B2RT_SUCCESS;
 }
 
+// The camera part of FrameArgs: frames and b2rt_camera_rays_device make their primary rays from the same values.
+static void camera_args(const b2rt_context* ctx, FrameArgs& a) {
+    a.width = ctx->width; a.height = ctx->height; a.frame_count = ctx->frame_count;
+    for (int k = 0; k < 3; ++k) { a.pos[k] = ctx->cam_pos[k]; a.front[k] = ctx->cam_front[k]; a.up[k] = ctx->cam_up[k]; }
+    a.angle = tanf(0.5f * (45.0f * 3.1415f / 180.0f));   // kernel_bvh.cl:392, evaluated by the host libm like the oracle
+}
+
 int frame_args(b2rt_context* ctx, FrameArgs& a) {
     for (int i = 0; i < B2RT_ARG_COUNT; ++i)
         if (!ctx->arg_set[i]) return fail(ctx, B2RT_INVALID_KERNEL_ARGS, "kernel argument " + std::to_string(i) + " was never set");
-    a.width = ctx->width; a.height = ctx->height; a.frame_count = ctx->frame_count;
+    camera_args(ctx, a);
     a.bounces = ctx->bounces; a.light_type = ctx->light_type; a.sky = ctx->sky;
-    for (int k = 0; k < 3; ++k) { a.pos[k] = ctx->cam_pos[k]; a.front[k] = ctx->cam_front[k]; a.up[k] = ctx->cam_up[k]; }
-    a.angle = tanf(0.5f * (45.0f * 3.1415f / 180.0f));   // kernel_bvh.cl:392, evaluated by the host libm like the oracle
     a.mirror = ctx->mirror;
     if (a.width == 0 || a.height == 0) return fail(ctx, B2RT_INVALID_KERNEL_ARGS, "WIDTH/HEIGHT must be non-zero");
     return B2RT_SUCCESS;
@@ -1224,31 +1213,37 @@ extern "C" int b2rt_build_bvh(b2rt_context* ctx, const void* triangles, uint64_t
 }
 
 // ---- ray streams -----------------------------------------------------------------------------
+// Host-buffer entries: a device group cuts the items into one contiguous range per member.
 extern "C" int b2rt_trace_closest(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, b2rt_hit* hits) {
     if (!ctx) return B2RT_INVALID_CONTEXT;
-    if (ctx->group) return group_trace_host(ctx, rays, n, hits, false);      // contiguous ranges, one per device
+    if (ctx->group) return group_split(ctx, n, [&](b2rt_context* m, uint64_t lo, uint64_t cnt) { return trace_host(m, rays + lo, cnt, hits + lo, false); });
     return trace_host(ctx, rays, n, hits, false);
 }
 extern "C" int b2rt_trace_any(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, uint32_t* occluded) {
     if (!ctx) return B2RT_INVALID_CONTEXT;
-    if (ctx->group) return group_trace_host(ctx, rays, n, occluded, true);
+    if (ctx->group) return group_split(ctx, n, [&](b2rt_context* m, uint64_t lo, uint64_t cnt) { return trace_host(m, rays + lo, cnt, occluded + lo, true); });
     return trace_host(ctx, rays, n, occluded, true);
+}
+// Device-buffer entries: the handle's device current and its scene built; a NULL stream means the context's stream.
+static int device_entry(b2rt_context* ctx, void* cuda_stream, cudaStream_t* st) {
+    int s = use_device(ctx);
+    if (s) return s;
+    s = ensure_scene(ctx);
+    if (s) return s;
+    *st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream;
+    return B2RT_SUCCESS;
 }
 extern "C" int b2rt_trace_closest_device(b2rt_context* ctx, const b2rt_ray* d_rays, uint64_t n, b2rt_hit* d_hits, void* cuda_stream) {
     if (!ctx) return B2RT_INVALID_CONTEXT;
-    int st = use_device(ctx);
-    if (st) return st;
-    st = ensure_scene(ctx);
-    if (st) return st;
-    return trace_device(ctx, d_rays, n, d_hits, false, cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream);
+    cudaStream_t s;
+    int st = device_entry(ctx, cuda_stream, &s);
+    return st ? st : trace_device(ctx, d_rays, n, d_hits, false, s);
 }
 extern "C" int b2rt_trace_any_device(b2rt_context* ctx, const b2rt_ray* d_rays, uint64_t n, uint32_t* d_occluded, void* cuda_stream) {
     if (!ctx) return B2RT_INVALID_CONTEXT;
-    int st = use_device(ctx);
-    if (st) return st;
-    st = ensure_scene(ctx);
-    if (st) return st;
-    return trace_device(ctx, d_rays, n, d_occluded, true, cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream);
+    cudaStream_t s;
+    int st = device_entry(ctx, cuda_stream, &s);
+    return st ? st : trace_device(ctx, d_rays, n, d_occluded, true, s);
 }
 // k nearest hits: k in [1, B2RT_MULTI_MAX_HITS] and no NULL pointer with n > 0, checked before anything is touched.
 static int multi_args(b2rt_context* ctx, const void* rays, uint64_t n, uint32_t k, const void* hits) {
@@ -1261,34 +1256,30 @@ extern "C" int b2rt_trace_multi(b2rt_context* ctx, const b2rt_ray* rays, uint64_
     if (!ctx) return B2RT_INVALID_CONTEXT;
     int st = multi_args(ctx, rays, n, k, hits);
     if (st) return st;
-    if (ctx->group) return group_trace_host(ctx, rays, n, hits, false, k);   // contiguous ranges, one per device
+    if (ctx->group) return group_split(ctx, n, [&](b2rt_context* m, uint64_t lo, uint64_t cnt) { return trace_host(m, rays + lo, cnt, hits + lo * k, false, k); });
     return trace_host(ctx, rays, n, hits, false, k);
 }
 extern "C" int b2rt_trace_multi_device(b2rt_context* ctx, const b2rt_ray* d_rays, uint64_t n, uint32_t k, b2rt_hit* d_hits, void* cuda_stream) {
     if (!ctx) return B2RT_INVALID_CONTEXT;
     int st = multi_args(ctx, d_rays, n, k, d_hits);
     if (st) return st;
-    st = use_device(ctx);
-    if (st) return st;
-    st = ensure_scene(ctx);
-    if (st) return st;
-    return trace_device(ctx, d_rays, n, d_hits, false, cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream, k);
+    cudaStream_t s;
+    st = device_entry(ctx, cuda_stream, &s);
+    return st ? st : trace_device(ctx, d_rays, n, d_hits, false, s, k);
 }
 // ---- closest point ----------------------------------------------------------------------------
 extern "C" int b2rt_closest_point(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out) {
     if (!ctx) return B2RT_INVALID_CONTEXT;
     if (n && (!q || !out)) return fail(ctx, B2RT_INVALID_VALUE, "null query or output pointer");
-    if (ctx->group) return group_point_host(ctx, q, n, out);                 // contiguous ranges, one per device
+    if (ctx->group) return group_split(ctx, n, [&](b2rt_context* m, uint64_t lo, uint64_t cnt) { return point_host(m, q + lo, cnt, out + lo); });
     return point_host(ctx, q, n, out);
 }
 extern "C" int b2rt_closest_point_device(b2rt_context* ctx, const b2rt_point_query* d_q, uint64_t n, b2rt_point_hit* d_out, void* cuda_stream) {
     if (!ctx) return B2RT_INVALID_CONTEXT;
     if (n && (!d_q || !d_out)) return fail(ctx, B2RT_INVALID_VALUE, "null query or output pointer");
-    int st = use_device(ctx);
-    if (st) return st;
-    st = ensure_scene(ctx);
-    if (st) return st;
-    return point_device(ctx, d_q, n, d_out, cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream);
+    cudaStream_t s;
+    int st = device_entry(ctx, cuda_stream, &s);
+    return st ? st : point_device(ctx, d_q, n, d_out, s);
 }
 extern "C" int b2rt_camera_rays_device(b2rt_context* ctx, size_t gid_begin, size_t gid_end, b2rt_ray* d_rays, void* cuda_stream) {
     if (!ctx) return B2RT_INVALID_CONTEXT;
@@ -1301,9 +1292,7 @@ extern "C" int b2rt_camera_rays_device(b2rt_context* ctx, size_t gid_begin, size
     if (gid_end < gid_begin || gid_end > 0xffffffffull || !d_rays) return fail(ctx, B2RT_INVALID_VALUE, "bad camera ray range");
     FrameArgs a;
     memset(&a, 0, sizeof(a));
-    a.width = ctx->width; a.height = ctx->height; a.frame_count = ctx->frame_count;
-    for (int k = 0; k < 3; ++k) { a.pos[k] = ctx->cam_pos[k]; a.front[k] = ctx->cam_front[k]; a.up[k] = ctx->cam_up[k]; }
-    a.angle = tanf(0.5f * (45.0f * 3.1415f / 180.0f));
+    camera_args(ctx, a);
     if (!a.width || !a.height) return fail(ctx, B2RT_INVALID_KERNEL_ARGS, "WIDTH/HEIGHT must be non-zero");
     CK(launch_camera_rays(a, gid_begin, gid_end, d_rays, cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->stream));
     ctx->launches += 1;

@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <functional>
 #include <map>
 #include <string>
 #include <unordered_map>
@@ -131,8 +132,6 @@ int install_scene(b2rt_context* ctx, const DerivedScene& d);
 // refit.cu: per-triangle shading records (normals + material) of `tris`
 cudaError_t launch_shade_records(b2rt::ShadeTri* shade, const b2rt::RefTriangle* tris, uint32_t n, cudaStream_t s);
 int render_items(b2rt_context* ctx, const b2rt::GidMap& map, uint64_t n);
-int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any, uint32_t k = 0);   // k > 0: k hits per ray
-int point_host(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out);            // b2rt_closest_point
 
 // multi.cu
 void group_destroy(b2rt_context* ctx);
@@ -141,8 +140,9 @@ int group_buffer_create(b2rt_context* ctx, uint32_t flags, size_t bytes, const v
 int group_each(b2rt_context* ctx, int (*fn)(b2rt_context*, void*), void* arg, bool parallel);
 int group_adopt_scene(b2rt_context* root);
 int group_execute(b2rt_context* ctx, size_t gid_begin, size_t gid_end);
-int group_trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any, uint32_t hits_per_ray = 0);   // > 0: b2rt_trace_multi
-int group_point_host(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out);      // b2rt_closest_point
+// Items [0, n) of a host-buffer entry: member k runs fn(member, first, count) over its contiguous range [n*k/world,
+// n*(k+1)/world); empty ranges are skipped.
+int group_split(b2rt_context* ctx, uint64_t n, const std::function<int(b2rt_context*, uint64_t, uint64_t)>& fn);
 int group_finish(b2rt_context* ctx);
 void group_bind_output(b2rt_context* ctx);
 int group_broadcast_buffer(b2rt_context* ctx, b2rt_buffer id);   // the root's contents of buffer `id` to every peer's copy

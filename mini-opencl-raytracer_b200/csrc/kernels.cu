@@ -27,6 +27,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <type_traits>
 #include "kernels.h"
 #include "shade.cuh"
 #include "coop.cuh"
@@ -877,32 +878,48 @@ point_binary_kernel(SceneView s, const float4* __restrict__ queries, uint64_t n,
 // ---------------------------------------------------------------------------------------
 static int pick_cap(uint32_t bound) { return bound <= 32 ? 32 : (bound <= 64 ? 64 : (bound <= 128 ? 128 : (bound <= 256 ? 256 : 0))); }
 
-template <int P, bool COUNT>
-static cudaError_t launch_persistent_cap(int cap, int grid, cudaStream_t st, const SceneView& s, const void* rays,
-                                         uint64_t n, void* out, unsigned long long* next, unsigned long long* counters,
-                                         uint32_t refill_min, uint32_t leaf_bias, const unsigned long long* n_dev, const TailQueue& tail,
-                                         const uint32_t* resume = nullptr, uint32_t k = 0) {
-    const RayIn* r = static_cast<const RayIn*>(rays);
-    // rays per pool top-up: about 1/8 of a warp's fair share, a multiple of 32 in [32, 512]
-    uint64_t warps = (uint64_t)grid * (TRACE_BLOCK / 32);
-    uint64_t c = n / (warps * 8u + 1u);
-    uint32_t chunk = (uint32_t)(c < 32 ? 32 : (c > 512 ? 512 : (c & ~31ull)));
-    switch (cap) {
-        case 32: trace_persistent<P, COUNT, 32><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume, k); break;
-        case 64: trace_persistent<P, COUNT, 64><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume, k); break;
-        case 128: trace_persistent<P, COUNT, 128><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume, k); break;
-        case 256: trace_persistent<P, COUNT, 256><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume, k); break;
+// Calls f(std::integral_constant<int, CAP>()) for the smallest stack capacity CAP that holds `bound` entries, then returns
+// the launch status; a bound past 256 has no kernel and returns cudaErrorInvalidValue.
+template <class F>
+static cudaError_t with_cap(uint32_t bound, F&& f) {
+    switch (pick_cap(bound)) {
+        case 32: f(std::integral_constant<int, 32>()); break;
+        case 64: f(std::integral_constant<int, 64>()); break;
+        case 128: f(std::integral_constant<int, 128>()); break;
+        case 256: f(std::integral_constant<int, 256>()); break;
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();
+}
+
+// Pool scheduling of the persistent kernels: items per pool top-up, about 1/8 of a warp's fair share, a multiple of 32
+// in [32, 512] ...
+static uint32_t pool_chunk(uint64_t n, int grid, int block) {
+    const uint64_t warps = (uint64_t)grid * (block / 32), c = n / (warps * 8u + 1u);
+    return (uint32_t)(c < 32 ? 32 : (c > 512 ? 512 : (c & ~31ull)));
+}
+// ... and the idle lanes that trigger a refill, 8 when out of range
+static uint32_t refill_or_default(uint32_t refill_min) { return (refill_min < 1 || refill_min > 32) ? 8u : refill_min; }
+
+template <int P, bool COUNT>
+static cudaError_t launch_persistent(uint32_t stack_bound, int grid, cudaStream_t st, const SceneView& s, const void* rays,
+                                     uint64_t n, void* out, unsigned long long* next, unsigned long long* counters,
+                                     uint32_t refill_min, uint32_t leaf_bias, const unsigned long long* n_dev, const TailQueue& tail,
+                                     const uint32_t* resume = nullptr, uint32_t k = 0) {
+    const RayIn* r = static_cast<const RayIn*>(rays);
+    const uint32_t chunk = pool_chunk(n, grid, TRACE_BLOCK);
+    refill_min = refill_or_default(refill_min);
+    if (leaf_bias < 1 || leaf_bias > 512) leaf_bias = 16;
+    return with_cap(stack_bound, [&](auto C) {
+        trace_persistent<P, COUNT, C><<<grid, TRACE_BLOCK, 0, st>>>(s, r, n, out, next, counters, chunk, refill_min, leaf_bias, n_dev, tail, resume, k);
+    });
 }
 
 cudaError_t launch_trace_wide(const SceneView& s, const void* d_rays, uint64_t n, void* d_out, bool any, bool count,
                               uint32_t stack_bound, int grid_blocks, unsigned long long* d_next,
                               unsigned long long* d_counters, uint32_t refill_min, uint32_t leaf_bias, cudaStream_t st,
                               const unsigned long long* d_n, const TailQueue* tail_in, int tail_grid, cudaEvent_t between) {
-    int cap = pick_cap(stack_bound);
-    if (!cap) return cudaErrorInvalidValue;
+    if (!pick_cap(stack_bound)) return cudaErrorInvalidValue;
     TailQueue tail = { nullptr, nullptr, nullptr, 0, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0, 0 };
     if (tail_in && tail_in->coop_max && tail_in->records) tail = *tail_in;
     const bool two_step = tail.coop_max && tail.resume_max && tail.records2;
@@ -911,8 +928,6 @@ cudaError_t launch_trace_wide(const SceneView& s, const void* d_rays, uint64_t n
         cudaError_t e = cudaMemsetAsync(d_next, 0, 8 * sizeof(unsigned long long), st);
         if (e != cudaSuccess) return e;
     }
-    if (refill_min < 1 || refill_min > 32) refill_min = 8;
-    if (leaf_bias < 1 || leaf_bias > 512) leaf_bias = 16;
     // what each pass hands over to: the first pass suspends into queue 1 (at resume_max live rays when a second pass follows)
     // helping: only when the helping warp's shared memory holds the tail kernel's frontier, and not in the two-step mode (its
     // first queue is the second pass's ray stream)
@@ -924,10 +939,10 @@ cudaError_t launch_trace_wide(const SceneView& s, const void* d_rays, uint64_t n
     TailQueue q2 = tail;
     if (two_step) { q2.count = tail.count2; q2.next = tail.next2; q2.records = tail.records2; }
     auto pass = [&](const unsigned long long* n_dev, unsigned long long* next, const TailQueue& q, const uint32_t* resume) -> cudaError_t {
-        if (any) return count ? launch_persistent_cap<HIT_ANY, true>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume)
-                              : launch_persistent_cap<HIT_ANY, false>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume);
-        return count ? launch_persistent_cap<HIT_CLOSEST, true>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume)
-                     : launch_persistent_cap<HIT_CLOSEST, false>(cap, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume);
+        if (any) return count ? launch_persistent<HIT_ANY, true>(stack_bound, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume)
+                              : launch_persistent<HIT_ANY, false>(stack_bound, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume);
+        return count ? launch_persistent<HIT_CLOSEST, true>(stack_bound, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume)
+                     : launch_persistent<HIT_CLOSEST, false>(stack_bound, grid_blocks, st, s, d_rays, n, d_out, next, d_counters, refill_min, leaf_bias, n_dev, q, resume);
     };
     cudaError_t e = pass(d_n, d_next, q1, nullptr);
     // second pass: the suspended rays are its ray stream (count and read position = queue 1's counters)
@@ -948,26 +963,17 @@ cudaError_t launch_trace_wide(const SceneView& s, const void* d_rays, uint64_t n
 cudaError_t launch_trace_multi(const SceneView& s, const void* d_rays, uint64_t n, uint32_t k, void* d_out, bool count,
                                uint32_t stack_bound, int grid_blocks, unsigned long long* d_next, unsigned long long* d_counters,
                                uint32_t refill_min, uint32_t leaf_bias, cudaStream_t st) {
-    const int cap = pick_cap(stack_bound);
-    if (!cap || k == 0) return cudaErrorInvalidValue;
+    if (!pick_cap(stack_bound) || k == 0) return cudaErrorInvalidValue;
     cudaError_t e = cudaMemsetAsync(d_next, 0, 8 * sizeof(unsigned long long), st);
     if (e != cudaSuccess) return e;
-    if (refill_min < 1 || refill_min > 32) refill_min = 8;
-    if (leaf_bias < 1 || leaf_bias > 512) leaf_bias = 16;
     const TailQueue none = { nullptr, nullptr, nullptr, 0, 0, 0, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0, 0 };
-    return count ? launch_persistent_cap<HIT_MULTI, true>(cap, grid_blocks, st, s, d_rays, n, d_out, d_next, d_counters, refill_min, leaf_bias, nullptr, none, nullptr, k)
-                 : launch_persistent_cap<HIT_MULTI, false>(cap, grid_blocks, st, s, d_rays, n, d_out, d_next, d_counters, refill_min, leaf_bias, nullptr, none, nullptr, k);
+    return count ? launch_persistent<HIT_MULTI, true>(stack_bound, grid_blocks, st, s, d_rays, n, d_out, d_next, d_counters, refill_min, leaf_bias, nullptr, none, nullptr, k)
+                 : launch_persistent<HIT_MULTI, false>(stack_bound, grid_blocks, st, s, d_rays, n, d_out, d_next, d_counters, refill_min, leaf_bias, nullptr, none, nullptr, k);
 }
 
 uint32_t trace_warp_smem_words() { return (B2_TAIL_HELP && B2_TAIL_CODE) ? (uint32_t)WARP_SMEM_WORDS : 0u; }
 uint32_t tail_frontier_words(uint32_t stack_bound) { uint32_t w = 4u * (stack_bound + 8u); return w < 256u ? 256u : w; }
 uint32_t tail_record_words(uint32_t stack_bound) { return TAIL_HEADER_WORDS + ((stack_bound + 8u + 3u) & ~3u); }
-
-template <int CAP>
-static void launch_binary_cap(bool any, unsigned blocks, cudaStream_t st, const SceneView& s, const RayIn* r, uint64_t n, void* out) {
-    if (any) trace_binary_kernel<true, CAP><<<blocks, 128, 0, st>>>(s, r, n, out);
-    else trace_binary_kernel<false, CAP><<<blocks, 128, 0, st>>>(s, r, n, out);
-}
 
 cudaError_t launch_trace_binary(const SceneView& s, const void* d_rays, uint64_t n, void* d_out, bool any, uint32_t max_depth_binary,
                                 cudaStream_t st) {
@@ -975,14 +981,10 @@ cudaError_t launch_trace_binary(const SceneView& s, const void* d_rays, uint64_t
     uint64_t blocks = (n + 127) / 128;
     if (blocks > 0x7fffffffull) return cudaErrorInvalidValue;
     const RayIn* r = static_cast<const RayIn*>(d_rays);
-    switch (pick_cap(max_depth_binary > 1u ? max_depth_binary : 1u)) {
-        case 32: launch_binary_cap<32>(any, (unsigned)blocks, st, s, r, n, d_out); break;
-        case 64: launch_binary_cap<64>(any, (unsigned)blocks, st, s, r, n, d_out); break;
-        case 128: launch_binary_cap<128>(any, (unsigned)blocks, st, s, r, n, d_out); break;
-        case 256: launch_binary_cap<256>(any, (unsigned)blocks, st, s, r, n, d_out); break;
-        default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
+    return with_cap(max_depth_binary, [&](auto C) {
+        if (any) trace_binary_kernel<true, C><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, d_out);
+        else trace_binary_kernel<false, C><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, d_out);
+    });
 }
 
 cudaError_t launch_trace_binary_multi(const SceneView& s, const void* d_rays, uint64_t n, uint32_t k, void* d_out, uint32_t max_depth_binary,
@@ -992,14 +994,7 @@ cudaError_t launch_trace_binary_multi(const SceneView& s, const void* d_rays, ui
     if (blocks > 0x7fffffffull || k == 0) return cudaErrorInvalidValue;
     const RayIn* r = static_cast<const RayIn*>(d_rays);
     HitX* out = static_cast<HitX*>(d_out);
-    switch (pick_cap(max_depth_binary > 1u ? max_depth_binary : 1u)) {
-        case 32: trace_binary_multi_kernel<32><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, out, k); break;
-        case 64: trace_binary_multi_kernel<64><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, out, k); break;
-        case 128: trace_binary_multi_kernel<128><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, out, k); break;
-        case 256: trace_binary_multi_kernel<256><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, out, k); break;
-        default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
+    return with_cap(max_depth_binary, [&](auto C) { trace_binary_multi_kernel<C><<<(unsigned)blocks, 128, 0, st>>>(s, r, n, out, k); });
 }
 
 cudaError_t launch_camera_rays(const FrameArgs& a, uint64_t gid0, uint64_t gid1, void* d_rays, cudaStream_t st) {
@@ -1010,26 +1005,15 @@ cudaError_t launch_camera_rays(const FrameArgs& a, uint64_t gid0, uint64_t gid1,
     return cudaGetLastError();
 }
 
-template <int CAP>
-static void launch_mega_cap(bool binary, unsigned g, cudaStream_t st, const SceneView& s, const FrameArgs& a, float* d_result, const GidMap& map,
-                            uint32_t n) {
-    if (binary) render_mega_kernel<true, CAP><<<g, 128, 0, st>>>(s, a, d_result, map, n);
-    else render_mega_kernel<false, CAP><<<g, 128, 0, st>>>(s, a, d_result, map, n);
-}
-
 cudaError_t launch_render_mega(const SceneView& s, const FrameArgs& a, float* d_result, const GidMap& map, uint32_t n,
                                bool binary, uint32_t stack_bound, uint32_t max_depth_binary, cudaStream_t st) {
     if (n == 0) return cudaSuccess;
     unsigned g = (n + 127u) / 128u;
     // the wide walk holds at most stack_bound entries, the reference-layout walk at most max_depth_binary
-    switch (binary ? pick_cap(max_depth_binary > 1u ? max_depth_binary : 1u) : pick_cap(stack_bound)) {
-        case 32: launch_mega_cap<32>(binary, g, st, s, a, d_result, map, n); break;
-        case 64: launch_mega_cap<64>(binary, g, st, s, a, d_result, map, n); break;
-        case 128: launch_mega_cap<128>(binary, g, st, s, a, d_result, map, n); break;
-        case 256: launch_mega_cap<256>(binary, g, st, s, a, d_result, map, n); break;
-        default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
+    return with_cap(binary ? max_depth_binary : stack_bound, [&](auto C) {
+        if (binary) render_mega_kernel<true, C><<<g, 128, 0, st>>>(s, a, d_result, map, n);
+        else render_mega_kernel<false, C><<<g, 128, 0, st>>>(s, a, d_result, map, n);
+    });
 }
 
 cudaError_t launch_wf_generate(const FrameArgs& a, const GidMap& map, uint32_t n, void* d_rays, void* d_state,
@@ -1062,26 +1046,17 @@ cudaError_t launch_closest_point(const SceneView& s, const void* d_queries, uint
                                  int grid_blocks, unsigned long long* d_next, unsigned long long* d_counters, uint32_t refill_min,
                                  cudaStream_t st) {
     if (n == 0) return cudaSuccess;
-    const int cap = pick_cap(stack_bound);
-    if (!cap || grid_blocks < 1) return cudaErrorInvalidValue;
+    if (!pick_cap(stack_bound) || grid_blocks < 1) return cudaErrorInvalidValue;
     cudaError_t e = cudaMemsetAsync(d_next, 0, sizeof(unsigned long long), st);
     if (e != cudaSuccess) return e;
-    if (refill_min < 1 || refill_min > 32) refill_min = 8;
-    const uint64_t warps = (uint64_t)grid_blocks * (POINT_BLOCK / 32), c = n / (warps * 8u + 1u);
-    const uint32_t chunk = (uint32_t)(c < 32 ? 32 : (c > 512 ? 512 : (c & ~31ull)));
+    refill_min = refill_or_default(refill_min);
+    const uint32_t chunk = pool_chunk(n, grid_blocks, POINT_BLOCK);
     const float4* q = static_cast<const float4*>(d_queries);
     float4* out = static_cast<float4*>(d_out);
-#define B2_POINT_LAUNCH(C) (count ? point_persistent<true, C><<<grid_blocks, POINT_BLOCK, 0, st>>>(s, q, n, out, d_next, d_counters, chunk, refill_min) \
-                                  : point_persistent<false, C><<<grid_blocks, POINT_BLOCK, 0, st>>>(s, q, n, out, d_next, d_counters, chunk, refill_min))
-    switch (cap) {
-        case 32: B2_POINT_LAUNCH(32); break;
-        case 64: B2_POINT_LAUNCH(64); break;
-        case 128: B2_POINT_LAUNCH(128); break;
-        case 256: B2_POINT_LAUNCH(256); break;
-        default: return cudaErrorInvalidValue;
-    }
-#undef B2_POINT_LAUNCH
-    return cudaGetLastError();
+    return with_cap(stack_bound, [&](auto C) {
+        if (count) point_persistent<true, C><<<grid_blocks, POINT_BLOCK, 0, st>>>(s, q, n, out, d_next, d_counters, chunk, refill_min);
+        else point_persistent<false, C><<<grid_blocks, POINT_BLOCK, 0, st>>>(s, q, n, out, d_next, d_counters, chunk, refill_min);
+    });
 }
 
 cudaError_t launch_closest_point_binary(const SceneView& s, const void* d_queries, uint64_t n, void* d_out, uint32_t max_depth_binary,
@@ -1091,14 +1066,7 @@ cudaError_t launch_closest_point_binary(const SceneView& s, const void* d_querie
     if (blocks > 0x7fffffffull) return cudaErrorInvalidValue;
     const float4* q = static_cast<const float4*>(d_queries);
     float4* out = static_cast<float4*>(d_out);
-    switch (pick_cap(max_depth_binary > 1u ? max_depth_binary : 1u)) {
-        case 32: point_binary_kernel<32><<<(unsigned)blocks, 128, 0, st>>>(s, q, n, out); break;
-        case 64: point_binary_kernel<64><<<(unsigned)blocks, 128, 0, st>>>(s, q, n, out); break;
-        case 128: point_binary_kernel<128><<<(unsigned)blocks, 128, 0, st>>>(s, q, n, out); break;
-        case 256: point_binary_kernel<256><<<(unsigned)blocks, 128, 0, st>>>(s, q, n, out); break;
-        default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
+    return with_cap(max_depth_binary, [&](auto C) { point_binary_kernel<C><<<(unsigned)blocks, 128, 0, st>>>(s, q, n, out); });
 }
 
 int trace_block_threads() { return TRACE_BLOCK; }
@@ -1116,15 +1084,11 @@ cudaError_t tail_occupancy(uint32_t stack_bound, int* blocks_per_sm) {
 }
 
 cudaError_t trace_occupancy(bool any, uint32_t stack_bound, int* blocks_per_sm) {
-    int cap = pick_cap(stack_bound);
     const void* fn = nullptr;
-    switch (cap) {
-        case 32: fn = any ? (const void*)trace_persistent<HIT_ANY, false, 32> : (const void*)trace_persistent<HIT_CLOSEST, false, 32>; break;
-        case 64: fn = any ? (const void*)trace_persistent<HIT_ANY, false, 64> : (const void*)trace_persistent<HIT_CLOSEST, false, 64>; break;
-        case 128: fn = any ? (const void*)trace_persistent<HIT_ANY, false, 128> : (const void*)trace_persistent<HIT_CLOSEST, false, 128>; break;
-        case 256: fn = any ? (const void*)trace_persistent<HIT_ANY, false, 256> : (const void*)trace_persistent<HIT_CLOSEST, false, 256>; break;
-        default: return cudaErrorInvalidValue;
-    }
+    cudaError_t e = with_cap(stack_bound, [&](auto C) {
+        fn = any ? (const void*)trace_persistent<HIT_ANY, false, C> : (const void*)trace_persistent<HIT_CLOSEST, false, C>;
+    });
+    if (e != cudaSuccess) return e;
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, fn, TRACE_BLOCK, 0);
 }
 

@@ -339,32 +339,17 @@ int group_execute(b2rt_context* ctx, size_t gid_begin, size_t gid_end) {
     return B2RT_SUCCESS;
 }
 
-int group_trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void* out, bool any, uint32_t hits_per_ray) {
+int group_split(b2rt_context* ctx, uint64_t n, const std::function<int(b2rt_context*, uint64_t, uint64_t)>& fn) {
     Group* g = ctx->group;
     int st = use_device(ctx);
     if (st) return st;
     st = ensure_scene(ctx);
     if (st) return st;
     const uint64_t world = g->members.size();
-    const size_t elem = hits_per_ray ? (size_t)hits_per_ray * sizeof(b2rt_hit) : (any ? sizeof(uint32_t) : sizeof(b2rt_hit));   // rows of k records (b2rt_trace_multi)
     return run_members(ctx, [&](b2rt_context* m, int k) {
         const uint64_t lo = n * (uint64_t)k / world, hi = n * (uint64_t)(k + 1) / world;     // contiguous ranges, no collective
         if (hi == lo) return (int)B2RT_SUCCESS;
-        return trace_host(m, rays + lo, hi - lo, static_cast<char*>(out) + lo * elem, any, hits_per_ray);
-    });
-}
-
-int group_point_host(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out) {
-    Group* g = ctx->group;
-    int st = use_device(ctx);
-    if (st) return st;
-    st = ensure_scene(ctx);
-    if (st) return st;
-    const uint64_t world = g->members.size();
-    return run_members(ctx, [&](b2rt_context* m, int k) {
-        const uint64_t lo = n * (uint64_t)k / world, hi = n * (uint64_t)(k + 1) / world;     // contiguous ranges, as for rays
-        if (hi == lo) return (int)B2RT_SUCCESS;
-        return point_host(m, q + lo, hi - lo, out + lo);
+        return fn(m, lo, hi - lo);
     });
 }
 
