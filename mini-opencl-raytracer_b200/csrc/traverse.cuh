@@ -202,6 +202,8 @@ B2_HD float lo2(F2 p) { float a; asm("mov.b64 {%0, _}, %1;" : "=f"(a) : "l"(p.v)
 B2_HD float hi2(F2 p) { float b; asm("mov.b64 {_, %0}, %1;" : "=f"(b) : "l"(p.v)); return b; }
 B2_HD F2 sub2(F2 a, F2 b) { F2 r; asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r.v) : "l"(a.v), "l"(b.v)); return r; }
 B2_HD F2 mul2(F2 a, F2 b) { F2 r; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r.v) : "l"(a.v), "l"(b.v)); return r; }
+B2_HD F2 add2(F2 a, F2 b) { F2 r; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r.v) : "l"(a.v), "l"(b.v)); return r; }
+B2_HD F2 fma2(F2 a, F2 b, F2 c) { F2 r; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r.v) : "l"(a.v), "l"(b.v), "l"(c.v)); return r; }   // two fma_rn
 #else
 // Host emulation: two scalar operations (the emulation cannot see a contraction; the SASS test does).
 struct F2 { float a, b; };
@@ -210,8 +212,11 @@ B2_HD float lo2(F2 p) { return p.a; }
 B2_HD float hi2(F2 p) { return p.b; }
 B2_HD F2 sub2(F2 x, F2 y) { return pack2(xsub(x.a, y.a), xsub(x.b, y.b)); }
 B2_HD F2 mul2(F2 x, F2 y) { return pack2(xmul(x.a, y.a), xmul(x.b, y.b)); }
+B2_HD F2 add2(F2 x, F2 y) { return pack2(xadd(x.a, y.a), xadd(x.b, y.b)); }
+B2_HD F2 fma2(F2 x, F2 y, F2 z) { return pack2(fma_rn(x.a, y.a, z.a), fma_rn(x.b, y.b, z.b)); }
 #endif
 B2_HD F2 both2(float v) { return pack2(v, v); }
+B2_HD F2 abs2(F2 p) { return pack2(fabsf(lo2(p)), fabsf(hi2(p))); }
 
 // OpenCL max()/min() as worded by the spec ("y if x < y, otherwise x"), the
 // convention the oracle pins for NaN operands (oracle/ref_build/cl_shim.hpp).
@@ -532,17 +537,27 @@ B2_HD WideHits test_wide_node_h2(const U4* wide, uint32_t index, const RayX& r, 
     out.meta_lo = prmt(w1.z, w1.w, sel_lo);
     out.meta_hi = prmt(w1.z, w1.w, sel_hi);
 
+    const uint32_t qlo_a[3] = { w2.x, w2.z, w3.x }, qlo_b[3] = { w2.y, w2.w, w3.y };   // slots 0..3 / 4..7
+    const uint32_t qhi_a[3] = { w3.z, w4.x, w4.z }, qhi_b[3] = { w3.w, w4.y, w4.w };
+    // From B on, the fp32 set-up runs with x and y as one packed pair (xy) and z scalar: the same operations with the same
+    // roundings, except where ptxas contracts a packed product into the packed sum it feeds (see "packed fp32 pairs"). The
+    // only such products here are by scale, a power of two: exact unless the result is subnormal or overflows. A
+    // contraction therefore drops a rounding that was nothing or below 2^-149; the error budget above already counts that
+    // rounding as one of its terms, so the slack still covers the contracted sequence. An overflowing B gives slack = inf
+    // and Bn / Bf = -inf / +inf instead of NaN / +inf: the near plane still drops out of the max and the far one out of the
+    // min. The fallback guard reads the scalar A and K1, which are not contracted.
+    // K1 and A stay scalar: packing the ray's origin and reciprocal into pairs costs more moves and registers (spills in
+    // trace_persistent) than the two paired products save
     const float o[3] = { r.ox, r.oy, r.oz };
     const float inv[3] = { r.ix, r.iy, r.iz };
     const float base[3] = { bits2f(w0.x), bits2f(w0.y), bits2f(w0.z) };
-    const uint32_t qlo_a[3] = { w2.x, w2.z, w3.x }, qlo_b[3] = { w2.y, w2.w, w3.y };   // slots 0..3 / 4..7
-    const uint32_t qhi_a[3] = { w3.z, w4.x, w4.z }, qhi_b[3] = { w3.w, w4.y, w4.w };
     float K1[3], A[3];
 #pragma unroll
     for (int a = 0; a < 3; ++a) {
         K1[a] = xmul(bits2f(((w0.w >> (8 * a)) & 0xffu) << 23), inv[a]);
         A[a] = xmul(xsub(base[a], o[a]), inv[a]);
     }
+    const F2 K1xy = pack2(K1[0], K1[1]), Axy = pack2(A[0], A[1]);
     const float kmax = max_nn(max_nn(fabsf(K1[0]), fabsf(K1[1])), fabsf(K1[2]));
     // magnitudes this frame cannot hold (overflow of (base - o) * inv or S * inv: coordinates or reciprocals beyond 2^100):
     // decide in fp32 instead. Written so that NaN takes the branch too.
@@ -556,20 +571,21 @@ B2_HD WideHits test_wide_node_h2(const U4* wide, uint32_t index, const RayX& r, 
     eb = eb < 15u ? 15u : eb;                                           // |K1| below 2^-112: keep the scale factors representable
     const float scale = bits2f((244u - eb) << 23);                     // 2^(117 - (eb - 127))
     const float kscale = bits2f((268u - eb) << 23);                    // scale * 2^24
-    uint32_t Kh[3], Bn[3], Bf[3];
     const float e32 = fma_rn(xmul(xadd(amax, t_ref), scale), 9.5367431640625e-7f, 2.384185791015625e-7f);   // the fp32 roundings' share, one bound for all axes
-#pragma unroll
-    for (int a = 0; a < 3; ++a) {
-        const float B = xmul(xsub(A[a], t_ref), scale);
-        const float K2 = xmul(K1[a], kscale);
-        const float slack = fma_rn(fma_rn(fabsf(K2), 1.52587890625e-5f, fabsf(B)), 1.0009765625e-3f, e32);
-        Kh[a] = h2_both(K2);
-        Bn[a] = h2_both(xsub(B, slack));
-        Bf[a] = h2_both(xadd(B, slack));
-    }
-    const float z = xmul(-t_ref, scale), b = xmul(xsub(best, t_ref), scale);
-    const uint32_t zero_h = h2_both(xsub(z, fma_rn(fabsf(z), 9.765625e-4f, 2.384185791015625e-7f)));     // 0 and best: one conversion each, 2^-11 relative
-    const uint32_t best_h = h2_both(xadd(b, fma_rn(fabsf(b), 9.765625e-4f, 2.384185791015625e-7f)));
+    const F2 Bxy = mul2(sub2(Axy, both2(t_ref)), both2(scale));
+    const F2 K2xy = mul2(K1xy, both2(kscale));
+    const F2 Sxy = fma2(fma2(abs2(K2xy), both2(1.52587890625e-5f), abs2(Bxy)), both2(1.0009765625e-3f), both2(e32));
+    const F2 Bnxy = sub2(Bxy, Sxy), Bfxy = add2(Bxy, Sxy);
+    const float Bz = xmul(xsub(A[2], t_ref), scale), K2z = xmul(K1[2], kscale);
+    const float Sz = fma_rn(fma_rn(fabsf(K2z), 1.52587890625e-5f, fabsf(Bz)), 1.0009765625e-3f, e32);
+    const uint32_t Kh[3] = { h2_both(lo2(K2xy)), h2_both(hi2(K2xy)), h2_both(K2z) };
+    const uint32_t Bn[3] = { h2_both(lo2(Bnxy)), h2_both(hi2(Bnxy)), h2_both(xsub(Bz, Sz)) };
+    const uint32_t Bf[3] = { h2_both(lo2(Bfxy)), h2_both(hi2(Bfxy)), h2_both(xadd(Bz, Sz)) };
+    // 0 and best as one pair (-z, b), z = -t_ref * scale, b = (best - t_ref) * scale: both moved up by 2^-10 of their
+    // magnitude + 2^-22, i.e. z lowered and b raised, one conversion each
+    const F2 zb = mul2(pack2(t_ref, xsub(best, t_ref)), both2(scale));
+    const F2 zbs = add2(zb, fma2(abs2(zb), both2(9.765625e-4f), both2(2.384185791015625e-7f)));
+    const uint32_t zero_h = h2_both(-lo2(zbs)), best_h = h2_both(hi2(zbs));
     uint32_t d[4];
 #pragma unroll
     for (int pr = 0; pr < 4; ++pr) {
