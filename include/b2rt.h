@@ -348,6 +348,35 @@ typedef struct { float d2, u, v; uint32_t tri; } b2rt_point_hit;   /* 16 B */
 int b2rt_closest_point(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out);
 int b2rt_closest_point_device(b2rt_context* ctx, const b2rt_point_query* d_q, uint64_t n, b2rt_point_hit* d_out, void* cuda_stream);
 
+/* ---- path-traced radiance (new) ------------------------------------------------------------ */
+/* Render() (kernel_bvh.cl:349-384) started from a caller's ray instead of the pinhole camera: one shaded sample per ray, for
+ * other cameras (fisheye, orthographic, thin lens, panoramas), own sample patterns, probes at arbitrary points.
+ *  Path i starts at InitRay((ox,oy,oz), (dx,dy,dz)) of rays[i] with RNG state seeds[i].
+ *  Segment 0 is the closest hit with isect.t = tmax, under the acceptance rule of b2rt_trace_closest (tmin ignored, front
+ *    faces only); a miss within tmax takes the sky term. Later segments start at pos + wi*0.01 with B2RT_MAX_RENDER_DIST,
+ *    exactly as Render() does: with tmax = 100000 the whole path is Render().
+ *  Shading arguments come from the bound slots LIGHT_BOUNCES (8), LIGHT_TYPE (9) and SKYBOX_INTENSITY (10) and the material
+ *    buffer (slot 3); an out-of-range mtlIndex takes the last material, as in frames. The frame-only slots (output image,
+ *    width, height, frame count, camera) are not needed.
+ *  out[i] = {max(radiance, 0) per channel (OpenCL max: NaN passes), RNG state after the path}. The returned state lets a
+ *    caller chain samples of one path. bounces <= 0 gives {0, 0, 0, seeds[i]}.
+ *  A NULL rays, seeds or out with n > 0 returns B2RT_INVALID_VALUE and writes nothing; n = 0 succeeds. Slots 8-10 never
+ *    set, no bound material buffer or no scene return B2RT_INVALID_KERNEL_ARGS.
+ * b2rt_trace_radiance: host buffers, synchronous, pipelined in chunks like b2rt_trace_closest; on a b2rt_create_multi handle
+ * the rays are cut into contiguous ranges, one per device.
+ * b2rt_trace_radiance_device: device buffers, asynchronous on cuda_stream (NULL = the context's stream); on a
+ * b2rt_create_multi handle it runs on the root. The launch uses the frame path's wavefront queues, so it runs on the
+ * context's stream, ordered after the work already enqueued on cuda_stream, and work enqueued on cuda_stream after the call
+ * sees the records (also after a failure, which may leave part of d_out written). Frames and radiance launches on
+ * different streams are therefore serialised through the context's stream and never share the queues concurrently.
+ * B2RT_OPT_TRAVERSAL = 1 runs one thread per path over the reference-layout arrays, B2RT_OPT_COUNTERS = 1 the counting build
+ * (rays = path segments traced). B2RT_OPT_WAVEFRONT_LANES, B2RT_OPT_COOP_MAX and B2RT_OPT_RESUME_MAX apply as in frames;
+ * B2RT_OPT_RENDER_MODE is ignored. Results do not depend on any of them. */
+typedef struct { float r, g, b; uint32_t seed; } b2rt_radiance;          /* 16 B */
+int b2rt_trace_radiance(b2rt_context* ctx, const b2rt_ray* rays, const uint32_t* seeds, uint64_t n, b2rt_radiance* out);
+int b2rt_trace_radiance_device(b2rt_context* ctx, const b2rt_ray* d_rays, const uint32_t* d_seeds, uint64_t n,
+                               b2rt_radiance* d_out, void* cuda_stream);
+
 /* CreateRay (kernel_bvh.cl:386-403) for gid in [gid_begin, gid_end) with the currently bound
  * WIDTH/HEIGHT/FRAME_COUNT/CAMERA_* arguments, written to device memory as b2rt_ray. */
 int b2rt_camera_rays_device(b2rt_context* ctx, size_t gid_begin, size_t gid_end, b2rt_ray* d_rays, void* cuda_stream);

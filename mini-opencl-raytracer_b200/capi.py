@@ -6,7 +6,7 @@ import time
 
 import numpy as np
 
-from .layouts import HIT_DTYPE, MAT_BYTES, NODE_BYTES, POINT_HIT_DTYPE, POINT_QUERY_DTYPE, RAY_DTYPE, TRI_BYTES
+from .layouts import HIT_DTYPE, MAT_BYTES, NODE_BYTES, POINT_HIT_DTYPE, POINT_QUERY_DTYPE, RADIANCE_DTYPE, RAY_DTYPE, TRI_BYTES
 
 MISS = 0xFFFFFFFF
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -30,7 +30,7 @@ SYMBOLS = [
     "b2rt_create_multi", "b2rt_group_size", "b2rt_group_info", "b2rt_comm_unique_id", "b2rt_comm_init", "b2rt_comm_share_output",
     "b2rt_execute_shard", "b2rt_shard_bands", "b2rt_refit_scene", "b2rt_stage_times",
     "b2rt_build_scene_device", "b2rt_refit_scene_device", "b2rt_trace_multi", "b2rt_trace_multi_device",
-    "b2rt_closest_point", "b2rt_closest_point_device",
+    "b2rt_closest_point", "b2rt_closest_point_device", "b2rt_trace_radiance", "b2rt_trace_radiance_device",
 ]
 MULTI_MAX_HITS = 64          # B2RT_MULTI_MAX_HITS: largest k of b2rt_trace_multi
 # status bits of b2rt_refit_scene_device
@@ -103,6 +103,8 @@ def lib():
         "b2rt_trace_multi_device": (C.c_int, [vp, vp, u64, u32, vp, vp]),
         "b2rt_closest_point": (C.c_int, [vp, vp, u64, vp]),
         "b2rt_closest_point_device": (C.c_int, [vp, vp, u64, vp, vp]),
+        "b2rt_trace_radiance": (C.c_int, [vp, vp, vp, u64, vp]),
+        "b2rt_trace_radiance_device": (C.c_int, [vp, vp, vp, u64, vp, vp]),
         "b2rt_camera_rays_device": (C.c_int, [vp, sz, sz, vp, vp]),
         "b2rt_device_pointer": (C.c_int, [vp, u64, C.POINTER(vp), C.POINTER(sz)]),
         "b2rt_bound_buffer": (C.c_int, [vp, u32, C.POINTER(u64)]),
@@ -340,6 +342,11 @@ class Context:
             f3 = (C.c_float * 4)(v[0], v[1], v[2], 0.0)
             self._ck(L.b2rt_set_arg(h, slot, f3, 16))
 
+    def set_shading(self, bounces, light_type=0, sky=1.0):
+        """Only the shading slots (light bounces, light type, sky intensity): all that trace_radiance needs besides the scene."""
+        for slot, v in ((ARG_LIGHT_BOUNCES, C.c_int32(bounces)), (ARG_LIGHT_TYPE, C.c_int32(light_type)), (ARG_SKYBOX_INTENSITY, C.c_float(sky))):
+            self._ck(self._L.b2rt_set_arg(self._h, slot, C.byref(v), 4))
+
     def set_option(self, option, value):
         self._ck(self._L.b2rt_set_option(self._h, int(option), int(value)))
 
@@ -432,6 +439,23 @@ class Context:
         """b2rt_closest_point_device: n query and n result records of 16 bytes in device memory."""
         self._ck(self._L.b2rt_closest_point_device(self._h, C.c_void_p(int(d_queries)), int(n), C.c_void_p(int(d_out)),
                                                    C.c_void_p(int(stream))))
+
+    def trace_radiance(self, rays, seeds):
+        """The path-traced radiance of every ray (b2rt_trace_radiance): a RADIANCE_DTYPE array of {r, g, b, seed}, the
+        seed being the RNG state after the path. Shading comes from the bound light bounces, light type, sky intensity and
+        materials (set_shading or set_frame)."""
+        rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
+        seeds = np.ascontiguousarray(seeds, dtype=np.uint32)
+        if seeds.shape != (rays.shape[0],):
+            raise ValueError("one seed per ray: %d rays, seeds of shape %s" % (rays.shape[0], seeds.shape))
+        out = np.empty(rays.shape[0], dtype=RADIANCE_DTYPE)
+        self._ck(self._L.b2rt_trace_radiance(self._h, _ptr(rays), _ptr(seeds), rays.shape[0], _ptr(out)))
+        return out
+
+    def trace_radiance_device(self, d_rays, d_seeds, n, d_out, stream=0):
+        """b2rt_trace_radiance_device: n rays (32 B), n uint32 seeds and n records of 16 bytes in device memory."""
+        self._ck(self._L.b2rt_trace_radiance_device(self._h, C.c_void_p(int(d_rays)), C.c_void_p(int(d_seeds)), int(n),
+                                                    C.c_void_p(int(d_out)), C.c_void_p(int(stream))))
 
     def trace_closest_device(self, d_rays, n, d_hits, stream=0):
         self._ck(self._L.b2rt_trace_closest_device(self._h, C.c_void_p(int(d_rays)), int(n), C.c_void_p(int(d_hits)),

@@ -388,23 +388,28 @@ int point_device(b2rt_context* ctx, const void* d_q, uint64_t n, void* d_out, cu
     return B2RT_SUCCESS;
 }
 
-int ensure_staging(b2rt_context* ctx, uint64_t chunk, size_t out_bytes) {
-    if (ctx->stage_capacity >= chunk && ctx->stage_out_bytes >= out_bytes) return B2RT_SUCCESS;
+int ensure_staging(b2rt_context* ctx, uint64_t chunk, size_t out_bytes, size_t in2_bytes) {
+    if (ctx->stage_capacity >= chunk && ctx->stage_out_bytes >= out_bytes && ctx->stage_in2_bytes >= in2_bytes) return B2RT_SUCCESS;
     chunk = std::max(chunk, ctx->stage_capacity);
     out_bytes = std::max(out_bytes, ctx->stage_out_bytes);
+    in2_bytes = std::max(in2_bytes, ctx->stage_in2_bytes);
     for (int i = 0; i < 2; ++i) {
         if (ctx->d_stage_rays[i]) cudaFree(ctx->d_stage_rays[i]);
         if (ctx->d_stage_out[i]) cudaFree(ctx->d_stage_out[i]);
-        ctx->d_stage_rays[i] = ctx->d_stage_out[i] = nullptr;
+        if (ctx->d_stage_in2[i]) cudaFree(ctx->d_stage_in2[i]);
+        ctx->d_stage_rays[i] = ctx->d_stage_out[i] = ctx->d_stage_in2[i] = nullptr;
     }
     ctx->stage_capacity = 0;
     ctx->stage_out_bytes = 0;
+    ctx->stage_in2_bytes = 0;
     for (int i = 0; i < 2; ++i) {
         CK(cudaMalloc(&ctx->d_stage_rays[i], chunk * sizeof(b2rt_ray)));
         CK(cudaMalloc(&ctx->d_stage_out[i], out_bytes));
+        if (in2_bytes) CK(cudaMalloc(&ctx->d_stage_in2[i], in2_bytes));
     }
     ctx->stage_capacity = chunk;
     ctx->stage_out_bytes = out_bytes;
+    ctx->stage_in2_bytes = in2_bytes;
     return B2RT_SUCCESS;
 }
 
@@ -415,12 +420,13 @@ static uint64_t stream_chunk() {
 }
 
 // Host-buffer query stream: chunks of at most `chunk_cap` records of `in_elem` bytes (at most a b2rt_ray) are copied in,
-// run through launch(d_in, m, d_out, stream) and their `out_elem`-byte results copied out, on three streams so that PCIe
-// transfers overlap the kernels. The output staging holds at least a chunk of b2rt_hit, so that every query kind fits the
-// same staging buffers without reallocating. `what` names the input in the NULL-pointer error.
+// run through launch(d_in, d_in2, m, d_out, stream) and their `out_elem`-byte results copied out, on three streams so that
+// PCIe transfers overlap the kernels. The output staging holds at least a chunk of b2rt_hit, so that every query kind fits
+// the same staging buffers without reallocating. `in2` (may be NULL): a second input array of `in2_elem`-byte records,
+// staged beside the first (d_in2). `what` names the input in the NULL-pointer error.
 template <class Launch>
-static int host_pipeline(b2rt_context* ctx, const void* in, size_t in_elem, uint64_t n, void* out, size_t out_elem, uint64_t chunk_cap,
-                         const char* what, Launch&& launch) {
+static int host_pipeline(b2rt_context* ctx, const void* in, size_t in_elem, const void* in2, size_t in2_elem, uint64_t n, void* out,
+                         size_t out_elem, uint64_t chunk_cap, const char* what, Launch&& launch) {
     int st = use_device(ctx);
     if (st) return st;
     st = ensure_scene(ctx);
@@ -428,7 +434,7 @@ static int host_pipeline(b2rt_context* ctx, const void* in, size_t in_elem, uint
     if (n == 0) return B2RT_SUCCESS;
     if (!in || !out) return fail(ctx, B2RT_INVALID_VALUE, std::string("null ") + what + " or output pointer");
     const uint64_t chunk = std::min<uint64_t>(n, chunk_cap);
-    st = ensure_staging(ctx, chunk, chunk * std::max(out_elem, sizeof(b2rt_hit)));
+    st = ensure_staging(ctx, chunk, chunk * std::max(out_elem, sizeof(b2rt_hit)), in2 ? chunk * in2_elem : 0);
     if (st) return st;
     // Chunk sizes ramp up from `ramp` to `chunk` and back down at the end: the first copy-in and the last kernel +
     // copy-out are the only parts of the pipeline that nothing overlaps, so they are kept short.
@@ -442,10 +448,11 @@ static int host_pipeline(b2rt_context* ctx, const void* in, size_t in_elem, uint
         else m = std::min<uint64_t>(m, std::max<uint64_t>(ramp, (left / 2 + 31) & ~31ull));            // ramp down: at most half of what is left
         if (c >= 2) CK(cudaStreamWaitEvent(ctx->stream_in, ctx->ev_comp[s], 0));     // in[s] free again
         CK(cudaMemcpyAsync(ctx->d_stage_rays[s], static_cast<const char*>(in) + off * in_elem, m * in_elem, cudaMemcpyHostToDevice, ctx->stream_in));
+        if (in2) CK(cudaMemcpyAsync(ctx->d_stage_in2[s], static_cast<const char*>(in2) + off * in2_elem, m * in2_elem, cudaMemcpyHostToDevice, ctx->stream_in));
         CK(cudaEventRecord(ctx->ev_in[s], ctx->stream_in));
         CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_in[s], 0));
         if (c >= 2) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_out[s], 0));         // out[s] drained
-        st = launch(ctx->d_stage_rays[s], m, ctx->d_stage_out[s], ctx->stream);
+        st = launch(ctx->d_stage_rays[s], ctx->d_stage_in2[s], m, ctx->d_stage_out[s], ctx->stream);
         if (st) return st;
         CK(cudaEventRecord(ctx->ev_comp[s], ctx->stream));
         CK(cudaStreamWaitEvent(ctx->stream_out, ctx->ev_comp[s], 0));
@@ -463,15 +470,14 @@ static int trace_host(b2rt_context* ctx, const b2rt_ray* rays, uint64_t n, void*
     uint64_t chunk = stream_chunk();
     if (k > 1) chunk = std::max<uint64_t>(chunk / k, 1024);
     const size_t out_elem = k ? (size_t)k * sizeof(b2rt_hit) : (any ? sizeof(uint32_t) : sizeof(b2rt_hit));
-    return host_pipeline(ctx, rays, sizeof(b2rt_ray), n, out, out_elem, chunk, "ray", [&](const void* d_in, uint64_t m, void* d_out, cudaStream_t s) {
-        return trace_device(ctx, d_in, m, d_out, any, s, k);
-    });
+    return host_pipeline(ctx, rays, sizeof(b2rt_ray), nullptr, 0, n, out, out_elem, chunk, "ray",
+                         [&](const void* d_in, const void*, uint64_t m, void* d_out, cudaStream_t s) { return trace_device(ctx, d_in, m, d_out, any, s, k); });
 }
 
 // Host-buffer closest-point queries on one device.
 static int point_host(b2rt_context* ctx, const b2rt_point_query* q, uint64_t n, b2rt_point_hit* out) {
-    return host_pipeline(ctx, q, sizeof(b2rt_point_query), n, out, sizeof(b2rt_point_hit), stream_chunk(), "query",
-                         [&](const void* d_in, uint64_t m, void* d_out, cudaStream_t s) { return point_device(ctx, d_in, m, d_out, s); });
+    return host_pipeline(ctx, q, sizeof(b2rt_point_query), nullptr, 0, n, out, sizeof(b2rt_point_hit), stream_chunk(), "query",
+                         [&](const void* d_in, const void*, uint64_t m, void* d_out, cudaStream_t s) { return point_device(ctx, d_in, m, d_out, s); });
 }
 
 int frame_args(b2rt_context* ctx, FrameArgs& a);
@@ -520,7 +526,7 @@ cudaEvent_t stage_mark(b2rt_context* ctx, bool on, uint32_t kind, cudaStream_t s
     } while (0)
 
 int wavefront_lane(b2rt_context* ctx, const FrameArgs& a, float* d_result, const GidMap& map, uint32_t n, int lane, uint64_t offset,
-                   cudaStream_t s, int share = 1) {
+                   cudaStream_t s, int share, const RadianceIO* io) {
     int st_pol = apply_l2_policy(ctx, s);
     if (st_pol) return st_pol;
     const bool timed = ctx->opt_stage_times != 0 && lane == 0;
@@ -530,7 +536,7 @@ int wavefront_lane(b2rt_context* ctx, const FrameArgs& a, float* d_result, const
     char* rays[2] = { static_cast<char*>(ctx->d_wf_rays[0]) + offset * sizeof(b2rt_ray), static_cast<char*>(ctx->d_wf_rays[1]) + offset * sizeof(b2rt_ray) };
     char* hits = static_cast<char*>(ctx->d_wf_hits) + offset * sizeof(b2rt_hit);
     char* state = static_cast<char*>(ctx->d_wf_state) + offset * 32;
-    CK(launch_wf_generate(a, map, n, rays[0], state, cnt, s));        // also resets the lane's four counters
+    CK(launch_wf_generate(a, map, n, rays[0], state, cnt, s, io));    // also resets the lane's four counters
     ctx->launches += 1;
     STAGE(B2RT_STAGE_GENERATE);
     // `share` wavefronts run side by side: each takes its part of the CTA slots (whole CTAs per SM)
@@ -549,7 +555,7 @@ int wavefront_lane(b2rt_context* ctx, const FrameArgs& a, float* d_result, const
                              stage_mark(ctx, timed, B2RT_STAGE_TRACE, s)));
         STAGE(B2RT_STAGE_TAIL);
         // the shade stage also clears the counter the NEXT shade stage appends to and the traversal kernels' three counters
-        CK(launch_wf_shade(ctx->view, a, map, n, rays[in], hits, n_in, rays[out], n_out, state, d_result, b == a.bounces - 1, n_clear, cnt + 3, s));
+        CK(launch_wf_shade(ctx->view, a, map, n, rays[in], hits, n_in, rays[out], n_out, state, d_result, b == a.bounces - 1, n_clear, cnt + 3, s, io));
         ctx->launches += tail.coop_max ? (tail.resume_max ? 4 : 3) : 2;
         STAGE(B2RT_STAGE_SHADE);
     }
@@ -560,12 +566,13 @@ int wavefront_lane(b2rt_context* ctx, const FrameArgs& a, float* d_result, const
 // KernelEntry for work items [0, n) of `map` as up to WF_LANES independent wavefronts on their own streams. A
 // stage's persistent traversal kernel ends with a tail (a few rays need 10-100x the average number of steps, on
 // one lane of one warp); with several wavefronts in flight the next one's CTAs fill the SMs the tail leaves idle.
-int render_wavefront(b2rt_context* ctx, const FrameArgs& a, float* d_result, const GidMap& map, uint32_t n) {
+// io != null: the paths of a caller's ray stream instead of pixels (b2rt_trace_radiance, kernels.h RadianceIO).
+int render_wavefront(b2rt_context* ctx, const FrameArgs& a, float* d_result, const GidMap& map, uint32_t n, const RadianceIO* io) {
     int st = ensure_wavefront(ctx, n);
     if (st) return st;
     if (a.bounces <= 0) {
         // Render() never enters its loop: radiance 0 for every pixel, which is what the megakernel does without tracing.
-        CK(launch_render_mega(ctx->view, a, d_result, map, n, false, ctx->stack_bound, ctx->info.max_depth_binary, ctx->stream));
+        CK(launch_render_mega(ctx->view, a, d_result, map, n, false, ctx->stack_bound, ctx->info.max_depth_binary, ctx->stream, io));
         ctx->launches += 1;
         return B2RT_SUCCESS;
     }
@@ -577,7 +584,7 @@ int render_wavefront(b2rt_context* ctx, const FrameArgs& a, float* d_result, con
     uint64_t per = (((uint64_t)n + lanes - 1) / lanes + unit - 1) / unit * unit;
     if (per == 0) per = unit;
     lanes = (int)std::min<uint64_t>(lanes, ((uint64_t)n + per - 1) / per);
-    if (lanes <= 1) return wavefront_lane(ctx, a, d_result, map, n, 0, 0, ctx->stream);
+    if (lanes <= 1) return wavefront_lane(ctx, a, d_result, map, n, 0, 0, ctx->stream, 1, io);
     CK(cudaEventRecord(ctx->ev_wf_fork, ctx->stream));
     for (int l = 0; l < lanes; ++l) {
         const uint64_t off = per * l, m = std::min<uint64_t>(per, n - off);
@@ -585,7 +592,7 @@ int render_wavefront(b2rt_context* ctx, const FrameArgs& a, float* d_result, con
         if (contiguous) { sub.begin = map.begin + off; sub.band = sub.stride = (uint32_t)m; }
         else sub.begin = map.begin + (off / map.band) * map.stride;
         CK(cudaStreamWaitEvent(ctx->wf_stream[l], ctx->ev_wf_fork, 0));
-        st = wavefront_lane(ctx, a, d_result, sub, (uint32_t)m, l, off, ctx->wf_stream[l], ctx->opt_wf_grid_split ? lanes : 1);
+        st = wavefront_lane(ctx, a, d_result, sub, (uint32_t)m, l, off, ctx->wf_stream[l], ctx->opt_wf_grid_split ? lanes : 1, io);
         if (st) return st;
         CK(cudaEventRecord(ctx->ev_wf_join[l], ctx->wf_stream[l]));
         CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_wf_join[l], 0));
@@ -593,7 +600,8 @@ int render_wavefront(b2rt_context* ctx, const FrameArgs& a, float* d_result, con
     return B2RT_SUCCESS;
 }
 
-int render_with_mode(b2rt_context* ctx, const FrameArgs& a, float* result, const GidMap& map, uint64_t n, int mode);
+int render_with_mode(b2rt_context* ctx, const FrameArgs& a, float* result, const GidMap& map, uint64_t n, int mode,
+                     const RadianceIO* io = nullptr);
 int render_tuned(b2rt_context* ctx, const FrameArgs& a, float* result, const GidMap& map, uint64_t n);
 
 // Folds a finished timing into the tuner table. Never waits: while the timed launch is still running `*busy` is set and the
@@ -668,15 +676,15 @@ int render_items(b2rt_context* ctx, const GidMap& map, uint64_t n) {
     return render_tuned(ctx, a, result, map, n);
 }
 
-// One frame launch in a given mode: 1 = megakernel, 0 = wavefront.
-int render_with_mode(b2rt_context* ctx, const FrameArgs& a, float* result, const GidMap& map, uint64_t n, int mode) {
+// One frame launch in a given mode: 1 = megakernel, 0 = wavefront. io != null: a caller's ray stream (see render_wavefront).
+int render_with_mode(b2rt_context* ctx, const FrameArgs& a, float* result, const GidMap& map, uint64_t n, int mode, const RadianceIO* io) {
     int st = B2RT_SUCCESS;
     if (mode == 1) {
         if (ctx->opt_traversal == 1) st = binary_walk_fits(ctx);
         if (!st) st = apply_l2_policy(ctx, ctx->stream);
         if (st) return st;
         CK(launch_render_mega(ctx->view, a, result, map, (uint32_t)n, ctx->opt_traversal == 1, ctx->stack_bound, ctx->info.max_depth_binary,
-                              ctx->stream));
+                              ctx->stream, io));
         ctx->launches += 1;
         return B2RT_SUCCESS;
     }
@@ -686,7 +694,7 @@ int render_with_mode(b2rt_context* ctx, const FrameArgs& a, float* result, const
             GidMap sub;
             const uint32_t m = (uint32_t)std::min<uint64_t>(WF_MAX_PATHS, count - off);
             sub.begin = first_gid + off; sub.band = sub.stride = m;
-            int rc = render_wavefront(ctx, a, result, sub, m);
+            int rc = render_wavefront(ctx, a, result, sub, m, io);
             if (rc) return rc;
         }
         return B2RT_SUCCESS;
@@ -703,7 +711,7 @@ int render_with_mode(b2rt_context* ctx, const FrameArgs& a, float* result, const
     for (uint64_t off = 0; off < n; off += per_pass) {
         GidMap sub = map;
         sub.begin = map.begin + (off / map.band) * map.stride;
-        st = render_wavefront(ctx, a, result, sub, (uint32_t)std::min<uint64_t>(per_pass, n - off));
+        st = render_wavefront(ctx, a, result, sub, (uint32_t)std::min<uint64_t>(per_pass, n - off), io);
         if (st) return st;
     }
     return B2RT_SUCCESS;
@@ -716,14 +724,59 @@ static void camera_args(const b2rt_context* ctx, FrameArgs& a) {
     a.angle = tanf(0.5f * (45.0f * 3.1415f / 180.0f));   // kernel_bvh.cl:392, evaluated by the host libm like the oracle
 }
 
+// The shading part of FrameArgs (slots 8-10): frames and b2rt_trace_radiance shade paths with the same values.
+static int shade_args(b2rt_context* ctx, FrameArgs& a) {
+    for (int i : { B2RT_ARG_LIGHT_BOUNCES, B2RT_ARG_LIGHT_TYPE, B2RT_ARG_SKYBOX_INTENSITY })
+        if (!ctx->arg_set[i]) return fail(ctx, B2RT_INVALID_KERNEL_ARGS, "kernel argument " + std::to_string(i) + " was never set");
+    a.bounces = ctx->bounces; a.light_type = ctx->light_type; a.sky = ctx->sky;
+    return B2RT_SUCCESS;
+}
+
 int frame_args(b2rt_context* ctx, FrameArgs& a) {
     for (int i = 0; i < B2RT_ARG_COUNT; ++i)
         if (!ctx->arg_set[i]) return fail(ctx, B2RT_INVALID_KERNEL_ARGS, "kernel argument " + std::to_string(i) + " was never set");
     camera_args(ctx, a);
-    a.bounces = ctx->bounces; a.light_type = ctx->light_type; a.sky = ctx->sky;
+    shade_args(ctx, a);                                  // cannot fail: every slot is set
     a.mirror = ctx->mirror;
     if (a.width == 0 || a.height == 0) return fail(ctx, B2RT_INVALID_KERNEL_ARGS, "WIDTH/HEIGHT must be non-zero");
     return B2RT_SUCCESS;
+}
+
+// Path-traced radiance per ray (b2rt_trace_radiance_device): the frame path's stages with the caller's rays and seeds as the
+// source and one b2rt_radiance record per path as the sink, always on the wavefront (the megakernel over the reference-layout
+// arrays with B2RT_OPT_TRAVERSAL = 1). The stages use the frame path's queues, counters and tail queues, which belong to the
+// context's stream, so the launch runs there between two edges with the caller's stream.
+int radiance_device(b2rt_context* ctx, const void* d_rays, const uint32_t* d_seeds, uint64_t n, void* d_out, cudaStream_t caller) {
+    FrameArgs a;
+    memset(&a, 0, sizeof(a));
+    int st = shade_args(ctx, a);
+    if (st) return st;
+    if (!ctx->view.mats || ctx->view.n_mats == 0) return fail(ctx, B2RT_INVALID_KERNEL_ARGS, "material buffer (slot 3) is not bound");
+    if (n == 0) return B2RT_SUCCESS;
+    if (a.bounces < 0) a.bounces = 0;      // the contract's "bounces <= 0": no segment (the kernels' loop bound is unsigned)
+    const RadianceIO io = { d_rays, d_seeds, d_out };
+    const cudaStream_t s = ctx->stream;
+    if (caller != s) CK(stream_edge(ctx->ev_refit[0], caller, s));           // behind the caller's work on its stream
+    // pieces that a 32-bit work-item count holds (the megakernel's launch); render_with_mode checks the reference-layout
+    // walk's stack in mode 1
+    for (uint64_t off = 0; off < n && !st; off += 1ull << 31) {
+        const uint64_t m = std::min<uint64_t>(n - off, 1ull << 31);
+        GidMap map;
+        map.begin = off;
+        map.band = map.stride = (uint32_t)m;
+        st = render_with_mode(ctx, a, nullptr, map, m, ctx->opt_traversal == 1 ? 1 : 0, &io);
+    }
+    // the caller's later work sees the records -- also after a failure, when stages that write d_out may be enqueued
+    if (caller != s) CK(stream_edge(ctx->ev_refit[1], s, caller));
+    return st;
+}
+
+// Host-buffer radiance on one device.
+static int radiance_host(b2rt_context* ctx, const b2rt_ray* rays, const uint32_t* seeds, uint64_t n, b2rt_radiance* out) {
+    return host_pipeline(ctx, rays, sizeof(b2rt_ray), seeds, sizeof(uint32_t), n, out, sizeof(b2rt_radiance), stream_chunk(), "ray",
+                         [&](const void* d_in, const void* d_seeds, uint64_t m, void* d_out, cudaStream_t s) {
+                             return radiance_device(ctx, d_in, static_cast<const uint32_t*>(d_seeds), m, d_out, s);
+                         });
 }
 
 }  // namespace b2rt_detail
@@ -809,6 +862,7 @@ extern "C" void b2rt_destroy(b2rt_context* ctx) {
     for (int i = 0; i < 2; ++i) {
         if (ctx->d_stage_rays[i]) cudaFree(ctx->d_stage_rays[i]);
         if (ctx->d_stage_out[i]) cudaFree(ctx->d_stage_out[i]);
+        if (ctx->d_stage_in2[i]) cudaFree(ctx->d_stage_in2[i]);
         if (ctx->ev_in[i]) cudaEventDestroy(ctx->ev_in[i]);
         if (ctx->ev_comp[i]) cudaEventDestroy(ctx->ev_comp[i]);
         if (ctx->ev_out[i]) cudaEventDestroy(ctx->ev_out[i]);
@@ -1280,6 +1334,22 @@ extern "C" int b2rt_closest_point_device(b2rt_context* ctx, const b2rt_point_que
     cudaStream_t s;
     int st = device_entry(ctx, cuda_stream, &s);
     return st ? st : point_device(ctx, d_q, n, d_out, s);
+}
+// ---- path-traced radiance ---------------------------------------------------------------------
+extern "C" int b2rt_trace_radiance(b2rt_context* ctx, const b2rt_ray* rays, const uint32_t* seeds, uint64_t n, b2rt_radiance* out) {
+    if (!ctx) return B2RT_INVALID_CONTEXT;
+    if (n && (!rays || !seeds || !out)) return fail(ctx, B2RT_INVALID_VALUE, "null ray, seed or output pointer");
+    if (ctx->group)
+        return group_split(ctx, n, [&](b2rt_context* m, uint64_t lo, uint64_t cnt) { return radiance_host(m, rays + lo, seeds + lo, cnt, out + lo); });
+    return radiance_host(ctx, rays, seeds, n, out);
+}
+extern "C" int b2rt_trace_radiance_device(b2rt_context* ctx, const b2rt_ray* d_rays, const uint32_t* d_seeds, uint64_t n, b2rt_radiance* d_out,
+                                          void* cuda_stream) {
+    if (!ctx) return B2RT_INVALID_CONTEXT;
+    if (n && (!d_rays || !d_seeds || !d_out)) return fail(ctx, B2RT_INVALID_VALUE, "null ray, seed or output pointer");
+    cudaStream_t s;
+    int st = device_entry(ctx, cuda_stream, &s);
+    return st ? st : radiance_device(ctx, d_rays, d_seeds, n, d_out, s);
 }
 extern "C" int b2rt_camera_rays_device(b2rt_context* ctx, size_t gid_begin, size_t gid_end, b2rt_ray* d_rays, void* cuda_stream) {
     if (!ctx) return B2RT_INVALID_CONTEXT;

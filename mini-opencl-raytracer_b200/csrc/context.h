@@ -72,6 +72,8 @@ struct b2rt_context {
     void* d_stage_out[2] = { nullptr, nullptr };
     uint64_t stage_capacity = 0;               // rays per staging buffer ...
     size_t stage_out_bytes = 0;                // ... and bytes per output staging buffer
+    void* d_stage_in2[2] = { nullptr, nullptr };   // second input of a host-buffer entry (b2rt_trace_radiance: the seeds) ...
+    size_t stage_in2_bytes = 0;                // ... and its bytes per staging buffer
     // wavefront frame path: two ray queues, hits, per-path state, three rotating queue counters
     void* d_wf_rays[2] = { nullptr, nullptr };
     void *d_wf_hits = nullptr, *d_wf_state = nullptr;
@@ -83,7 +85,7 @@ struct b2rt_context {
     std::pair<uint64_t, int> tune_pending_key;
     int tune_pending_mode = -1;
     cudaEvent_t ev_tune[2] = { nullptr, nullptr };
-    cudaEvent_t ev_refit[2] = { nullptr, nullptr };   // b2rt_refit_scene_device: caller's stream -> context's stream and back
+    cudaEvent_t ev_refit[2] = { nullptr, nullptr };   // b2rt_refit_scene_device, b2rt_trace_radiance_device: caller's stream -> context's stream and back
     void* d_rgba8 = nullptr;            // 8-bit read-back staging
     uint64_t rgba8_capacity = 0;
     cudaEvent_t ev_in[2] = { nullptr, nullptr }, ev_comp[2] = { nullptr, nullptr }, ev_out[2] = { nullptr, nullptr };
@@ -132,6 +134,9 @@ int install_scene(b2rt_context* ctx, const DerivedScene& d);
 // refit.cu: per-triangle shading records (normals + material) of `tris`
 cudaError_t launch_shade_records(b2rt::ShadeTri* shade, const b2rt::RefTriangle* tris, uint32_t n, cudaStream_t s);
 int render_items(b2rt_context* ctx, const b2rt::GidMap& map, uint64_t n);
+// `to` waits for the work enqueued on `from` so far (ev: one of the context's events; the wait takes the recorded state, so
+// the event can be recorded again by the next call).
+cudaError_t stream_edge(cudaEvent_t ev, cudaStream_t from, cudaStream_t to);
 
 // multi.cu
 void group_destroy(b2rt_context* ctx);

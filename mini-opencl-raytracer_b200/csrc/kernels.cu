@@ -17,6 +17,8 @@
 //      one shade / accumulate / compact stage; queue lengths never leave the device.
 //  render_mega_kernel               KernelEntry as one launch: one thread per pixel, path loop
 //      around the same traversal primitives (bit-identical to the wavefront).
+//      STREAM = true (template argument of all three): the same stages with a caller's ray stream as the source and one
+//      {radiance, seed} record per path as the sink (b2rt_trace_radiance).
 //  tonemap_rgba8_kernel             accumulation image -> clamped 8-bit RGBA for display read-back.
 //  point_persistent<COUNT,CAP>      closest point on the scene per query point (point_query.cuh), persistent like
 //      trace_persistent; point_binary_kernel<CAP> the same over the reference-layout arrays, one thread per query.
@@ -663,27 +665,52 @@ __device__ __forceinline__ bool path_step(const SceneView& s, const FrameArgs& a
     return true;
 }
 
-template <bool BINARY, int CAP>
+// Where a path of the frame kernels starts and where its radiance goes. STREAM = false (frames): the camera ray of pixel
+// g with seed g + hash(frame_count), segment 0 bounded by B2RT_MAX_RENDER_DIST, radiance into the running average of the
+// pixel. STREAM = true (b2rt_trace_radiance): the caller's ray g with its tmax and RNG state io.seeds[g]; the record
+// {radiance, seed after the path} goes to io.out[g].
+__device__ __forceinline__ void stream_path_start(const RadianceIO& io, uint64_t g, float4& q0, float4& q1, uint32_t& seed) {
+    const float4* p = static_cast<const float4*>(io.rays) + 2 * g;
+    q0 = __ldcs(p); q1 = __ldcs(p + 1);
+    seed = __ldcs(io.seeds + g);
+}
+__device__ __forceinline__ void store_radiance(const RadianceIO& io, uint64_t g, V3 radiance, uint32_t seed) {
+    __stcs(static_cast<float4*>(io.out) + g, make_float4(radiance.x, radiance.y, radiance.z, __uint_as_float(seed)));
+}
+
+template <bool BINARY, int CAP, bool STREAM>
 __global__ void __launch_bounds__(128)
-render_mega_kernel(SceneView s, FrameArgs a, float* __restrict__ result, GidMap map, uint32_t n) {
+render_mega_kernel(SceneView s, FrameArgs a, float* __restrict__ result, GidMap map, uint32_t n, RadianceIO io) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const uint64_t g = map.gid(i);
-    uint32_t gid = (uint32_t)g;
-    uint32_t seed = gid + hash_u32(a.frame_count);                        // kernel_bvh.cl:445
-    V3 dir = camera_dir(a, gid, seed);
-    RayX r = make_ray(a.pos[0], a.pos[1], a.pos[2], dir.x, dir.y, dir.z);
+    uint32_t seed;
+    RayX r;
+    float tmax = 100000.0f;                                               // segment 0 of a frame: kernel_bvh.cl:355
+    if (STREAM) {
+        float4 q0, q1;
+        stream_path_start(io, g, q0, q1, seed);
+        r = make_ray(q0.x, q0.y, q0.z, q1.x, q1.y, q1.z);
+        tmax = q1.w;
+    } else {
+        uint32_t gid = (uint32_t)g;
+        seed = gid + hash_u32(a.frame_count);                             // kernel_bvh.cl:445
+        V3 dir = camera_dir(a, gid, seed);
+        r = make_ray(a.pos[0], a.pos[1], a.pos[2], dir.x, dir.y, dir.z);
+    }
     V3 radiance = v3(0.0f, 0.0f, 0.0f), beta = v3(1.0f, 1.0f, 1.0f);
     for (int b = 0; (uint32_t)b < (uint32_t)a.bounces; ++b) {              // Render(), kernel_bvh.cl:349-384
         HitX h;
-        if (BINARY) h = trace_binary<false, CAP>(s.tris, s.nodes, r, 100000.0f);
-        else h = trace_wide<false, false, CAP>(s.wide, s.leaf, r, 100000.0f, nullptr, nullptr, s.one_bits);
+        if (BINARY) h = trace_binary<false, CAP>(s.tris, s.nodes, r, tmax);
+        else h = trace_wide<false, false, CAP>(s.wide, s.leaf, r, tmax, nullptr, nullptr, s.one_bits);
         V3 no, nd;
         if (!path_step(s, a, r, h, radiance, beta, seed, no, nd)) break;
         r = make_ray(no.x, no.y, no.z, nd.x, nd.y, nd.z);
+        if (STREAM) tmax = 100000.0f;
     }
     radiance = v3(max_cl(radiance.x, 0.0f), max_cl(radiance.y, 0.0f), max_cl(radiance.z, 0.0f));
-    accumulate(result + 4 * g, a.mirror ? a.mirror + 4 * g : nullptr, radiance, a.frame_count);
+    if (STREAM) store_radiance(io, g, radiance, seed);
+    else accumulate(result + 4 * g, a.mirror ? a.mirror + 4 * g : nullptr, radiance, a.frame_count);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -693,29 +720,40 @@ render_mega_kernel(SceneView s, FrameArgs a, float* __restrict__ result, GidMap 
 // b2rt_ray records whose (ignored) tmin slot carries i, so only the 32-byte ray is compacted between
 // bounces. Hits are written by trace_persistent at the ray's queue position. Every path runs the same
 // arithmetic in the same order as KernelEntry, so frames are bit-identical to the megakernel's.
+// STREAM = true: the same stages for a caller's ray stream (b2rt_trace_radiance, see render_mega_kernel).
 // ---------------------------------------------------------------------------------------
+template <bool STREAM>
 __global__ void __launch_bounds__(256)
 wf_generate_kernel(FrameArgs a, GidMap map, uint32_t n, RayIn* __restrict__ rays, float4* __restrict__ state,
-                   unsigned long long* __restrict__ queue_count) {
+                   unsigned long long* __restrict__ queue_count, RadianceIO io) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     // counter block of this wavefront: [0..2] rotating queue lengths, [3] the traversal kernel's ray counter, [4] [5] its tail queue's length and read position, [6] [7] the second tail queue's, [8] [9] [10] helping: warps past their hand-over, warps started, tickets given back
     if (i == 0) { queue_count[0] = n; for (int k = 1; k < 16; ++k) queue_count[k] = 0; }
     if (i >= n) return;
-    uint32_t gid = (uint32_t)map.gid(i);
-    uint32_t seed = gid + hash_u32(a.frame_count);                        // kernel_bvh.cl:445
-    V3 d = camera_dir(a, gid, seed);
+    uint32_t seed;
+    float4 q0, q1;
+    if (STREAM) {
+        stream_path_start(io, map.gid(i), q0, q1, seed);                  // the direction as given and the caller's tmax
+    } else {
+        uint32_t gid = (uint32_t)map.gid(i);
+        seed = gid + hash_u32(a.frame_count);                             // kernel_bvh.cl:445
+        V3 d = camera_dir(a, gid, seed);
+        q0 = make_float4(a.pos[0], a.pos[1], a.pos[2], 0.0f);
+        q1 = make_float4(d.x, d.y, d.z, 100000.0f);                       // InitRay normalises again inside the trace stage
+    }
     float4* p = reinterpret_cast<float4*>(rays + i);
-    p[0] = make_float4(a.pos[0], a.pos[1], a.pos[2], __uint_as_float(i));
-    p[1] = make_float4(d.x, d.y, d.z, 100000.0f);                         // InitRay normalises again inside the trace stage
+    p[0] = make_float4(q0.x, q0.y, q0.z, __uint_as_float(i));
+    p[1] = q1;
     state[2 * (size_t)i] = make_float4(0.0f, 0.0f, 0.0f, __uint_as_float(seed));
     state[2 * (size_t)i + 1] = make_float4(1.0f, 1.0f, 1.0f, 0.0f);
 }
 
+template <bool STREAM>
 __global__ void __launch_bounds__(256)
 wf_shade_kernel(SceneView s, FrameArgs a, GidMap map, const RayIn* __restrict__ rays_in, const float4* __restrict__ hits,
                 const unsigned long long* __restrict__ n_in, RayIn* __restrict__ rays_out,
                 unsigned long long* __restrict__ n_out, float4* __restrict__ state, float* __restrict__ result, int last,
-                unsigned long long* __restrict__ clear_a, unsigned long long* __restrict__ clear_b) {
+                unsigned long long* __restrict__ clear_a, unsigned long long* __restrict__ clear_b, RadianceIO io) {
     const uint64_t n = *n_in;
     const uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     // reset what the NEXT stages start from: the traversal kernel's ray counter and the queue length the next
@@ -742,7 +780,8 @@ wf_shade_kernel(SceneView s, FrameArgs a, GidMap map, const RayIn* __restrict__ 
         if (!go_on) {
             radiance = v3(max_cl(radiance.x, 0.0f), max_cl(radiance.y, 0.0f), max_cl(radiance.z, 0.0f));
             const uint64_t g = map.gid(i);
-            accumulate(result + 4 * g, a.mirror ? a.mirror + 4 * g : nullptr, radiance, a.frame_count);
+            if (STREAM) store_radiance(io, g, radiance, seed);
+            else accumulate(result + 4 * g, a.mirror ? a.mirror + 4 * g : nullptr, radiance, a.frame_count);
         }
     }
     // append the surviving rays to the next queue: one atomic per warp
@@ -1030,31 +1069,44 @@ cudaError_t launch_camera_rays(const FrameArgs& a, uint64_t gid0, uint64_t gid1,
 }
 
 cudaError_t launch_render_mega(const SceneView& s, const FrameArgs& a, float* d_result, const GidMap& map, uint32_t n,
-                               bool binary, uint32_t stack_bound, uint32_t max_depth_binary, cudaStream_t st) {
+                               bool binary, uint32_t stack_bound, uint32_t max_depth_binary, cudaStream_t st, const RadianceIO* io) {
     if (n == 0) return cudaSuccess;
     unsigned g = (n + 127u) / 128u;
     // the wide walk holds at most stack_bound entries, the reference-layout walk at most max_depth_binary
     return with_cap(binary ? max_depth_binary : stack_bound, [&](auto C) {
-        if (binary) render_mega_kernel<true, C><<<g, 128, 0, st>>>(s, a, d_result, map, n);
-        else render_mega_kernel<false, C><<<g, 128, 0, st>>>(s, a, d_result, map, n);
+        if (io) {
+            if (binary) render_mega_kernel<true, C, true><<<g, 128, 0, st>>>(s, a, nullptr, map, n, *io);
+            else render_mega_kernel<false, C, true><<<g, 128, 0, st>>>(s, a, nullptr, map, n, *io);
+        } else {
+            if (binary) render_mega_kernel<true, C, false><<<g, 128, 0, st>>>(s, a, d_result, map, n, RadianceIO{ nullptr, nullptr, nullptr });
+            else render_mega_kernel<false, C, false><<<g, 128, 0, st>>>(s, a, d_result, map, n, RadianceIO{ nullptr, nullptr, nullptr });
+        }
     });
 }
 
 cudaError_t launch_wf_generate(const FrameArgs& a, const GidMap& map, uint32_t n, void* d_rays, void* d_state,
-                               unsigned long long* d_queue_count, cudaStream_t st) {
+                               unsigned long long* d_queue_count, cudaStream_t st, const RadianceIO* io) {
     if (n == 0) return cudaSuccess;
-    wf_generate_kernel<<<(n + 255u) / 256u, 256, 0, st>>>(a, map, n, static_cast<RayIn*>(d_rays), static_cast<float4*>(d_state), d_queue_count);
+    RayIn* rays = static_cast<RayIn*>(d_rays);
+    float4* state = static_cast<float4*>(d_state);
+    if (io) wf_generate_kernel<true><<<(n + 255u) / 256u, 256, 0, st>>>(a, map, n, rays, state, d_queue_count, *io);
+    else wf_generate_kernel<false><<<(n + 255u) / 256u, 256, 0, st>>>(a, map, n, rays, state, d_queue_count, RadianceIO{ nullptr, nullptr, nullptr });
     return cudaGetLastError();
 }
 
 cudaError_t launch_wf_shade(const SceneView& s, const FrameArgs& a, const GidMap& map, uint32_t n_max, const void* d_rays_in,
                             const void* d_hits, const unsigned long long* d_n_in, void* d_rays_out, unsigned long long* d_n_out,
                             void* d_state, float* d_result, bool last, unsigned long long* d_clear_a, unsigned long long* d_clear_b,
-                            cudaStream_t st) {
+                            cudaStream_t st, const RadianceIO* io) {
     if (n_max == 0) return cudaSuccess;
-    wf_shade_kernel<<<(n_max + 255u) / 256u, 256, 0, st>>>(s, a, map, static_cast<const RayIn*>(d_rays_in), static_cast<const float4*>(d_hits),
-                                                           d_n_in, static_cast<RayIn*>(d_rays_out), d_n_out, static_cast<float4*>(d_state),
-                                                           d_result, last ? 1 : 0, d_clear_a, d_clear_b);
+    const unsigned g = (n_max + 255u) / 256u;
+    const RayIn* in = static_cast<const RayIn*>(d_rays_in);
+    const float4* hits = static_cast<const float4*>(d_hits);
+    RayIn* out = static_cast<RayIn*>(d_rays_out);
+    float4* state = static_cast<float4*>(d_state);
+    if (io) wf_shade_kernel<true><<<g, 256, 0, st>>>(s, a, map, in, hits, d_n_in, out, d_n_out, state, nullptr, last ? 1 : 0, d_clear_a, d_clear_b, *io);
+    else wf_shade_kernel<false><<<g, 256, 0, st>>>(s, a, map, in, hits, d_n_in, out, d_n_out, state, d_result, last ? 1 : 0, d_clear_a, d_clear_b,
+                                                    RadianceIO{ nullptr, nullptr, nullptr });
     return cudaGetLastError();
 }
 

@@ -66,16 +66,24 @@ cudaError_t launch_closest_point(const SceneView& s, const void* d_queries, uint
 cudaError_t launch_closest_point_binary(const SceneView& s, const void* d_queries, uint64_t n, void* d_out, uint32_t max_depth_binary,
                                         cudaStream_t st);
 cudaError_t launch_camera_rays(const FrameArgs& a, uint64_t gid0, uint64_t gid1, void* d_rays, cudaStream_t st);
+// A caller's ray stream as the source and sink of the frame kernels below (b2rt_trace_radiance): the path of work item g =
+// map.gid(i) starts from rays[g] (b2rt_ray) with RNG state seeds[g], and out[g] (b2rt_radiance) receives its record. Only
+// bounces, light_type and sky of the FrameArgs are read then, and d_result is not used.
+struct RadianceIO {
+    const void* rays;
+    const uint32_t* seeds;
+    void* out;
+};
 // KernelEntry for the n pixels map.gid(0..n-1), one thread per pixel; binary: over the reference-layout arrays.
 cudaError_t launch_render_mega(const SceneView& s, const FrameArgs& a, float* d_result, const GidMap& map, uint32_t n,
-                               bool binary, uint32_t stack_bound, uint32_t max_depth_binary, cudaStream_t st);
+                               bool binary, uint32_t stack_bound, uint32_t max_depth_binary, cudaStream_t st, const RadianceIO* io = nullptr);
 // Wavefront stages of the same frame (kernels.cu): camera rays + path state, and the per-bounce shade/compact stage.
 cudaError_t launch_wf_generate(const FrameArgs& a, const GidMap& map, uint32_t n, void* d_rays, void* d_state,
-                               unsigned long long* d_queue_count, cudaStream_t st);
+                               unsigned long long* d_queue_count, cudaStream_t st, const RadianceIO* io = nullptr);
 cudaError_t launch_wf_shade(const SceneView& s, const FrameArgs& a, const GidMap& map, uint32_t n_max, const void* d_rays_in,
                             const void* d_hits, const unsigned long long* d_n_in, void* d_rays_out, unsigned long long* d_n_out,
                             void* d_state, float* d_result, bool last, unsigned long long* d_clear_a, unsigned long long* d_clear_b,
-                            cudaStream_t st);
+                            cudaStream_t st, const RadianceIO* io = nullptr);
 // float4 accumulation image -> clamped 8-bit RGBA (alpha 255), n pixels.
 cudaError_t launch_tonemap_rgba8(const void* d_image, void* d_out, uint64_t n, cudaStream_t st);
 int trace_block_threads();

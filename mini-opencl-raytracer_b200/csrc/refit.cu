@@ -303,17 +303,14 @@ bool overlap(const void* a, size_t a_bytes, const void* b, size_t b_bytes) {
     return x < y + b_bytes && y < x + a_bytes;
 }
 
-// `to` waits for the work enqueued on `from` so far (ev: one of the context's events; the wait takes the recorded state, so
-// the event can be recorded again by the next call).
+}  // namespace
+
+namespace b2rt_detail {
 cudaError_t stream_edge(cudaEvent_t ev, cudaStream_t from, cudaStream_t to) {
     cudaError_t e = cudaEventRecord(ev, from);
     if (e == cudaSuccess) e = cudaStreamWaitEvent(to, ev, 0);
     return e;
 }
-
-}  // namespace
-
-namespace b2rt_detail {
 cudaError_t launch_shade_records(ShadeTri* shade, const RefTriangle* tris, uint32_t n, cudaStream_t s) {
     if (n) refit_shade_kernel<<<(n + 255u) / 256u, 256, 0, s>>>(shade, tris, n);
     return cudaGetLastError();

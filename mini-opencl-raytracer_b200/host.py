@@ -7,7 +7,7 @@ import os
 import numpy as np
 
 from . import capi
-from .layouts import HIT_DTYPE, POINT_HIT_DTYPE, POINT_QUERY_DTYPE, RAY_DTYPE
+from .layouts import HIT_DTYPE, POINT_HIT_DTYPE, POINT_QUERY_DTYPE, RADIANCE_DTYPE, RAY_DTYPE
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
@@ -64,6 +64,7 @@ def lib():
         "g3d_engine_trace_any": (C.c_int, [vp, vp, u64, vp, cs, sz]),
         "g3d_engine_trace_multi": (C.c_int, [vp, vp, u64, C.c_uint32, vp, cs, sz]),
         "g3d_engine_closest_point": (C.c_int, [vp, vp, u64, vp, cs, sz]),
+        "g3d_engine_trace_radiance": (C.c_int, [vp, vp, vp, u64, vp, cs, sz]),
         "g3d_write_icosphere_obj": (C.c_longlong, [cs, C.c_int, C.c_double, C.c_double, C.c_ulonglong]),
         "g3d_write_scattered_obj": (C.c_longlong, [cs, C.c_longlong, C.c_double, C.c_double, C.c_double, C.c_ulonglong]),
     }
@@ -291,4 +292,15 @@ class Engine:
         out = np.empty(queries.shape[0], dtype=POINT_HIT_DTYPE)
         e = _err()
         self._ck(self._L.g3d_engine_closest_point(self._h, queries.ctypes.data, queries.shape[0], out.ctypes.data, e, len(e)), e)
+        return out
+
+    def trace_radiance(self, rays, seeds):
+        """CLRaytracer::TraceRadiance: the path-traced radiance of every ray as a RADIANCE_DTYPE array {r, g, b, seed}."""
+        rays = np.ascontiguousarray(rays, dtype=RAY_DTYPE)
+        seeds = np.ascontiguousarray(seeds, dtype=np.uint32)
+        if seeds.shape != (rays.shape[0],):
+            raise ValueError("one seed per ray: %d rays, seeds of shape %s" % (rays.shape[0], seeds.shape))
+        out = np.empty(rays.shape[0], dtype=RADIANCE_DTYPE)
+        e = _err()
+        self._ck(self._L.g3d_engine_trace_radiance(self._h, rays.ctypes.data, seeds.ctypes.data, rays.shape[0], out.ctypes.data, e, len(e)), e)
         return out

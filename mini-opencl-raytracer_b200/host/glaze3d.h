@@ -14,7 +14,7 @@
 //   CLOBJloader ........................... CLOBJloader.h, CLOBJloader.cpp:10-176
 //   CLRaytracer ........................... CLRaytracer.h:16-40, CLRaytracer.cpp:12-148
 //   CLui (state only) / CLEngineBase ...... CLui.h:17-40, CLEngineBase.h:13-93, CLEngineBase.cpp:141-211
-// New (the reference has no ray-stream API): CLRaytracer::TraceClosest / TraceAny / TraceMulti / ClosestPoint.
+// New (the reference has no ray-stream API): CLRaytracer::TraceClosest / TraceAny / TraceMulti / ClosestPoint / TraceRadiance.
 #pragma once
 #include <cstddef>
 #include <cstdint>
@@ -265,6 +265,9 @@ namespace Glaze3D
         void TraceMulti(const b2rt_ray* rays, uint64_t n, uint32_t k, b2rt_hit* hits);
         // The nearest surface point per query point (b2rt_closest_point): out[i] = {d2, u, v, tri}, {max_d2, 0, 0, B2RT_MISS} if none.
         void ClosestPoint(const b2rt_point_query* queries, uint64_t n, b2rt_point_hit* out);
+        // The path-traced radiance per ray (b2rt_trace_radiance): out[i] = {r, g, b, RNG state after the path}, shaded with
+        // the bound light bounces, light type, sky intensity and materials.
+        void TraceRadiance(const b2rt_ray* rays, const uint32_t* seeds, uint64_t n, b2rt_radiance* out);
 
         std::shared_ptr<CLContext> m_CLContext = nullptr;
         std::shared_ptr<CLKernel> m_RenderKernel = nullptr;

@@ -259,3 +259,11 @@ extern "C" int g3d_engine_closest_point(void* engine, const b2rt_point_query* qu
     return 0;
     G3D_CATCH(-1)
 }
+extern "C" int g3d_engine_trace_radiance(void* engine, const b2rt_ray* rays, const uint32_t* seeds, uint64_t n, b2rt_radiance* out, char* err,
+                                         size_t errLen)
+{
+    G3D_TRY
+    static_cast<EngineBox*>(engine)->engine->render->TraceRadiance(rays, seeds, n, out);
+    return 0;
+    G3D_CATCH(-1)
+}

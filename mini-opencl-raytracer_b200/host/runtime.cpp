@@ -172,6 +172,11 @@ namespace Glaze3D
         int st = b2rt_closest_point(m_CLContext->GetContext(), queries, n, out);
         if (st) throw CLException(std::string("Failed to query closest points: ") + b2rt_last_error(m_CLContext->GetContext()), st);
     }
+    void CLRaytracer::TraceRadiance(const b2rt_ray* rays, const uint32_t* seeds, uint64_t n, b2rt_radiance* out)
+    {
+        int st = b2rt_trace_radiance(m_CLContext->GetContext(), rays, seeds, n, out);
+        if (st) throw CLException(std::string("Failed to trace radiance: ") + b2rt_last_error(m_CLContext->GetContext()), st);
+    }
 
     // ---- CLEngineBase (headless) -------------------------------------------------------------------
     CLEngineBase::CLEngineBase()

@@ -12,6 +12,9 @@ assert RAY_DTYPE.itemsize == 32 and HIT_DTYPE.itemsize == 16
 POINT_QUERY_DTYPE = np.dtype([("x", "<f4"), ("y", "<f4"), ("z", "<f4"), ("max_d2", "<f4")])
 POINT_HIT_DTYPE = np.dtype([("d2", "<f4"), ("u", "<f4"), ("v", "<f4"), ("tri", "<u4")])
 assert POINT_QUERY_DTYPE.itemsize == 16 and POINT_HIT_DTYPE.itemsize == 16
+# b2rt_trace_radiance record: the path's radiance and the RNG state after it
+RADIANCE_DTYPE = np.dtype([("r", "<f4"), ("g", "<f4"), ("b", "<f4"), ("seed", "<u4")])
+assert RADIANCE_DTYPE.itemsize == 16
 
 # CLLinearBVHNode, 48 B
 NODE_DTYPE = np.dtype({"names": ["bmin", "bmax", "offset", "nPrimitives", "axis"],

@@ -18,9 +18,14 @@ KERNELS = {
     "trace_persistent<any-hit, no counters, CAP 64>": "trace_persistentILi1ELb0ELi64E",
     "trace_persistent<multi, no counters, CAP 64>": "trace_persistentILi2ELb0ELi64E",
     "trace_tail_kernel<closest, no counters>": "trace_tail_kernelILb0ELb0E",
-    "wf_shade_kernel": "wf_shade_kernel",
-    "wf_generate_kernel": "wf_generate_kernel",
-    "render_mega_kernel<wide, CAP 64>": "render_mega_kernelILb0ELi64E",
+    # frame instantiations (STREAM = false) under the row names they had before the kernels took the STREAM argument
+    "wf_shade_kernel": "wf_shade_kernelILb0E",
+    "wf_generate_kernel": "wf_generate_kernelILb0E",
+    "render_mega_kernel<wide, CAP 64>": "render_mega_kernelILb0ELi64ELb0E",
+    "wf_shade_kernel<radiance stream>": "wf_shade_kernelILb1E",
+    "wf_generate_kernel<radiance stream>": "wf_generate_kernelILb1E",
+    "render_mega_kernel<wide, CAP 64, radiance stream>": "render_mega_kernelILb0ELi64ELb1E",
+    "render_mega_kernel<binary, CAP 64, radiance stream>": "render_mega_kernelILb1ELi64ELb1E",
     "point_persistent<no counters, CAP 64>": "point_persistentILb0ELi64E",
     "point_binary_kernel<CAP 64>": "point_binary_kernelILi64E",
 }
